@@ -2,7 +2,7 @@
 """bench.py — benchmark of the B200 backend for VGL's frontier-processing hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload pr|bfs|sssp|cc|bfs20|config5] [--scaling weak|strong] [--no-extras]
+                    [--workload pr|bfs|sssp|cc|bfs20|config5] [--scaling weak|strong] [--no-extras] [--dump-outputs DIR]
 
 Headline (default) = BASELINE.json configs[1]: PageRank pull, 20 iterations fp32, RMAT scale-24 edge-factor 16 on one
 B200; a "step" is one complete PageRank run (20 sweeps) over the resident graph. Metric = GTEPS in the reference's
@@ -27,6 +27,11 @@ convention: iterations x graph edges / time / 1e9 (performance_stats.hpp:272-275
 
 `--impl reference` times the reference's CPU path alone (same metric / config / unit). Under torchrun (N > 1) every rank
 owns a 1D vertex range of the graph (DESIGN.md §5); `--scaling strong` keeps the graph fixed as N grows.
+
+`--dump-outputs DIR` writes what the headline's last timed step computed, in ORIGINAL vertex numbering, to DIR/<name>.npy
+(PageRank ranks and SSSP distances as float32, BFS levels and CC labels as float64). An output larger than 64 MB is
+written at 2^22 seeded positions (sorted; the same positions for the same vertex count). The graph, the sources and the
+sample depend only on the arguments, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -54,6 +59,9 @@ WORKLOADS = {
 }
 PR_ITERS = 20
 GOLDEN = ("rmat_s8_ef4", "kron_s10_ef16", "ru_s10_ef32", "rmat_s11_ef8")
+OUTPUT_NAMES = {"pr": "pagerank_ranks", "bfs": "bfs_levels", "sssp": "sssp_distances", "cc": "cc_labels"}
+DUMP_BUDGET_BYTES = 64 * 10 ** 6
+DUMP_SAMPLE = 1 << 22
 T0 = time.perf_counter()
 
 
@@ -360,8 +368,24 @@ class Bench:
                         "(outputs of the unmodified reference), on every rank through the " + ("partitioned" if self.world > 1 else "single-GPU") + " path",
                 "seconds": time.perf_counter() - t0}
 
+    def dump_outputs(self, runner, algo, out_dir):
+        """--dump-outputs: the result array of the runner's last step in ORIGINAL numbering -> out_dir/<name>.npy.
+        Collective on a partitioned graph (every rank takes part in the reorder); rank 0 writes."""
+        full = runner.g.to_original(runner.out)
+        if self.rank != 0:
+            return None
+        dtype = np.dtype(np.float32 if full.dtype == np.float32 else np.float64)  # int32 labels / levels stay exact
+        sampled = full.size * dtype.itemsize > DUMP_BUDGET_BYTES
+        if sampled:
+            full = full[np.sort(np.random.default_rng(self.vgl.MASTER_SEED).choice(full.size, DUMP_SAMPLE, replace=False))]
+        os.makedirs(out_dir, exist_ok=True)
+        name = OUTPUT_NAMES[algo]
+        np.save(os.path.join(out_dir, name + ".npy"), full.astype(dtype))
+        return {name: {"dtype": dtype.name, "values": int(full.size), "sampled": sampled}}
+
     # ---- one workload: device-timed value, roofline, e2e ----
-    def run_workload(self, workload, scale, steps, warmup, weak=True, sample_clocks=False, e2e_steps=None, td_only=False):
+    def run_workload(self, workload, scale, steps, warmup, weak=True, sample_clocks=False, e2e_steps=None, td_only=False,
+                     dump_dir=None):
         vgl, ctx, torch = self.vgl, self.ctx, self.torch
         kind, _, ef, _ = WORKLOADS[workload]
         algo = algo_of(workload)
@@ -392,6 +416,7 @@ class Bench:
             ms_per_step = self.max_float(float(np.mean([s["seconds"] for s in stats])) * 1e3)
         else:
             ms_per_step = self.max_float(ev0.elapsed_time(ev1)) / steps
+        dumped = self.dump_outputs(runner, algo, dump_dir) if dump_dir else None
         edges_per_step = runner.edges_per_step  # whole job, all ranks
         value = edges_per_step / (ms_per_step * 1e-3) / 1e9
         # dominant kernel(s): duration from the library's own CUDA events around the algorithm loop
@@ -431,6 +456,8 @@ class Bench:
         }
         if clocks is not None:
             res["clocks"] = clocks
+        if dumped is not None:
+            res["dumped_outputs"] = dumped
         runner.close()
         return res
 
@@ -466,7 +493,8 @@ def ours(args):
     headline = "pr" if config5 else args.workload
     scale = args.scale or (28 if config5 else WORKLOADS[headline][1])
     head_weak = weak and not config5
-    res = B.run_workload(headline, scale, args.steps, args.warmup, weak=head_weak, sample_clocks=True, td_only=args.top_down_only)
+    res = B.run_workload(headline, scale, args.steps, args.warmup, weak=head_weak, sample_clocks=True, td_only=args.top_down_only,
+                         dump_dir=args.dump_outputs)
 
     line = None
     if rank == 0:
@@ -485,6 +513,8 @@ def ours(args):
             "per_source_gteps": res["per_source_gteps"], "parity_check": parity,
             "extras": {"workloads": {}, "runner": res["runner_extras"]},
         }
+        if "dumped_outputs" in res:
+            line["dumped_outputs"] = {"dir": os.path.abspath(args.dump_outputs), "files": res["dumped_outputs"]}
         line_holder["line"] = line
 
     # ---- the other BASELINE configs, after (and outside) the headline's timed region ----
@@ -558,7 +588,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="headline only (profiling runs)")
     ap.add_argument("--top-down-only", action="store_true", help="BFS workloads: no direction switch (the reference's BFS::vgl_top_down)")
     ap.add_argument("--extras-budget", type=float, default=420.0, help="seconds after which no further extra workload is started")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline's result of its last timed step to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: W >= 3
     if args.impl == "reference":
