@@ -69,7 +69,7 @@ struct vglb_ctx
     // PCIe write instead of cudaMemcpyAsync + cudaStreamSynchronize
     unsigned long long *h_mailbox; // 64 words, word 63 = sequence number
     unsigned long long mailbox_seq;
-    int pr_carveout_set;   // pr_sweep_kernel's shared-memory carve-out preference has been set on this device
+    int pr_carveout_set;   // the PageRank sweep kernels' shared-memory carve-out preferences have been set on this device
     int upload_hint;       // VGLB_HINT_* (vglb_set_upload_hint)
     int prb_smem_set;      // pr_bin_kernel's dynamic shared-memory limit has been raised on this device
 };

@@ -49,6 +49,7 @@
 
 #include <time.h>
 
+#include <algorithm>
 #include <vector>
 
 #include <cub/device/device_scan.cuh>
@@ -826,18 +827,43 @@ int64_t vglb_pr_plan(const vglb_graph *g, int32_t rows, PrParams *P)
     return nblocks;
 }
 
+// Shared-memory carve-outs of the sweep's kernels (a function attribute is per device: remembered per context, not per process).
+static int pr_set_carveouts(vglb_ctx *ctx)
+{
+    if (ctx->pr_carveout_set) return VGLB_OK;
+    const bool trace = getenv("VGLB_PR_TRACE") != NULL;
+    auto occupancy = [&](const char *when) -> int {
+        if (!trace) return VGLB_OK;
+        int cold = 0, tail = 0;
+        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cold, pr_cold_bin_kernel, PR_THREADS, 0));
+        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&tail, pr_sweep_kernel<false>, PR_THREADS, 0));
+        fprintf(stderr, "pr carve-outs %s: resident CTAs per SM: pr_cold_bin_kernel %d, pr_sweep_kernel<false> %d\n", when, cold, tail);
+        return VGLB_OK;
+    };
+    int rc = occupancy("before");
+    if (rc != VGLB_OK) return rc;
+    // every KB of L1 holds hub contributions: the sweep kernel asks for the smallest carve-out (64 B static are used)
+    CUDA_TRY(cudaFuncSetAttribute(pr_sweep_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1));
+    CUDA_TRY(cudaFuncSetAttribute(pr_sweep_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1));
+    // the cold bin's gathers hit L1 < 1 % of the time, and it is latency-bound: its carve-out must hold PR_COLD_CTAS CTAs' staging
+    // (the smallest carve-out that holds one CTA's 8 KB holds only that one)
+    cudaFuncAttributes fa;
+    int reserved = 0, per_sm = 0;
+    CUDA_TRY(cudaFuncGetAttributes(&fa, pr_cold_bin_kernel));
+    CUDA_TRY(cudaDeviceGetAttribute(&reserved, cudaDevAttrReservedSharedMemoryPerBlock, ctx->device));
+    CUDA_TRY(cudaDeviceGetAttribute(&per_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, ctx->device));
+    const int64_t need = (int64_t)PR_COLD_CTAS * ((int64_t)fa.sharedSizeBytes + reserved);
+    const int pct = (int)std::min<int64_t>(100, ceil_div64(100 * need, per_sm));
+    CUDA_TRY(cudaFuncSetAttribute(pr_cold_bin_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct));
+    rc = occupancy("after");
+    if (rc != VGLB_OK) return rc;
+    ctx->pr_carveout_set = 1;
+    return VGLB_OK;
+}
+
 int vglb_pr_launch_sweep(vglb_ctx *ctx, const PrParams &P, int64_t nblocks)
 {
     if (nblocks <= 0) return VGLB_OK;
-    // every KB of L1 holds hub contributions: ask for the smallest shared-memory carve-out (64 B static are used)
-    // (a function attribute is per device: remembered per context, not per process)
-    if (!ctx->pr_carveout_set)
-    {
-        CUDA_TRY(cudaFuncSetAttribute(pr_sweep_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1));
-        CUDA_TRY(cudaFuncSetAttribute(pr_sweep_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1));
-        CUDA_TRY(cudaFuncSetAttribute(pr_cold_bin_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1));
-        ctx->pr_carveout_set = 1;
-    }
     if (P.heavy_blocks > 0) pr_sweep_kernel<true><<<(unsigned)nblocks, PR_THREADS, 0, ctx->stream>>>(P);
     else pr_sweep_kernel<false><<<(unsigned)nblocks, PR_THREADS, 0, ctx->stream>>>(P);
     KERNEL_TRY();
@@ -917,6 +943,8 @@ extern "C" int vglb_pagerank_ex(vglb_ctx *ctx, vglb_graph *g, int iters, float d
         return VGLB_OK;
     };
 
+    rc = pr_set_carveouts(ctx);
+    if (rc != VGLB_OK) return rc;
     CUDA_TRY(cudaEventRecord(ctx->ev_start, ctx->stream));
     CUDA_TRY(cudaMemsetAsync(g->d_pr_dangling, 0, (size_t)(iters + 1) * sizeof(double), ctx->stream));
     const float r0 = (float)(1.0 / (double)g->V_orig); // pr.hpp:42

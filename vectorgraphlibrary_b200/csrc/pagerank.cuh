@@ -32,6 +32,9 @@
 #ifndef PR_COLD_SPU
 #define PR_COLD_SPU 8            // steps of the cold bin handled by one warp of pr_cold_bin_kernel (A/B at RMAT-24, ms per sweep: 1 -> 0.618, 2 -> 0.578, 4 -> 0.548, 8 -> 0.531, 16 -> 0.543, 32 -> 0.576)
 #endif
+#ifndef PR_COLD_CTAS
+#define PR_COLD_CTAS 5            // resident CTAs of pr_cold_bin_kernel per SM that its shared-memory carve-out must hold (8 KB of staging each; A/B at RMAT-24, cold pass µs / ms per sweep: 1 -> 122.4 / 0.539, 3 -> 115.5 / 0.532, 5 -> 97.3 / 0.513; 2 is no carve-out of its own: the one that holds 2 holds 3)
+#endif
 #ifndef PR_ZERO_ROWS_PER_CTA
 #define PR_ZERO_ROWS_PER_CTA 4096 // rows without out-edges handled by one CTA
 #endif
