@@ -220,6 +220,25 @@ typedef struct vglb_bfs_opts
 int vglb_bfs(vglb_ctx *ctx, vglb_graph *g, int32_t source_sorted, int32_t *d_levels, const vglb_bfs_opts *opts,
              vglb_stats *stats);
 
+/* Multi-source BFS: the levels of num_sources (1..VGLB_BFS_MULTI_MAX_SOURCES) BFS runs over one graph in one traversal
+ * (bit-parallel frontiers: bit i of a vertex's word = source i). Row i of d_levels (d_levels + i*V, SCATTER numbering)
+ * equals what vglb_bfs(g, h_sources_sorted[i], ...) writes: source = 1, unreachable = -1. Sources may repeat.
+ * h_sources_sorted is a host array. opts as for vglb_bfs (direction_optimising, alpha, beta); the direction choice never
+ * changes the levels. One-GPU graphs only: a partitioned graph returns VGLB_EINVAL.
+ * The per-vertex words are w = 4 bytes for num_sources <= 32 and 8 bytes above; the call takes 3*V*w bytes of scratch for its
+ * duration. stats: edges_inspected (e) and vertices_processed (f) count each edge / row once per level, not once per source;
+ * iterations = levels. With e_l, f_l the edges and rows of level l, R the (vertex, source) pairs reached (sources included)
+ * and k = num_sources:
+ *   algorithmic_bytes = sum_l [ (4 + w) e_l + (12 + w) f_l + g_l ] + 4 k V + 4 R
+ * (an edge reads its 4-byte id and one gathered word; a row its two row pointers, its queue entry and its own word; 4kV
+ * initialises the output, 4R are the level stores), where the frontier traffic g_l (= frontier_bytes) is (8 + w) n_l for a
+ * top-down level that queues n_l vertices, plus (4 + w) per queued vertex whose word is cleared for the next top-down level,
+ * 2 w V + V/8 for a bottom-up level (seen and next words, no-in-edge mask), and 2 w V + 4 n for turning n dense words back
+ * into queues. */
+#define VGLB_BFS_MULTI_MAX_SOURCES 64
+int vglb_bfs_multi(vglb_ctx *ctx, vglb_graph *g, int32_t num_sources, const int32_t *h_sources_sorted,
+                   int32_t *d_levels, const vglb_bfs_opts *opts, vglb_stats *stats);
+
 /* SSSP, frontier Bellman-Ford (algorithms/sssp/shortest_paths.hpp:7-78, gpu_shortest_paths.hpp:133-196): min-plus
  * fixed point in fp32 (bit-identical to the reference's seq_dijkstra), unreachable = FLT_MAX; d_weights indexed by
  * out-CSR position. The frontier is scheduled near/far around a moving distance threshold (fewer re-relaxations than the

@@ -31,6 +31,7 @@ GRAPH_WITH_INCOMING, GRAPH_WITH_EDGE_ORDER = 1, 2
 HINT_PAGERANK = 1  # vglb_set_upload_hint
 MASTER_SEED = 0xB200
 NUM_TIERS = 8
+BFS_MULTI_MAX_SOURCES = 64  # VGLB_BFS_MULTI_MAX_SOURCES: sources of one vglb_bfs_multi call
 
 
 class VglbError(RuntimeError):
@@ -110,6 +111,7 @@ _SIGNATURES = {
     "vglb_pagerank": (C.c_int, [_P, _P, C.c_int, C.c_float, _P, C.POINTER(Stats)]),
     "vglb_pagerank_ex": (C.c_int, [_P, _P, C.c_int, C.c_float, C.POINTER(PrOpts), _P, C.POINTER(Stats)]),
     "vglb_bfs": (C.c_int, [_P, _P, C.c_int32, _P, C.POINTER(BfsOpts), C.POINTER(Stats)]),
+    "vglb_bfs_multi": (C.c_int, [_P, _P, C.c_int32, _P, _P, C.POINTER(BfsOpts), C.POINTER(Stats)]),
     "vglb_sssp": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.POINTER(Stats)]),
     "vglb_cc": (C.c_int, [_P, _P, _P, C.POINTER(Stats)]),
     "vglb_frontier_create": (C.c_int, [_P, _P, C.POINTER(_P)]),
@@ -478,6 +480,18 @@ class Graph:
     def set_exchange(self, mode: int):
         _check(lib().vglb_graph_set_exchange(self.ctx.h, self.h, mode))
 
+    def to_original_rows(self, arr: DeviceArray, k: int) -> np.ndarray:
+        """(k, V) array in ORIGINAL numbering of k consecutive V-sized rows in SCATTER numbering (vglb_bfs_multi's output).
+        One-GPU graphs only."""
+        assert arr.dtype.itemsize == 4 and arr.n >= k * self.V
+        row = self.ctx.empty(self.V, arr.dtype)
+        out = np.empty((k, self.V), arr.dtype)
+        for i in range(k):
+            _check(lib().vglb_varray_reorder_u32(self.ctx.h, self.h, arr.ptr + i * self.V * 4, row.ptr, SCATTER, ORIGINAL))
+            out[i] = row.to_numpy()
+        row.free()
+        return out
+
     def to_original(self, arr: DeviceArray) -> np.ndarray:
         """VerticesArray::reorder(ORIGINAL) + move_to_host (a collective on a partitioned graph: every rank gets the
         whole array)."""
@@ -520,6 +534,18 @@ class Graph:
         st = Stats()
         opts = BfsOpts(int(direction_optimising), alpha, beta, 0)
         _check(lib().vglb_bfs(self.ctx.h, self.h, int(source_sorted), levels.ptr, C.byref(opts), C.byref(st)))
+        return levels, st
+
+    def bfs_multi(self, sources_sorted, direction_optimising: bool = True, levels: DeviceArray | None = None,
+                  alpha: int = 0, beta: int = 0):
+        """vglb_bfs_multi: up to BFS_MULTI_MAX_SOURCES BFS runs in one traversal. Returns (k*V int32 levels, row i =
+        Graph.bfs(sources_sorted[i]), Stats)."""
+        src = np.ascontiguousarray(np.asarray(sources_sorted, np.int32).reshape(-1))
+        k = len(src)
+        levels = levels or self.ctx.empty(max(1, k) * self.V, np.int32)
+        st = Stats()
+        opts = BfsOpts(int(direction_optimising), alpha, beta, 0)
+        _check(lib().vglb_bfs_multi(self.ctx.h, self.h, k, src.ctypes.data, levels.ptr, C.byref(opts), C.byref(st)))
         return levels, st
 
     def sssp(self, weights: DeviceArray, source_sorted: int, dist: DeviceArray | None = None):

@@ -40,45 +40,11 @@ static double trace_now()
 #define BFS_BU_PROBE 4       // in-neighbours probed per batch by one lane
 #define BFS_BU_PROBE_MAX 16  // lane-private probes before the warp takes the row over
 #define BFS_BIG_CHUNK 8192 // a "big" row is expanded by CTAs, one per chunk of this many edges
-#define BFS_BIG_DEGREE 512 // one GPU: rows with at least this many edges are big (a 2691-edge source row took one warp 150 us)
 
 // NT threads (a CTA, a warp or an 8-lane group) expand the out-row [s,e) of one frontier vertex.
 // Every thread of the warp must call this together (ballots inside); `e <= s` for idle groups.
 // PART = the graph is one rank's part: `visited` is the replicated bitmap (read only here) and discoveries are only
 // marked in the candidate bitmap `levels` points to (reinterpreted) — owners resolve them after the exchange.
-#define BFS_TD_UNROLL 4 // edges per thread and step: their loads, visited tests and atomics are independent
-
-// one warp-aggregated queue claim per degree tier for BFS_TD_UNROLL candidates per lane
-__device__ __forceinline__ void enqueue_binned_multi(const bool (&won)[BFS_TD_UNROLL], const int32_t (&v)[BFS_TD_UNROLL], int32_t b0,
-                                                     int32_t b1, const TierQueues &nq, unsigned long long *counters)
-{
-    const unsigned lane = threadIdx.x & 31;
-    const unsigned below = (1u << lane) - 1u;
-#pragma unroll
-    for (int t = 0; t < 3; t++)
-    {
-        unsigned mask[BFS_TD_UNROLL];
-        int total = 0;
-#pragma unroll
-        for (int k = 0; k < BFS_TD_UNROLL; k++)
-        {
-            const int tier = v[k] < b0 ? 0 : (v[k] < b1 ? 1 : 2);
-            mask[k] = __ballot_sync(0xffffffffu, won[k] && tier == t);
-            total += __popc(mask[k]);
-        }
-        if (total == 0) continue;
-        unsigned long long base = 0;
-        if (lane == 0) base = atomicAdd(&counters[C_NEXT_BIG + t], (unsigned long long)total);
-        base = __shfl_sync(0xffffffffu, base, 0);
-#pragma unroll
-        for (int k = 0; k < BFS_TD_UNROLL; k++)
-        {
-            if ((mask[k] >> lane) & 1u) nq.q[t][base + __popc(mask[k] & below)] = v[k];
-            base += __popc(mask[k]);
-        }
-    }
-}
-
 // how a partitioned top-down level hands a discovery to the vertex's owner
 struct PartArgs
 {
@@ -551,7 +517,7 @@ __global__ void bfs_no_in_edges_kernel(const int64_t *__restrict__ in_ptr, int32
     }
 }
 
-static int bfs_prepare_no_in_edges(vglb_ctx *ctx, vglb_graph *g)
+int bfs_prepare_no_in_edges(vglb_ctx *ctx, vglb_graph *g)
 {
     if (g->d_scratch_i32 || !g->d_in_ptr) return VGLB_OK;
     CUDA_TRY(vglb_dev_alloc(&g->d_scratch_i32, (((size_t)g->V + 31) / 32 + 32) * 4));
