@@ -6,7 +6,8 @@ ms per sweep from the library's CUDA events over `reps` runs of 20 sweeps (media
 activities) of 2 x 20 sweeps with every kernel's mean duration per sweep (the passes run one after another on one stream, so
 each duration is the time of that pass by itself). VGLB_PR_TRACE=1 is set for the first run, so the library prints each
 kernel's resident CTAs per SM before and after it sets the shared-memory carve-outs. With VGLB_LIB_PATH it times a developer
-A/B build (scripts/dev_build_variant.sh)."""
+A/B build (scripts/dev_build_variant.sh); the kernels a build does not have (pr_finish_kernel ran as a pass of its own until
+pr_sweep_kernel<false> took its blocks) are left out of the per-kernel line."""
 import os
 import statistics
 import subprocess
@@ -19,7 +20,7 @@ from torch.profiler import ProfilerActivity, profile
 
 import vectorgraphlibrary_b200 as vgl
 
-KERNELS = ["pr_bin_kernel", "pr_cold_bin_kernel", "pr_sweep_kernel", "pr_finish_kernel"]
+KERNELS = ["pr_bin_kernel", "pr_cold_bin_kernel", "pr_sweep_kernel", "pr_finish_kernel"]  # the passes of a sweep, in order
 ITERS = 20
 reps = int(sys.argv[1]) if len(sys.argv) > 1 else 7
 
@@ -52,7 +53,7 @@ with vgl.Context(0) as ctx:
             if e.key.split("(")[0].split(" ")[-1].split("<")[0] == k:
                 per[k] = per.get(k, 0.0) + e.device_time_total
     sweeps = 2 * ITERS
-    parts = "  ".join(f"{k} {per.get(k, 0.0) / sweeps:.1f}" for k in KERNELS)
+    parts = "  ".join(f"{k} {per[k] / sweeps:.1f}" for k in KERNELS if k in per)
     print(f"us per sweep per kernel (torch.profiler): {parts}  sum {sum(per.values()) / sweeps:.1f}", flush=True)
     out.free()
     g.free()

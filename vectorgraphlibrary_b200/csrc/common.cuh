@@ -104,6 +104,9 @@ struct vglb_graph
     int32_t pr_ve_segments;
     void *pr_bins;              // column-binned copy of the heavy rows (PrBins, pagerank_bins.cu); NULL = warp tasks
     int pr_bins_tried;
+    int pr_zero_ready;          // pr_zero_kept / pr_zero_dangling are counted (one GPU; PrParams::zero_kept)
+    int32_t pr_zero_kept;
+    int32_t pr_zero_dangling;
     int32_t col_of_row0;        // column id of local row 0 (0 unless the graph is one rank's part of a partitioned graph)
     // 1D partition (partition.cu). On one GPU: cols = V_orig = vp = V, E_global = E, comm = NULL.
     // On a partitioned graph V / E are this rank's rows / edges; vertex state is indexed by COLUMN id in [0, cols):

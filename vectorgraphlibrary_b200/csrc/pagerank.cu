@@ -9,9 +9,11 @@
 // B200 design: no atomics on the rank vector, no host sync inside the loop, a fixed summation order.
 //   Round 2 (one GPU, 2-rank partitions): the rows with >= 32 edges go through the COLUMN BINS of pagerank_bins.cu — their edges
 //   regrouped by column bin, a bin's slice of the contribution vector in shared memory, 16-bit columns — so a sweep is
-//   pr_bin_kernel + pr_cold_bin_kernel + pr_sweep_kernel<false> (the rows with < 32 edges, below) + pr_finish_kernel
-//   (0.743 -> 0.53 ms per sweep at RMAT-24, DESIGN.md §4.1). What follows describes the one-kernel sweep that still runs on
-//   partitions of more than 2 ranks (and with VGLB_PR_NO_BINS), and whose tail / zero-row / epilogue code both forms share.
+//   pr_bin_kernel + pr_cold_bin_kernel + pr_sweep_kernel<false> (the sums of the heavy rows' partial sums, interleaved with
+//   the rows with < 32 edges, below) (0.743 -> 0.53 ms per sweep at RMAT-24, DESIGN.md §4.1). On one GPU the rows without
+//   out-edges past the bins' columns are only written by the sweep that stores the ranks (PrParams::zero_kept). What follows
+//   describes the one-kernel sweep that still runs on partitions of more than 2 ranks (and with VGLB_PR_NO_BINS), and whose
+//   tail / zero-row / epilogue code both forms share.
 //   ONE kernel per sweep:
 //   * contrib[v] = r[v]*inv[v] is produced by the epilogue of the previous sweep, so the E-pass gathers one fp32 per
 //     edge (the product is the same fp32 multiply the reference does per edge, pr.hpp:112-115).
@@ -57,13 +59,17 @@
 #include "common.cuh"
 #include "pagerank.cuh"
 
+// A gather in two halves (pr_zero_scale, pagerank.cuh): the load of contrib[v], or of inv[v] for a column from zero_kept on,
+// then the multiply that makes the latter a contribution, applied where the value is summed
 __device__ __forceinline__ float pr_gather(const PrParams &P, const L2Pol &pol, int32_t v)
 {
     // hubs have the smallest local rows of every rank's slice: column = owner * vp + local row
     const uint32_t local = P.vp_mask ? ((uint32_t)v & P.vp_mask) : (P.vp ? (uint32_t)v % P.vp : (uint32_t)v);
-    if (local >= P.cold_local) return ld_gather_cold_f32(P.contrib_in + v, pol.keep);
-    return ld_gather_f32(P.contrib_in + v, pol.keep);
+    const float *src = (v >= P.zero_kept ? P.inv : P.contrib_in) + v;
+    if (local >= P.cold_local) return ld_gather_cold_f32(src, pol.keep);
+    return ld_gather_f32(src, pol.keep);
 }
+__device__ __forceinline__ float pr_gathered(const PrParams &P, int32_t v, float z0, float x) { return pr_zero_scale(v >= P.zero_kept, z0, x); }
 
 __device__ __forceinline__ void pr_epilogue(const PrParams &P, const L2Pol &pol, int32_t row, float sum, float dang, double &dang_local)
 {
@@ -90,7 +96,7 @@ struct Quad
     float left, right; // sums of the elements before / at-or-after the boundary
 };
 
-__device__ __forceinline__ Quad pr_quad(const PrParams &P, const L2Pol &pol, const int4 a, int p, int e_lo, int e_hi, int nb, int col_cur)
+__device__ __forceinline__ Quad pr_quad(const PrParams &P, const L2Pol &pol, float z0, const int4 a, int p, int e_lo, int e_hi, int nb, int col_cur)
 {
     // element j lives at relative position p + j; valid iff e_lo <= p + j < e_hi; its row's column id is col_cur (+1 past nb)
     const int c[4] = {a.x, a.y, a.z, a.w};
@@ -102,6 +108,8 @@ __device__ __forceinline__ Quad pr_quad(const PrParams &P, const L2Pol &pol, con
         const int self = col_cur + (q >= nb ? 1 : 0);
         x[j] = (q >= e_lo && q < e_hi && c[j] != self) ? pr_gather(P, pol, c[j]) : 0.f;
     }
+#pragma unroll
+    for (int j = 0; j < 4; j++) x[j] = pr_gathered(P, c[j], z0, x[j]);
     Quad r;
     r.left = 0.f;
     r.right = 0.f;
@@ -114,7 +122,7 @@ __device__ __forceinline__ Quad pr_quad(const PrParams &P, const L2Pol &pol, con
     return r;
 }
 
-__device__ __forceinline__ void pr_heavy_task(const PrParams &P, const L2Pol &pol, const PrTask T, int lane, float dang, double &dang_local)
+__device__ __forceinline__ void pr_heavy_task(const PrParams &P, const L2Pol &pol, const PrTask T, int lane, float dang, float z0, double &dang_local)
 {
     const unsigned FULL = 0xffffffffu;
     const int64_t a4 = T.e0 & ~(int64_t)3;
@@ -144,10 +152,10 @@ __device__ __forceinline__ void pr_heavy_task(const PrParams &P, const L2Pol &po
                 const float x1 = (p + 1 >= e_lo && p + 1 < e_hi && a[u].y != self) ? pr_gather(P, pol, a[u].y) : 0.f;
                 const float x2 = (p + 2 >= e_lo && p + 2 < e_hi && a[u].z != self) ? pr_gather(P, pol, a[u].z) : 0.f;
                 const float x3 = (p + 3 >= e_lo && p + 3 < e_hi && a[u].w != self) ? pr_gather(P, pol, a[u].w) : 0.f;
-                acc0 += x0;
-                acc1 += x1;
-                acc2 += x2;
-                acc3 += x3;
+                acc0 += pr_gathered(P, a[u].x, z0, x0);
+                acc1 += pr_gathered(P, a[u].y, z0, x1);
+                acc2 += pr_gathered(P, a[u].z, z0, x2);
+                acc3 += pr_gathered(P, a[u].w, z0, x3);
             }
         }
         const float acc = warp_sum_f32((acc0 + acc1) + (acc2 + acc3));
@@ -212,7 +220,7 @@ __device__ __forceinline__ void pr_heavy_task(const PrParams &P, const L2Pol &po
         for (int u = 0; u < 2; u++)
         {
             const int p = (s + u) * 128 + lane * 4;
-            qd[u] = pr_quad(P, pol, a[u], p, e_lo, e_hi, nb[u], P.col_of_row0 + T.row0 + curs[u]);
+            qd[u] = pr_quad(P, pol, z0, a[u], p, e_lo, e_hi, nb[u], P.col_of_row0 + T.row0 + curs[u]);
         }
 #pragma unroll
         for (int u = 0; u < 2; u++)
@@ -254,7 +262,8 @@ __device__ __forceinline__ void pr_heavy_task(const PrParams &P, const L2Pol &po
 //  vector_extension.hpp:45-106: segments of 32 consecutive rows, padded to the segment's longest row with the row's own
 //  id; rows are degree-sorted, so the padding is a few per cent). No row pointers, no shuffles, every load coalesced and
 //  independent; two segments are in flight per warp.
-__device__ __forceinline__ void pr_tail_segments(const PrParams &P, const L2Pol &pol, int seg0, int seg1, int lane, float dang, double &dang_local)
+__device__ __forceinline__ void pr_tail_segments(const PrParams &P, const L2Pol &pol, int seg0, int seg1, int lane, float dang, float z0,
+                                                 double &dang_local)
 {
     for (int seg = seg0; seg < seg1; seg += 2)
     {
@@ -287,8 +296,8 @@ __device__ __forceinline__ void pr_tail_segments(const PrParams &P, const L2Pol 
 #pragma unroll
             for (int u = 0; u < PR_TAIL_J; u += 2)
             {
-                acc_a += x[u] + x[u + 1];
-                acc_b += y[u] + y[u + 1];
+                acc_a += pr_gathered(P, a[u], z0, x[u]) + pr_gathered(P, a[u + 1], z0, x[u + 1]);
+                acc_b += pr_gathered(P, c[u], z0, y[u]) + pr_gathered(P, c[u + 1], z0, y[u + 1]);
             }
         }
         if (row_a < P.zero_first) pr_epilogue(P, pol, row_a, acc_a, dang, dang_local);
@@ -351,8 +360,15 @@ __device__ __forceinline__ void pr_dangling_reduce(const PrParams &P, double *s_
     }
 }
 
-// HEAVY = false: the graph's heavy rows went through the column bins — only tail and zero-row blocks, so the kernel needs fewer
-// registers and more CTAs fit an SM (the tail rows are latency-bound).
+// rank0 of the previous sweep: the contributions of the rows without out-edges that the gathers compute are rank0_prev * inv
+__device__ __forceinline__ float pr_zero_rank_prev(const PrParams &P)
+{
+    return P.dangling_prev ? pr_zero_rank(P.k, P.d, (float)(*P.dangling_prev)) : P.r0;
+}
+
+// HEAVY = false: the graph's heavy rows went through the column bins, and the heavy blocks add up their partial sums
+// (pr_finish_binned). That coalesced stream runs next to the latency-bound gathers of the tail rows instead of in a pass of its
+// own; the kernel needs fewer registers, and more CTAs fit an SM.
 template <bool HEAVY>
 __global__ void __launch_bounds__(PR_THREADS, HEAVY ? PR_MIN_CTAS : PR_TAIL_MIN_CTAS) pr_sweep_kernel(const __grid_constant__ PrParams P)
 {
@@ -373,23 +389,29 @@ __global__ void __launch_bounds__(PR_THREADS, HEAVY ? PR_MIN_CTAS : PR_TAIL_MIN_
     double dang_local = 0.0;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 
-    if (HEAVY && b < P.heavy_blocks)
+    if (b < P.heavy_blocks)
     {
-        const int t = b * PR_WARPS + warp;
-        if (t < P.ntasks) pr_heavy_task(P, pol, P.tasks[t], lane, dang, dang_local);
+        if (HEAVY)
+        {
+            const int t = b * PR_WARPS + warp;
+            if (t < P.ntasks) pr_heavy_task(P, pol, P.tasks[t], lane, dang, pr_zero_rank_prev(P), dang_local);
+        }
+        else
+            pr_finish_binned(P, pol, b, warp, lane, dang, dang_local);
     }
     else if (b < P.heavy_blocks + P.tail_blocks)
     {
         const int seg0 = ((b - P.heavy_blocks) * PR_WARPS + warp) * PR_VE_SEGS_PER_WARP;
-        pr_tail_segments(P, pol, seg0, min(seg0 + PR_VE_SEGS_PER_WARP, P.ve_segments), lane, dang, dang_local);
+        pr_tail_segments(P, pol, seg0, min(seg0 + PR_VE_SEGS_PER_WARP, P.ve_segments), lane, dang, pr_zero_rank_prev(P), dang_local);
     }
     else
     {
         // rows without out-edges: only the post-op, coalesced
         const int32_t row0 = P.zero_first + (b - P.heavy_blocks - P.tail_blocks) * PR_ZERO_ROWS_PER_CTA;
-        const int32_t row1 = min(row0 + PR_ZERO_ROWS_PER_CTA, P.rows);
-        // every such row gets the same rank k + d * (0 + dangling) (pr_epilogue with sum = 0): one multiply and one store per row
-        const float rank0 = __fadd_rn(P.k, __fmul_rn(P.d, __fadd_rn(0.f, dang)));
+        int32_t row1 = min(row0 + PR_ZERO_ROWS_PER_CTA, P.rows);
+        if (!P.rank_out) row1 = min(row1, P.zero_kept); // (the one block a sweep of nothing else launches)
+        // every such row gets the same rank: one multiply and one store per row
+        const float rank0 = pr_zero_rank(P.k, P.d, dang);
         int ndang = 0;
 #pragma unroll 4
         for (int32_t row = row0 + threadIdx.x; row < row1; row += PR_THREADS)
@@ -405,9 +427,12 @@ __global__ void __launch_bounds__(PR_THREADS, HEAVY ? PR_MIN_CTAS : PR_TAIL_MIN_
                 ndang++;
             if (P.rank_out) st_stream_f32(P.rank_out + row, rank0);
         }
-        // (n equal terms: every partial sum is an exact multiple of a 24-bit value, so n * term is what adding them one by one gives)
-        dang_local += (double)__fdiv_rn(rank0, P.v_as_float) * (double)ndang;
+        // (n equal terms: every partial sum is an exact multiple of a 24-bit value, so n * term is what adding them one by one gives;
+        // zero_kept is a block boundary, and the rows from there on are counted once per sweep, below)
+        if (row0 < P.zero_kept) dang_local += (double)__fdiv_rn(rank0, P.v_as_float) * (double)ndang;
     }
+    if (blockIdx.x == 0 && threadIdx.x == 0)
+        dang_local += (double)__fdiv_rn(pr_zero_rank(P.k, P.d, dang), P.v_as_float) * (double)P.zero_dangling;
     pr_dangling_reduce(P, s_dang, dang_local, lane, warp);
 }
 
@@ -423,20 +448,8 @@ __global__ void __launch_bounds__(PR_THREADS, PR_MIN_CTAS) pr_cold_bin_kernel(co
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int end_step = P.bin_nkchunks * PRB_SPC;
     const int s0 = P.bins.cold_chunk0 * PRB_SPC + (blockIdx.x * PR_WARPS + warp) * PR_COLD_SPU; // units of PR_COLD_SPU steps
-    if (s0 < end_step) prb_unit<true>(P.bins, pol, NULL, s0, min(s0 + PR_COLD_SPU, end_step), end_step, lane, s_stage[warp]);
-}
-
-__global__ void __launch_bounds__(PR_THREADS) pr_finish_kernel(const __grid_constant__ PrParams P)
-{
-    L2Pol pol;
-    pol.stream = l2_policy_evict_first();
-    pol.keep = l2_policy_evict_last();
-    __shared__ double s_dang[PR_WARPS];
-    const float dang = (float)(*P.dangling_in);
-    double dang_local = 0.0;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    pr_finish_binned(P, pol, blockIdx.x, warp, lane, dang, dang_local);
-    pr_dangling_reduce(P, s_dang, dang_local, lane, warp);
+    if (s0 < end_step)
+        prb_unit<true>(P.bins, pol, NULL, s0, min(s0 + PR_COLD_SPU, end_step), end_step, lane, s_stage[warp], pr_zero_rank_prev(P));
 }
 
 // inv[v] = (float)(1.0 / indeg_noloops[v]) or 0 — pr.hpp:66-73 (double division then narrowing, like the reference)
@@ -448,6 +461,15 @@ __global__ void pr_inverse_degree_kernel(const int32_t *__restrict__ indeg, int3
         const int32_t d = indeg[v];
         inv[v] = d == 0 ? 0.0f : (float)(1.0 / (double)d);
     }
+}
+
+// rows [first, V) with inv == 0
+__global__ void pr_count_no_inv_kernel(const float *__restrict__ inv, int32_t first, int32_t V, unsigned long long *__restrict__ count)
+{
+    int n = 0;
+    for (int64_t v = first + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; v < V; v += (int64_t)gridDim.x * blockDim.x) n += inv[v] == 0.0f;
+    n = __reduce_add_sync(0xffffffffu, n);
+    if ((threadIdx.x & 31) == 0 && n > 0) atomicAdd(count, (unsigned long long)n);
 }
 
 // in-degree without self loops by column id, counted over this rank's rows (summed over ranks by the caller)
@@ -769,6 +791,35 @@ int vglb_pr_prepare(vglb_ctx *ctx, vglb_graph *g, int iters)
         if (rc != VGLB_OK) return rc;
         lap("padded copy of the tail rows");
     }
+    if (!g->comm)
+    {
+        // the rows without out-edges whose contributions the sweeps may leave unstored: pr_bin_kernel loads its bins' columns
+        // from the stored vector, so they start past those, at a block boundary of the zero-row blocks
+        const int32_t zero_first = g->tier_border[VGLB_NUM_TIERS - 2];
+        const int64_t smem_cols = g->pr_bins ? std::min<int64_t>((int64_t)((const PrBins *)g->pr_bins)->nb * PRB_H, g->V) : 0;
+        const int32_t kept = (int32_t)std::min<int64_t>(
+            g->V, zero_first + ceil_div64(std::max<int64_t>(0, smem_cols - zero_first), PR_ZERO_ROWS_PER_CTA) * PR_ZERO_ROWS_PER_CTA);
+        if (!g->pr_zero_ready || g->pr_zero_kept != kept)
+        {
+            unsigned long long *d_n = NULL, n = 0;
+            CUDA_TRY(vglb_dev_alloc(&d_n, sizeof(*d_n)));
+            CUDA_TRY(cudaMemsetAsync(d_n, 0, sizeof(*d_n), ctx->stream));
+            if (kept < g->V)
+            {
+                pr_count_no_inv_kernel<<<(unsigned)std::min<int64_t>(ctx->sm_count * 8, ceil_div64(g->V - kept, 256)), 256, 0, ctx->stream>>>(
+                    g->d_pr_inv, kept, g->V, d_n);
+                KERNEL_TRY();
+                ctx->launches++;
+            }
+            CUDA_TRY(cudaMemcpyAsync(&n, d_n, sizeof(n), cudaMemcpyDeviceToHost, ctx->stream));
+            CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+            vglb_dev_free(d_n);
+            g->pr_zero_kept = kept;
+            g->pr_zero_dangling = (int32_t)n;
+            g->pr_zero_ready = 1;
+            lap("rows without out-edges");
+        }
+    }
     if (g->pr_dangling_slots < iters + 1)
     {
         vglb_dev_free(g->d_pr_dangling);
@@ -805,7 +856,7 @@ int64_t vglb_pr_plan(const vglb_graph *g, int32_t rows, PrParams *P)
         vglb_pr_bins_params(g, NULL, &P->bins);
         P->bin_cold_blocks = (int32_t)ceil_div64(ceil_div64((int64_t)(B->nkchunks - B->cold_chunk0) * PRB_SPC, PR_COLD_SPU), PR_WARPS);
         P->ntasks = 0;
-        P->heavy_blocks = 0;
+        P->heavy_blocks = P->bin_finish_blocks;
     }
     P->ve_adj = g->d_pr_ve_adj;
     P->ve_ptr = g->d_pr_ve_ptr;
@@ -842,7 +893,9 @@ static int pr_set_carveouts(vglb_ctx *ctx)
     };
     int rc = occupancy("before");
     if (rc != VGLB_OK) return rc;
-    // every KB of L1 holds hub contributions: the sweep kernel asks for the smallest carve-out (64 B static are used)
+    // every KB of L1 holds hub contributions: the sweep kernel asks for the smallest carve-out (64 B static are used). For
+    // pr_sweep_kernel<false> it holds 7 CTAs, not the 8 its registers allow: the next larger carve-out, which holds 8, made that
+    // pass 15 µs slower at RMAT-24 (DESIGN.md §4.1)
     CUDA_TRY(cudaFuncSetAttribute(pr_sweep_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1));
     CUDA_TRY(cudaFuncSetAttribute(pr_sweep_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1));
     // the cold bin's gathers hit L1 < 1 % of the time, and it is latency-bound: its carve-out must hold PR_COLD_CTAS CTAs' staging
@@ -864,7 +917,7 @@ static int pr_set_carveouts(vglb_ctx *ctx)
 int vglb_pr_launch_sweep(vglb_ctx *ctx, const PrParams &P, int64_t nblocks)
 {
     if (nblocks <= 0) return VGLB_OK;
-    if (P.heavy_blocks > 0) pr_sweep_kernel<true><<<(unsigned)nblocks, PR_THREADS, 0, ctx->stream>>>(P);
+    if (!P.bin_slot && P.heavy_blocks > 0) pr_sweep_kernel<true><<<(unsigned)nblocks, PR_THREADS, 0, ctx->stream>>>(P);
     else pr_sweep_kernel<false><<<(unsigned)nblocks, PR_THREADS, 0, ctx->stream>>>(P);
     KERNEL_TRY();
     ctx->launches++;
@@ -903,6 +956,19 @@ extern "C" int vglb_pagerank_ex(vglb_ctx *ctx, vglb_graph *g, int iters, float d
     VGLB_REQUIRE(nblocks < 0x7fffffffLL, "vglb_pagerank: grid too large");
     P.inv = g->d_pr_inv;
     P.col_of_row0 = col0;
+    // The rows without out-edges from zero_kept on (PrParams). Every sweep stores them on a partitioned graph (the sweep writes
+    // the peers' copies of the vector) and in reference order (its dangling sum reads every rank after each sweep), and with
+    // VGLB_PR_STORE_ZERO_ROWS (developer A/B knob).
+    const bool store_zero_rows = comm || ref_order || getenv("VGLB_PR_STORE_ZERO_ROWS") != NULL;
+    P.zero_kept = store_zero_rows ? INT32_MAX : g->pr_zero_kept;
+    P.zero_dangling = store_zero_rows ? 0 : g->pr_zero_dangling;
+    P.bins.zero_col = P.zero_kept;
+    // a sweep that stores no ranks launches no blocks for them (but one at least where block 0 has their dangling share to add)
+    const int64_t nblocks_lean =
+        store_zero_rows ? nblocks
+                        : std::max<int64_t>(P.zero_dangling > 0 ? 1 : 0,
+                                            std::min<int64_t>(nblocks, (int64_t)P.heavy_blocks + P.tail_blocks +
+                                                                           ceil_div64(P.zero_kept - P.zero_first, PR_ZERO_ROWS_PER_CTA)));
     P.npeers = 0;
     P.d = damping;
     P.v_as_float = (float)g->V_orig;
@@ -948,6 +1014,7 @@ extern "C" int vglb_pagerank_ex(vglb_ctx *ctx, vglb_graph *g, int iters, float d
     CUDA_TRY(cudaEventRecord(ctx->ev_start, ctx->stream));
     CUDA_TRY(cudaMemsetAsync(g->d_pr_dangling, 0, (size_t)(iters + 1) * sizeof(double), ctx->stream));
     const float r0 = (float)(1.0 / (double)g->V_orig); // pr.hpp:42
+    P.r0 = r0;
     if (iters == 0)
     {
         if (V > 0)
@@ -980,6 +1047,7 @@ extern "C" int vglb_pagerank_ex(vglb_ctx *ctx, vglb_graph *g, int iters, float d
         P.contrib_out = g->d_pr_contrib[(it + 1) & 1] + col0;
         P.rank_out = (it == iters - 1 || ref_order) ? d_ranks : NULL; // reference order: the next dangling sum reads the ranks
         P.dangling_in = g->d_pr_dangling + it;
+        P.dangling_prev = it > 0 ? g->d_pr_dangling + it - 1 : NULL;
         P.dangling_out = g->d_pr_dangling + it + 1;
         P.npeers = 0;
         if (p2p && it < iters - 1)
@@ -997,14 +1065,9 @@ extern "C" int vglb_pagerank_ex(vglb_ctx *ctx, vglb_graph *g, int iters, float d
             KERNEL_TRY();
             ctx->launches++;
         }
-        rc = vglb_pr_launch_sweep(ctx, P, nblocks); // the rows with < 32 edges (all rows without the bins)
+        // the heavy rows' sums (all rows without the bins), the rows with < 32 edges and the rows without out-edges
+        rc = vglb_pr_launch_sweep(ctx, P, P.rank_out ? nblocks : nblocks_lean);
         if (rc != VGLB_OK) return rc;
-        if (g->pr_bins && P.bin_finish_blocks > 0)
-        {
-            pr_finish_kernel<<<(unsigned)P.bin_finish_blocks, PR_THREADS, 0, ctx->stream>>>(P);
-            KERNEL_TRY();
-            ctx->launches++;
-        }
         if (ref_order && it < iters - 1)
         {
             rc = reference_dangling(it + 1); // replaces the fp64 sum the sweep's epilogue accumulated

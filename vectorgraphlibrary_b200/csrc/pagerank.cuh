@@ -21,7 +21,7 @@
 #define PR_MIN_CTAS 5             // __launch_bounds__ minimum resident CTAs per SM (48 registers)
 #endif
 #ifndef PR_TAIL_MIN_CTAS
-#define PR_TAIL_MIN_CTAS 8        // the same for the sweep kernel without heavy blocks (32 registers)
+#define PR_TAIL_MIN_CTAS 8        // the same for pr_sweep_kernel<false>, whose heavy blocks only add up partial sums (32 registers)
 #endif
 #ifndef PR_VE_SEGS_PER_WARP
 #define PR_VE_SEGS_PER_WARP 8     // 32-row segments of the padded tail copy handled by one warp (r2 A/B with the column bins: 16 -> 0.611, 8 -> 0.527 ms)
@@ -89,8 +89,10 @@ struct PrbBinParams
     const uint32_t *meta;
     const int32_t *step_run0, *run_slot, *bin_chunk0, *cta_chunk0;
     const float *contrib_in;
+    const float *inv;
     float *slot;
     int32_t nb, cold_chunk0, nruns;
+    int32_t zero_col;  // the cold bin's PrParams::zero_kept (INT32_MAX in pr_bin_kernel)
     int64_t cols;      // columns of the gathered vector (sorted ids 0 .. cols-1)
     int32_t world, vp; // partitioned graph: column = owner * vp + local row, sorted id = local row * world + owner
     long long *cta_ns; // developer trace: time of every CTA (NULL = off)
@@ -116,7 +118,7 @@ struct PrParams
     float *piece_partial;
     int32_t *piece_count;          // one arrival counter per long row (row < tier_border[0])
     int32_t ntasks;
-    int32_t heavy_blocks;          // blocks [0, heavy_blocks) run warp tasks
+    int32_t heavy_blocks;          // blocks [0, heavy_blocks) run warp tasks, or with the column bins finish the heavy rows
     int32_t rows;                  // local rows
     int32_t col_of_row0;           // column id of local row 0 (0 on one GPU); row r is column col_of_row0 + r
     int32_t npeers;
@@ -130,12 +132,20 @@ struct PrParams
     int32_t ve_segments;
     int32_t tail_first, zero_first;
     int32_t tail_blocks;           // blocks [heavy_blocks, heavy_blocks + tail_blocks) run tail segments, the rest zero rows
-    // binned heavy rows (pagerank_bins.cu): there are no heavy blocks; pr_bin_kernel + pr_cold_bin_kernel leave partial sums,
-    // pr_finish_kernel adds up every heavy row's and runs its epilogue
+    // Rows without out-edges all get the same rank, rank0 = k + d * (0 + dangling). From zero_kept on (one GPU) their
+    // contributions are stored only by sweeps that store the ranks: the other sweeps launch no blocks for them, a gather of
+    // such a column computes rank0_prev * inv[v] (pr_zero_scale), and their share of the next dangling mass is
+    // zero_dangling (their rows with inv == 0) equal terms. zero_kept is INT32_MAX where every sweep stores them.
+    int32_t zero_kept;
+    int32_t zero_dangling;
+    const double *dangling_prev;   // the previous sweep's dangling_in, from which its rank0 follows (NULL on sweep 0)
+    float r0;                      // the rank pr_init_kernel's contributions are made of (sweep 0's rank0_prev)
+    // binned heavy rows (pagerank_bins.cu): pr_bin_kernel + pr_cold_bin_kernel leave partial sums, and the heavy blocks of
+    // pr_sweep_kernel<false> add up every heavy row's and run its epilogue (pr_finish_binned)
     const float *bin_slot;         // NULL: the heavy blocks run warp tasks
     const int32_t *bin_rc_ptr;
     int32_t bin_nc, bin_nch, bin_xc, bin_long_rows, bin_rows;
-    int32_t bin_long_blocks;       // pr_finish_kernel: blocks [0, bin_long_blocks): one warp per long row; then one lane per row
+    int32_t bin_long_blocks;       // heavy blocks [0, bin_long_blocks): one warp per long row; then one lane per row
     int32_t bin_finish_blocks;
     int32_t bin_cold_blocks;       // pr_cold_bin_kernel: one chunk of the cold bin per warp
     int32_t bin_nkchunks;          // all chunks of the binned copy; the cold bin's are bins.cold_chunk0 .. bin_nkchunks - 1
@@ -167,6 +177,15 @@ __device__ __forceinline__ uint4 prb_ld_v4u(const uint4 *p, uint64_t pol)
     return r;
 }
 
+// rank of every row without out-edges: pr_epilogue with sum = 0
+__device__ __forceinline__ float pr_zero_rank(float k, float d, float dang) { return __fadd_rn(k, __fmul_rn(d, __fadd_rn(0.f, dang))); }
+
+// A column at or above PrParams::zero_kept is a row without out-edges whose contribution the previous sweep did not store: the
+// gather loads inv[v] instead, and the value is z0 * inv[v], z0 being that sweep's rank0, which is the product it would have
+// stored. The multiply is applied where the gathered values are summed: next to the load it would wait for the load before the
+// next gather goes out.
+__device__ __forceinline__ float pr_zero_scale(bool zero, float z0, float x) { return zero ? __fmul_rn(z0, x) : x; }
+
 struct PrbStep
 {
     uint4 a, b;
@@ -176,7 +195,7 @@ struct PrbStep
 // the four 4-slot group sums of this lane's 16 slots
 template <bool COLD>
 __device__ __forceinline__ void prb_groups(const PrbBinParams &P, const L2Pol &pol, const float *sl, const PrbStep &cur, int64_t s, int lane,
-                                           float (&g)[4])
+                                           float z0, float (&g)[4])
 {
     if (!COLD)
     {
@@ -191,15 +210,27 @@ __device__ __forceinline__ void prb_groups(const PrbBinParams &P, const L2Pol &p
         int4 v[4];
 #pragma unroll
         for (int j = 0; j < 4; j++) v[j] = ld_stream_v4(c4 + j * 32, pol.stream);
+        float x[16];
+        unsigned zero = 0; // bit i: slot i is a column from zero_col on (pr_zero_scale)
 #pragma unroll
         for (int j = 0; j < 4; j++)
         {
-            const float x0 = v[j].x >= 0 ? ld_gather_cold_f32(P.contrib_in + v[j].x, pol.keep) : 0.f;
-            const float x1 = v[j].y >= 0 ? ld_gather_cold_f32(P.contrib_in + v[j].y, pol.keep) : 0.f;
-            const float x2 = v[j].z >= 0 ? ld_gather_cold_f32(P.contrib_in + v[j].z, pol.keep) : 0.f;
-            const float x3 = v[j].w >= 0 ? ld_gather_cold_f32(P.contrib_in + v[j].w, pol.keep) : 0.f;
-            g[j] = (x0 + x1) + (x2 + x3);
+            const int c[4] = {v[j].x, v[j].y, v[j].z, v[j].w};
+#pragma unroll
+            for (int i = 0; i < 4; i++)
+            {
+                x[4 * j + i] = 0.f; // (padding: -1)
+                if (c[i] >= 0)
+                {
+                    zero |= (c[i] >= P.zero_col ? 1u : 0u) << (4 * j + i);
+                    x[4 * j + i] = ld_gather_cold_f32((c[i] >= P.zero_col ? P.inv : P.contrib_in) + c[i], pol.keep);
+                }
+            }
         }
+#pragma unroll
+        for (int i = 0; i < 16; i++) x[i] = pr_zero_scale((zero >> i) & 1, z0, x[i]);
+#pragma unroll
+        for (int j = 0; j < 4; j++) g[j] = (x[4 * j] + x[4 * j + 1]) + (x[4 * j + 2] + x[4 * j + 3]);
     }
 }
 
@@ -230,7 +261,7 @@ __device__ __forceinline__ void prb_prefetch_l2(const void *p, uint32_t bytes)
 // stored one step later, with slot numbers fetched meanwhile (`stage` holds 2 x PRB_STAGE floats).
 template <bool COLD>
 __device__ __forceinline__ void prb_unit(const PrbBinParams &P, const L2Pol &pol, const float *sl, int s0, int s1, int bin_end_step, int lane,
-                                         float *stage)
+                                         float *stage, float z0)
 {
     const unsigned FULL = 0xffffffffu;
     const int r_first = P.step_run0[s0], r_end = P.step_run0[s1]; // runs that start here
@@ -261,7 +292,7 @@ __device__ __forceinline__ void prb_unit(const PrbBinParams &P, const L2Pol &pol
         const int sb = (lane + 32 < total && rb >= r_first && rb < r_end) ? __ldg(P.run_slot + rb) : -1;
         float *st = stage + (s & 1) * PRB_STAGE;
         float g[4] = {0.f, 0.f, 0.f, 0.f};
-        if (!beyond || !((m >> 17) & 1)) prb_groups<COLD>(P, pol, sl, cur, s, lane, g);
+        if (!beyond || !((m >> 17) & 1)) prb_groups<COLD>(P, pol, sl, cur, s, lane, z0, g);
         // in-lane pass: head = sum before the first start, tail = open run; the sums of the runs that close inside the lane are
         // staged in shared memory by their index within the step
         float run = 0.f, head = 0.f;

@@ -563,7 +563,7 @@ __global__ void __launch_bounds__(PRB_THREADS, 1) pr_bin_kernel(const __grid_con
             // every warp streams one contiguous piece of this CTA's steps of the bin
             const int64_t nst = (int64_t)(b_hi - b_lo) * PRB_SPC;
             const int s0 = b_lo * PRB_SPC + (int)(nst * warp / PRB_WARPS), s1 = b_lo * PRB_SPC + (int)(nst * (warp + 1) / PRB_WARPS);
-            if (s0 < s1) prb_unit<false>(P, pol, prb_smem, s0, s1, bin_end_step, lane, stage);
+            if (s0 < s1) prb_unit<false>(P, pol, prb_smem, s0, s1, bin_end_step, lane, stage, 0.f);
         }
     }
     if (P.cta_ns) // developer trace (VGLB_PR_BIN_TRACE)
@@ -589,6 +589,7 @@ void vglb_pr_bins_params(const vglb_graph *g, const float *contrib_in, PrbBinPar
     P->bin_chunk0 = B->d_bin_chunk0;
     P->cta_chunk0 = B->d_cta_chunk0;
     P->contrib_in = contrib_in;
+    P->inv = g->d_pr_inv;
     P->slot = B->d_slot;
     P->nb = B->nb;
     P->cold_chunk0 = B->cold_chunk0;
@@ -596,6 +597,7 @@ void vglb_pr_bins_params(const vglb_graph *g, const float *contrib_in, PrbBinPar
     P->world = g->comm ? g->part_world : 1;
     P->vp = g->vp;
     P->nruns = B->nruns;
+    P->zero_col = INT32_MAX;
     P->cta_ns = NULL;
 }
 
