@@ -241,8 +241,12 @@ int vglb_bfs_multi(vglb_ctx *ctx, vglb_graph *g, int32_t num_sources, const int3
 
 /* SSSP, frontier Bellman-Ford (algorithms/sssp/shortest_paths.hpp:7-78, gpu_shortest_paths.hpp:133-196): min-plus
  * fixed point in fp32 (bit-identical to the reference's seq_dijkstra), unreachable = FLT_MAX; d_weights indexed by
- * out-CSR position. The frontier is scheduled near/far around a moving distance threshold (fewer re-relaxations than the
- * reference's "everything that changed" schedule, same fixed point); stats->edges_inspected = edges actually relaxed. */
+ * out-CSR position. Weights must be non-negative (+0.0 and -0.0 included; a distance is never -0.0). +inf and NaN weights
+ * (either sign) are edges that never relax, as in seq_dijkstra; a sum that overflows to +inf leaves the distance as it was.
+ * Negative weights are outside the contract: candidates are ordered on their uint32 view, where a negative candidate sorts
+ * above every distance and is dropped. The frontier is scheduled near/far around a moving distance threshold (fewer
+ * re-relaxations than the reference's "everything that changed" schedule, same fixed point); stats->edges_inspected =
+ * edges actually relaxed. */
 int vglb_sssp(vglb_ctx *ctx, vglb_graph *g, const float *d_weights, int32_t source_sorted, float *d_dist,
               vglb_stats *stats);
 

@@ -20,6 +20,7 @@
 //     (ld.global.nc.L1::no_allocate + L2 evict-first), the distance vector is the L2-resident gather target.
 // HBM roofline: algorithmic bytes = sum_rounds [ 12 e_i (index + weight + dist[dst]) + 24 f_i + 8 n(F_{i+1}) ] + scans.
 #include <float.h>
+#include <math.h>
 #include <time.h>
 #include <stdlib.h>
 
@@ -1056,7 +1057,11 @@ static int sssp_run(vglb_ctx *ctx, vglb_graph *g, const float *d_weights, int32_
             const uint32_t min_bits = 0xffffffffu - (uint32_t)(part ? h_cnt[2 * C_COUNT] : h_cnt[C_MF]);
             float min_pending;
             memcpy(&min_pending, &min_bits, 4);
-            threshold = fmaxf(threshold, min_pending) + delta; // nothing below the moved threshold: jump
+            // nothing below the moved threshold: jump. The far select takes d < threshold, so the new threshold must lie
+            // strictly above min_pending; a delta below half an ulp of min_pending rounds away in the sum (a sampled
+            // w_max that missed the heavy edges, a tiny VGLB_SSSP_DELTA_SCALE), and the same empty select would repeat
+            const float jumped = fmaxf(threshold, min_pending) + delta;
+            threshold = jumped > min_pending ? jumped : nextafterf(min_pending, INFINITY);
             continue;
         }
         from_far = false;
