@@ -6,8 +6,7 @@
 //   * include/vgl_b200/overlay/vgl_compute_api/gpu/graph_abstractions_gpu.h — the drop-in backend the reference's own
 //     algorithms compile against, unchanged, and
 //   * include/vgl_b200/graph_abstractions_b200.cuh — the stand-alone operator API over C-ABI objects,
-// while the data structures, compaction and the fused algorithms live behind the C ABI. libvgl_b200 itself instantiates
-// them for CC (cc.cu, VGLB_CC_GENERIC).
+// while the data structures, compaction and the fused algorithms live behind the C ABI.
 //
 // Functor contracts = the reference's (architecture_independent_api.h:17-30):
 //   edge_op  (int src_id, int dst_id, int local_edge_pos, long long global_edge_pos, int vector_index)

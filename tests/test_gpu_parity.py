@@ -256,10 +256,6 @@ def test_hubs_and_long_chain(vgl, ctx, oracle, monkeypatch):
         monkeypatch.delenv("VGLB_SSSP_DELTA_SCALE")
     lab, _ = G.cc()
     assert np.array_equal(G.to_original(lab), og.cc()[0])
-    monkeypatch.setenv("VGLB_CC_GENERIC", "1")  # the hook through the lambda-generic advance template: same labels
-    lab2, _ = G.cc()
-    assert np.array_equal(lab2.to_numpy(), lab.to_numpy())
-    monkeypatch.delenv("VGLB_CC_GENERIC")
     ranks, _ = G.pagerank(20)
     assert O.rel_l1(G.to_original(ranks), og.pagerank_f64(20)) <= PR_TOL
     G.free()

@@ -49,7 +49,6 @@ static double trace_now()
 struct PartArgs
 {
     int32_t col0, vp, P, rank;
-    int32_t visited_via_l2; // developer A/B knob (VGLB_BFS_VISITED_L2): test the visited bitmap with L2 (.cg) loads instead of L1-cached ones
     unsigned long long *lists; // P counters, then vp 4-byte entries per owner starting at byte offset 8 * P
 };
 
@@ -101,7 +100,7 @@ __device__ __forceinline__ void td_expand(const int64_t *__restrict__ ptr, const
         // (L1-cached: a stale "unvisited" only costs an atomic that cannot win, while the hubs' words — most of the edges of a big
         // level point at them — are answered by L1 instead of L2: top-down-only Kronecker s26 22.3 -> 8.6 ms, RMAT s20 0.75 -> 0.46 ms)
         for (int k = 0; k < BFS_TD_UNROLL; k++)
-            seen[k] = v[k] >= 0 ? (A.visited_via_l2 ? __ldcg(&visited[v[k] >> 5]) : visited[v[k] >> 5]) : 0xffffffffu;
+            seen[k] = v[k] >= 0 ? visited[v[k] >> 5] : 0xffffffffu;
 #pragma unroll
         for (int k = 0; k < BFS_TD_UNROLL; k++)
         {
@@ -1116,12 +1115,8 @@ extern "C" int vglb_bfs(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t *d
         int rc_in = vglb_graph_derive_incoming(ctx, g);
         if (rc_in != VGLB_OK) return rc_in;
     }
-    long long alpha = (opts && opts->alpha > 0) ? opts->alpha : BFS_DEFAULT_ALPHA;
-    long long beta = (opts && opts->beta > 0) ? opts->beta : BFS_DEFAULT_BETA;
-    if (!(opts && opts->alpha > 0) && getenv("VGLB_BFS_ALPHA")) alpha = atoll(getenv("VGLB_BFS_ALPHA")); // developer knobs (A/B runs)
-    if (!(opts && opts->beta > 0) && getenv("VGLB_BFS_BETA")) beta = atoll(getenv("VGLB_BFS_BETA"));
-    if (alpha < 1) alpha = 1;
-    if (beta < 1) beta = 1;
+    const long long alpha = (opts && opts->alpha > 0) ? opts->alpha : BFS_DEFAULT_ALPHA;
+    const long long beta = (opts && opts->beta > 0) ? opts->beta : BFS_DEFAULT_BETA;
     CUDA_TRY(cudaSetDevice(ctx->device));
     int rc = bfs_prepare(ctx, g);
     if (rc != VGLB_OK) return rc;
@@ -1178,13 +1173,11 @@ extern "C" int vglb_bfs(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t *d
         trace_t = trace_now();
     }
 
-    const int visited_l2 = getenv("VGLB_BFS_VISITED_L2") != NULL; // developer knob
     long long m_f_cur = 0; // out-edges of the current frontier (accumulated by the level that produced it; unknown for the source)
-    const long long bitmap_out_edges = getenv("VGLB_BFS_NO_BITMAP_OUT") ? (1LL << 62) : (1LL << 20); // developer knob
     while (n_cur > 0)
     {
         // a top-down level that is about to inspect more than a million edges emits its discoveries as a bitmap
-        const bool bitmap_out = !bottom_up && m_f_cur > bitmap_out_edges;
+        const bool bitmap_out = !bottom_up && m_f_cur > (1LL << 20);
         if (!bottom_up)
         {
             const int blocks_mid = (int)min((int64_t)max_blocks, ceil_div64(n[1], BFS_THREADS / 32));
@@ -1195,7 +1188,6 @@ extern "C" int vglb_bfs(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t *d
             {
                 PartArgs out;
                 memset(&out, 0, sizeof(out));
-                out.visited_via_l2 = visited_l2;
                 out.lists = reinterpret_cast<unsigned long long *>(next_bm);
                 CUDA_TRY(cudaMemsetAsync(next_bm, 0, words * 4, st));
                 bfs_td_kernel<3><<<(unsigned)grid, BFS_THREADS, 0, st>>>(g->d_out_ptr, g->d_out_adj, cq, n[0], hub_ctas, n[1], n[2], blocks_mid,
@@ -1206,7 +1198,6 @@ extern "C" int vglb_bfs(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t *d
             {
                 PartArgs none;
                 memset(&none, 0, sizeof(none));
-                none.visited_via_l2 = visited_l2;
                 bfs_td_kernel<0><<<(unsigned)grid, BFS_THREADS, 0, st>>>(g->d_out_ptr, g->d_out_adj, cq, n[0], hub_ctas, n[1], n[2], blocks_mid,
                                                                        blocks_small, g->d_visited, d_levels, level + 1, b0, b1, nq, d_cnt, none);
             }

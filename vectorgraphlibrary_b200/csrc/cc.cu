@@ -9,26 +9,24 @@
 // symmetric graphs, so any schedule of monotone hooks and jumps reaches bit-identical labels.
 //
 // B200 design: the hook is an all-active advance with an atomicMin edge op, one launch covering all degree tiers —
-// cc_hook_kernel below (load-balanced, several independent gathers per lane), or with VGLB_CC_GENERIC=1 the
-// lambda-generic template of include/vgl_b200/advance.cuh that the GraphAbstractionsB200 shim instantiates for user
-// lambdas (same labels, a third of the edge rate); hooks are applied in place, so a label travels many hops within one round (Gauss-Seidel), and the
-// whole jump loop of the reference collapses into ONE kernel that chases every vertex to its current root
-// (comp[x] <= x always holds, so the chase terminates and concurrent writes only shorten it). The convergence flag is
-// a device word read back once per round (the reference returns a reduce<int> to the host per round, :47-52).
+// cc_hook_kernel below (load-balanced, several independent gathers per lane); hooks are applied in place, so a label
+// travels many hops within one round (Gauss-Seidel), and the whole jump loop of the reference collapses into ONE kernel
+// that chases every vertex to its current root (comp[x] <= x always holds, so the chase terminates and concurrent writes
+// only shorten it). The convergence flag is a device word read back once per round (the reference returns a reduce<int> to
+// the host per round, :47-52).
 // HBM roofline: algorithmic bytes = sum_hook [ 8E + 12V ] + sum_jump 8V (SURVEY §8d).
 #include <limits.h>
-#include <stdlib.h>
 
 #include "common.cuh"
-#include "vgl_b200/advance.cuh"
 
 
 // ---- the hook as a load-balanced all-active advance specialised for min-label propagation ---------------------------
-// Same edge op as CcHookOp below (shiloach_vishkin.hpp:38-46), but scheduled for memory-level parallelism: the generic
-// per-row advance issues one dependent chain (index -> label -> atomic) per lane and step and reaches a third of the
-// PageRank sweep's edge rate. Here rows with >= 4096 edges get one CTA per CC_BIG_CHUNK edges, and a warp takes 32
-// consecutive smaller rows and walks the concatenation of their edge ranges (shuffle search over the degree prefix
-// sums, as in sssp.cu), CC_UNROLL edges per lane: the index loads, then the label gathers, are independent.
+// The edge op of shiloach_vishkin.hpp:38-46, scheduled for memory-level parallelism: the lambda-generic per-row advance
+// that the GraphAbstractionsB200 shim instantiates for user lambdas (include/vgl_b200/advance.cuh) issues one dependent
+// chain (index -> label -> atomic) per lane and step and reaches a third of the PageRank sweep's edge rate. Here rows with
+// >= 4096 edges get one CTA per CC_BIG_CHUNK edges, and a warp takes 32 consecutive smaller rows and walks the
+// concatenation of their edge ranges (shuffle search over the degree prefix sums, as in sssp.cu), CC_UNROLL edges per lane:
+// the index loads, then the label gathers, are independent.
 #define CC_THREADS 256
 #define CC_UNROLL 4
 #define CC_BIG_CHUNK 8192
@@ -175,22 +173,6 @@ static int cc_launch_hook(vglb_ctx *ctx, const vglb_graph *g, int32_t *comp, int
     return VGLB_OK;
 }
 
-// the same hook as a functor of the lambda-generic advance (include/vgl_b200/advance.cuh); VGLB_CC_GENERIC=1 routes the
-// hook through that template — the path an unmodified VGL algorithm source takes through the GraphAbstractionsB200 shim
-struct CcHookOp
-{
-    int32_t *comp;
-    int *changed;
-    __device__ __forceinline__ void operator()(int src, int dst, int, long long, int) const
-    {
-        const int32_t cs = comp[src];
-        if (cs < comp[dst])                       // shiloach_vishkin.hpp:38-46
-        {
-            if (atomicMin(&comp[dst], cs) > cs) *changed = 1;
-        }
-    }
-};
-
 __global__ void cc_init_kernel(int32_t *__restrict__ comp, int32_t V)
 {
     for (int32_t v = blockIdx.x * blockDim.x + threadIdx.x; v < V; v += gridDim.x * blockDim.x) comp[v] = v;
@@ -309,23 +291,6 @@ extern "C" int vglb_cc(vglb_ctx *ctx, vglb_graph *g, int32_t *d_labels, vglb_sta
     int *d_changed = (int *)(ctx->d_counters + 40);
     int *h_changed = (int *)(ctx->h_counters + 40);
 
-    vglb::CsrView view;
-    view.ptr = g->d_out_ptr;
-    view.adj = g->d_out_adj;
-    view.V = V;
-    for (int t = 0; t < VGLB_NUM_TIERS; t++) view.tier_border[t] = g->tier_border[t];
-    view.max_degree = g->max_degree;
-    const bool generic = getenv("VGLB_CC_GENERIC") != NULL;
-    int64_t hub_edges = 0; // edges of the rows with >= 4096 edges = row pointer at the first tier border
-    if (generic && g->tier_border[0] > 0)
-    {
-        CUDA_TRY(cudaMemcpyAsync(&hub_edges, g->d_out_ptr + g->tier_border[0], 8, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
-    }
-    const vglb::AllActivePlan plan = vglb::plan_all_active<vglb::NoVertexOp, vglb::NoVertexOp>(view, g->E, hub_edges);
-    VGLB_REQUIRE(plan.blocks < 0x7fffffffLL, "vglb_cc: grid too large");
-    CcHookOp hook{d_labels, d_changed};
-    vglb::NoVertexOp none;
 
     CUDA_TRY(cudaEventRecord(ctx->ev_start, st));
     cc_init_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(d_labels, V);
@@ -335,20 +300,8 @@ extern "C" int vglb_cc(vglb_ctx *ctx, vglb_graph *g, int32_t *d_labels, vglb_sta
     for (;;)
     {
         CUDA_TRY(cudaMemsetAsync(d_changed, 0, sizeof(int), st));
-        if (generic)
-        {
-            if (plan.blocks > 0)
-            {
-                vglb::advance_all_active_kernel<<<(unsigned)plan.blocks, vglb::kAdvThreads, 0, st>>>(view, plan, 0LL, hook, none, none);
-                KERNEL_TRY();
-                ctx->launches++;
-            }
-        }
-        else
-        {
-            int rc = cc_launch_hook(ctx, g, d_labels, 0, d_changed);
-            if (rc != VGLB_OK) return rc;
-        }
+        int rc = cc_launch_hook(ctx, g, d_labels, 0, d_changed);
+        if (rc != VGLB_OK) return rc;
         hook_rounds++;
         CUDA_TRY(cudaMemcpyAsync(h_changed, d_changed, sizeof(int), cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));

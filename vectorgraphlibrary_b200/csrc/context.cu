@@ -231,14 +231,6 @@ __global__ void counters_publish_kernel(const unsigned long long *__restrict__ s
 int vglb_counters_fetch(vglb_ctx *ctx, const void *d_src, int words)
 {
     VGLB_REQUIRE(words > 0 && words <= 56, "vglb_counters_fetch: at most 56 counters");
-    static int use_mailbox = -1;
-    if (use_mailbox < 0) use_mailbox = getenv("VGLB_NO_MAILBOX") ? 0 : 1; // developer knob: plain memcpy + stream sync
-    if (!use_mailbox)
-    {
-        CUDA_TRY(cudaMemcpyAsync(ctx->h_counters, d_src, (size_t)words * 8, cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-        return VGLB_OK;
-    }
     const unsigned long long seq = ++ctx->mailbox_seq;
     counters_publish_kernel<<<1, 64, 0, ctx->stream>>>((const unsigned long long *)d_src, words, ctx->h_mailbox, seq);
     KERNEL_TRY();

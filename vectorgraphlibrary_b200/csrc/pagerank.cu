@@ -376,15 +376,11 @@ __global__ void __launch_bounds__(PR_THREADS, HEAVY ? PR_MIN_CTAS : PR_TAIL_MIN_
     pol.stream = l2_policy_evict_first();
     pol.keep = l2_policy_evict_last();
     __shared__ double s_dang[PR_WARPS];
-    int b = blockIdx.x;
-    if (P.interleave)
-    {
-        // the tail tiers are latency-bound, the heavy region is throughput-bound: mix their blocks so that both kinds
-        // are resident on every SM at any time. Block m is a tail block whenever floor((m+1)*ntail/M) advances.
-        const long long ntail = (long long)gridDim.x - P.heavy_blocks, M = gridDim.x, m = b;
-        const long long tails_before = m * ntail / M, tails_after = (m + 1) * ntail / M;
-        b = tails_after > tails_before ? (int)(P.heavy_blocks + tails_before) : (int)(m - tails_before);
-    }
+    // the tail tiers are latency-bound, the heavy region is throughput-bound: mix their blocks so that both kinds are resident on
+    // every SM at any time. Block m is a tail block whenever floor((m+1)*ntail/M) advances.
+    const long long ntail = (long long)gridDim.x - P.heavy_blocks, M = gridDim.x, m = blockIdx.x;
+    const long long tails_before = m * ntail / M, tails_after = (m + 1) * ntail / M;
+    const int b = tails_after > tails_before ? (int)(P.heavy_blocks + tails_before) : (int)(m - tails_before);
     const float dang = (float)(*P.dangling_in);
     double dang_local = 0.0;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -864,18 +860,7 @@ int64_t vglb_pr_plan(const vglb_graph *g, int32_t rows, PrParams *P)
     P->tail_first = g->tier_border[1];
     P->zero_first = g->tier_border[VGLB_NUM_TIERS - 2];
     P->tail_blocks = (int32_t)ceil_div64(g->pr_ve_segments, PR_WARPS * PR_VE_SEGS_PER_WARP);
-    int64_t nblocks = (int64_t)P->heavy_blocks + P->tail_blocks + ceil_div64(rows - P->zero_first, PR_ZERO_ROWS_PER_CTA);
-    // developer knob for timing experiments (results are wrong when set): 1 = heavy region only, 2 = tail tiers only
-    if (const char *m = getenv("VGLB_PR_ONLY"))
-    {
-        if (atoi(m) == 1) nblocks = P->heavy_blocks;
-        if (atoi(m) == 2) P->ntasks = 0;
-        if (atoi(m) == 3) { P->ntasks = 0; P->ve_segments = 0; }
-    }
-    P->interleave = 1;
-    if (const char *m = getenv("VGLB_PR_INTERLEAVE")) P->interleave = atoi(m);
-    if (getenv("VGLB_PR_ONLY")) P->interleave = 0;
-    return nblocks;
+    return (int64_t)P->heavy_blocks + P->tail_blocks + ceil_div64(rows - P->zero_first, PR_ZERO_ROWS_PER_CTA);
 }
 
 // Shared-memory carve-outs of the sweep's kernels (a function attribute is per device: remembered per context, not per process).
@@ -985,9 +970,8 @@ extern "C" int vglb_pagerank_ex(vglb_ctx *ctx, vglb_graph *g, int iters, float d
     // them into the peers' vectors (then the dangling-mass allreduce is also the barrier between sweeps: a rank starts
     // sweep i+1 only after every peer finished sweep i, i.e. finished both reading buffer i and writing buffer i+1)
     const bool p2p = comm && g->pr_exchange == VGLB_EXCHANGE_P2P;
-    const bool no_exchange = getenv("VGLB_PR_NO_EXCHANGE") != NULL; // developer knob: time one rank's sweeps alone (results are wrong)
     auto exchange = [&](float *vec, double *dangling, bool stored_by_peers) -> int {
-        if (!comm || no_exchange) return VGLB_OK;
+        if (!comm) return VGLB_OK;
         if (!stored_by_peers)
         {
             int rc = vglb_comm_allgather_async(comm, vec, (size_t)g->vp * 4);

@@ -56,8 +56,7 @@ struct vglb_graph;
 // ---- column-binned heavy rows (pagerank_bins.cu) --------------------------------------------------------------------------
 #define PRB_H 49152     // columns per bin: its slice of the contribution vector fills 192 KB of shared memory
 #define PRB_RC 4096     // a row's edges are cut into chunks of this many before binning: no (bin,row) run is longer
-#define PRB_MIN_BINS 32  // shared-memory bins used (columns beyond them form the cold bin)
-#define PRB_MAX_BINS 128 // what the VGLB_PR_BINS developer knob may ask for
+#define PRB_BINS 32     // shared-memory bins used (columns beyond them form the cold bin)
 
 struct PrBins
 {
@@ -71,7 +70,6 @@ struct PrBins
     int64_t slots;
     int32_t nruns;
     int grid;            // persistent CTAs (one per SM)
-    int traced;          // VGLB_PR_BIN_TRACE printed this graph's per-CTA times
     uint16_t *d_wcol;    // column - bin * PRB_H of every slot of the shared-memory bins (PRB_H = padding)
     int32_t *d_cold;     // column of every slot of the cold bin (-1 = padding)
     uint32_t *d_meta;    // per lane and step: static part of the segmented sum
@@ -95,7 +93,6 @@ struct PrbBinParams
     int32_t zero_col;  // the cold bin's PrParams::zero_kept (INT32_MAX in pr_bin_kernel)
     int64_t cols;      // columns of the gathered vector (sorted ids 0 .. cols-1)
     int32_t world, vp; // partitioned graph: column = owner * vp + local row, sorted id = local row * world + owner
-    long long *cta_ns; // developer trace: time of every CTA (NULL = off)
 };
 
 int vglb_pr_bins_build(vglb_ctx *ctx, vglb_graph *g);
@@ -122,10 +119,9 @@ struct PrParams
     int32_t rows;                  // local rows
     int32_t col_of_row0;           // column id of local row 0 (0 on one GPU); row r is column col_of_row0 + r
     int32_t npeers;
-    int32_t interleave;            // mix heavy and tail blocks in the grid
+    uint32_t cold_local;           // gathers of local rows at or above this bypass L1 (PR_COLD_ID / ranks)
     float k, d, v_as_float;
     uint32_t vp, vp_mask;          // partitioned graphs: rows per rank (slice stride) and vp - 1 when vp is a power of two
-    uint32_t cold_local;           // gathers of local rows at or above this bypass L1 (PR_COLD_ID / ranks)
     // tail: rows [tail_first, zero_first) have degree 1..31 and are read from the padded column-major copy
     const int32_t *ve_adj;         // segment s: ve_adj[ve_ptr[s] + j*32 + lane] = j-th neighbour of row tail_first + 32 s + lane
     const int64_t *ve_ptr;         // ve_segments + 1 offsets
@@ -164,9 +160,6 @@ struct L2Pol
 #define PRB_SPC (PRB_CHUNK / PRB_STEP)  // steps per chunk
 #define PRB_ALIGN 4                     // runs start at multiples of this many slots
 #define PRB_STAGE 128                   // a step closes at most PRB_STEP / PRB_ALIGN runs
-#ifndef PRB_L2_AHEAD
-#define PRB_L2_AHEAD 0                   // steps ahead whose columns and metadata are pulled into L2 by a bulk prefetch (0 = off; A/B at RMAT-24: 0 -> 0.529, 3 -> 0.545, 6 -> 0.548, 12 -> 0.574 ms per sweep)
-#endif
 
 __device__ __forceinline__ uint4 prb_ld_v4u(const uint4 *p, uint64_t pol)
 {
@@ -249,12 +242,6 @@ __device__ __forceinline__ PrbStep prb_load_step(const PrbBinParams &P, const L2
     return d;
 }
 
-// pull `bytes` (a multiple of 16, 16-byte aligned) into L2 ahead of the loads that will want them
-__device__ __forceinline__ void prb_prefetch_l2(const void *p, uint32_t bytes)
-{
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory");
-}
-
 // One unit = the steps [s0, s1) of one bin: emits the sums of the runs that START in it. The warp ignores the leading part of a
 // run that started earlier and runs on past s1 until the next start (in those steps only the lanes up to the first start
 // gather). Latency: the unit is a stream — columns and metadata are fetched two steps ahead, and the sums a step closes are
@@ -279,14 +266,6 @@ __device__ __forceinline__ void prb_unit(const PrbBinParams &P, const L2Pol &pol
         const bool ahead2 = s + 2 <= s1 || (beyond && total == 0);
         PrbStep nx2 = nxt;
         if (ahead2 && s + 2 < bin_end_step) nx2 = prb_load_step(P, pol, s + 2, lane, COLD);
-        if (PRB_L2_AHEAD > 0 && s + PRB_L2_AHEAD < min(s1 + 1, bin_end_step))
-        {
-            // (the register prefetch above then meets L2 instead of DRAM latency)
-            const int64_t sp = s + PRB_L2_AHEAD;
-            if (!COLD && lane == 0) prb_prefetch_l2(P.wcol + sp * PRB_STEP, PRB_STEP * 2);
-            if (COLD && lane == 0) prb_prefetch_l2(P.cold + (sp - (int64_t)P.cold_chunk0 * PRB_SPC) * PRB_STEP, PRB_STEP * 4);
-            if (lane == 1) prb_prefetch_l2(P.meta + sp * 32, 128);
-        }
         const int ra = run0 + lane - 1, rb = ra + 32;
         const int sa = (lane < total && ra >= r_first && ra < r_end) ? __ldg(P.run_slot + ra) : -1;
         const int sb = (lane + 32 < total && rb >= r_first && rb < r_end) ? __ldg(P.run_slot + rb) : -1;

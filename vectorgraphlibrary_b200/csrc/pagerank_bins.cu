@@ -16,10 +16,7 @@
 // Persistent kernel: one CTA of 32 warps per SM walks a contiguous, cost-balanced range of 4096-slot chunks; the warp that owns
 // a chunk emits the runs that START in it (it runs on past the end of the chunk until the next start). No atomics, fixed
 // summation order.
-#include <stdio.h>
 #include <stdlib.h>
-
-#include <vector>
 
 #include <cub/device/device_scan.cuh>
 
@@ -29,7 +26,6 @@
 #define PRB_THREADS 1024
 #define PRB_WARPS (PRB_THREADS / 32)
 #define PRB_DROP 0xff                   // class of a self loop: not part of the sum (pr.hpp:112)
-#define PRB_MAX_CLASSES (PRB_MAX_BINS + 8)
 #define PRB_SMEM_BYTES ((PRB_H + 4) * 4 + PRB_WARPS * 2 * PRB_STAGE * 4)
 
 // meta word of one lane and step:
@@ -103,7 +99,7 @@ __global__ void __launch_bounds__(256) prb_scatter_kernel(const int64_t *__restr
                                                            const int64_t *__restrict__ run_pos, int64_t w_smem, uint16_t *__restrict__ wcol,
                                                            int32_t *__restrict__ cold)
 {
-    __shared__ long long s_acc[8][PRB_MAX_CLASSES];
+    __shared__ long long s_acc[8][PRB_BINS + 1];
     const unsigned FULL = 0xffffffffu;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nc = nb + 1;
     const int32_t ci = blockIdx.x * 8 + warp;
@@ -212,40 +208,6 @@ __global__ void prb_run_pos_kernel(const int64_t *__restrict__ pos_scan, const i
     if (i >= n) return;
     const int c = (int)(i / nch);
     run_pos[i] = bin_start[c] + (pos_scan[i] - pos_scan[(int64_t)c * nch]);
-}
-
-// Shared-memory bank conflicts: a warp's e-th gather reads slot e of every lane. Inside a run the order of the slots is free, so
-// every lane sorts the slots of each run piece it holds by (column - lane) mod 32: its e-th slot then sits near bank lane + 2 e,
-// a different bank for every lane. Measured: wavefronts per gather instruction 4.4 -> 2.9, time per sweep unchanged (the kernel
-// is not bound by the shared-memory pipe), so the pass is off unless VGLB_PR_BANK_SORT is set.
-__global__ void prb_sort_lanes_kernel(uint4 *__restrict__ wcol8, const uint32_t *__restrict__ meta, int64_t nsteps)
-{
-    const int lane = threadIdx.x & 31;
-    const int64_t s = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (s >= nsteps) return;
-    const uint4 a = wcol8[s * 64 + lane], b = wcol8[s * 64 + 32 + lane];
-    const uint32_t fl = meta[s * 32 + lane] & 15u;
-    uint32_t c[16] = {a.x & 0xffff, a.x >> 16, a.y & 0xffff, a.y >> 16, a.z & 0xffff, a.z >> 16, a.w & 0xffff, a.w >> 16,
-                      b.x & 0xffff, b.x >> 16, b.y & 0xffff, b.y >> 16, b.z & 0xffff, b.z >> 16, b.w & 0xffff, b.w >> 16};
-#pragma unroll
-    for (int phase = 0; phase < 16; phase++)
-    {
-#pragma unroll
-        for (int i = phase & 1; i + 1 < 16; i += 2)
-        {
-            // slots i and i + 1 belong to the same run unless a run starts at slot i + 1
-            const bool same = ((i + 1) & 3) != 0 || !((fl >> ((i + 1) >> 2)) & 1);
-            const uint32_t ki = (c[i] - lane) & 31u, kj = (c[i + 1] - lane) & 31u;
-            if (same && ki > kj)
-            {
-                const uint32_t t = c[i];
-                c[i] = c[i + 1];
-                c[i + 1] = t;
-            }
-        }
-    }
-    wcol8[s * 64 + lane] = make_uint4(c[0] | (c[1] << 16), c[2] | (c[3] << 16), c[4] | (c[5] << 16), c[6] | (c[7] << 16));
-    wcol8[s * 64 + 32 + lane] = make_uint4(c[8] | (c[9] << 16), c[10] | (c[11] << 16), c[12] | (c[13] << 16), c[14] | (c[15] << 16));
 }
 
 // one warp per step: the static part of the segmented sum
@@ -392,10 +354,7 @@ int vglb_pr_bins_build_rows(vglb_ctx *ctx, vglb_graph *g, int32_t rows)
     // 32 bins = the hottest 9.4 % of the columns of the BASELINE graph = 91 % of the gathers of its heavy rows. Every further bin
     // costs the finish pass one more partial sum per heavy row: 64 bins are no faster there, and on 4 GPUs (scale 26: 32 bins hold
     // 74 % of the gathers) 32 / 64 / 128 bins gave 1034 / 1075 / 939 GTEPS against 1108 with the warp tasks.
-    int64_t want = PRB_MIN_BINS;
-    if (const char *e = getenv("VGLB_PR_BINS")) want = atoi(e); // developer knob
-    want = std::max<int64_t>(1, std::min<int64_t>(PRB_MAX_BINS, want));
-    const int nb = (int)std::min<int64_t>(want, ceil_div64(ncols, PRB_H));
+    const int nb = (int)std::min<int64_t>(PRB_BINS, ceil_div64(ncols, PRB_H));
     const int nc = nb + 1;
 
     PrBins *B = (PrBins *)calloc(1, sizeof(PrBins));
@@ -487,12 +446,6 @@ int vglb_pr_bins_build_rows(vglb_ctx *ctx, vglb_graph *g, int32_t rows)
     prb_runs_kernel<<<(unsigned)ceil_div64(n + nc, 256), 256, 0, st>>>(d_cnt, d_run_pos, d_pos_scan, d_flag_scan, d_bin_start, nch, nc,
                                                                       B->d_meta, B->d_run_slot);
     PRB_CUDA(cudaGetLastError());
-    if (w_smem > 0 && getenv("VGLB_PR_BANK_SORT")) // (developer A/B knob; off: 0.35 ms of the build and no faster sweeps)
-    {
-        const int64_t steps_smem = w_smem / PRB_STEP;
-        prb_sort_lanes_kernel<<<(unsigned)ceil_div64(steps_smem * 32, 256), 256, 0, st>>>(reinterpret_cast<uint4 *>(B->d_wcol), B->d_meta, steps_smem);
-        PRB_CUDA(cudaGetLastError());
-    }
     PRB_CUDA(vglb_dev_alloc(&d_step_total, ((size_t)nsteps + 1) * 4));
     prb_meta_kernel<<<(unsigned)ceil_div64(nsteps * 32, 256), 256, 0, st>>>(B->d_meta, nsteps, d_step_total);
     PRB_CUDA(cudaGetLastError());
@@ -526,8 +479,6 @@ __global__ void __launch_bounds__(PRB_THREADS, 1) pr_bin_kernel(const __grid_con
     pol.keep = l2_policy_evict_last();
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int k_lo = P.cta_chunk0[blockIdx.x], k_hi = P.cta_chunk0[blockIdx.x + 1];
-    long long t_begin = 0;
-    if (P.cta_ns && threadIdx.x == 0) asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t_begin));
     float *stage = prb_smem + PRB_H + 4 + warp * 2 * PRB_STAGE;
     const int nc = P.nb; // (the cold bin's chunks are blocks of pr_sweep_kernel: they need the L1 this kernel gives to shared memory)
     int bin = 0;
@@ -566,16 +517,6 @@ __global__ void __launch_bounds__(PRB_THREADS, 1) pr_bin_kernel(const __grid_con
             if (s0 < s1) prb_unit<false>(P, pol, prb_smem, s0, s1, bin_end_step, lane, stage, 0.f);
         }
     }
-    if (P.cta_ns) // developer trace (VGLB_PR_BIN_TRACE)
-    {
-        __syncthreads();
-        if (threadIdx.x == 0)
-        {
-            long long t_end;
-            asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t_end));
-            P.cta_ns[blockIdx.x] = t_end - t_begin;
-        }
-    }
 }
 
 void vglb_pr_bins_params(const vglb_graph *g, const float *contrib_in, PrbBinParams *P)
@@ -598,7 +539,6 @@ void vglb_pr_bins_params(const vglb_graph *g, const float *contrib_in, PrbBinPar
     P->vp = g->vp;
     P->nruns = B->nruns;
     P->zero_col = INT32_MAX;
-    P->cta_ns = NULL;
 }
 
 int vglb_pr_bins_launch(vglb_ctx *ctx, vglb_graph *g, const float *contrib_in)
@@ -612,33 +552,8 @@ int vglb_pr_bins_launch(vglb_ctx *ctx, vglb_graph *g, const float *contrib_in)
     }
     PrbBinParams P;
     vglb_pr_bins_params(g, contrib_in, &P);
-    long long *d_ns = NULL;
-    if (!B->traced && getenv("VGLB_PR_BIN_TRACE") && g->V > (1 << 20))
-    {
-        CUDA_TRY(vglb_dev_alloc(&d_ns, (size_t)B->grid * 8));
-        P.cta_ns = d_ns;
-    }
     pr_bin_kernel<<<B->grid, PRB_THREADS, PRB_SMEM_BYTES, ctx->stream>>>(P);
     KERNEL_TRY();
     ctx->launches++;
-    if (d_ns)
-    {
-        B->traced = 1;
-        std::vector<long long> ns((size_t)B->grid);
-        std::vector<int32_t> c0((size_t)B->grid + 1), b0((size_t)B->nb + 2);
-        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-        CUDA_TRY(cudaMemcpy(ns.data(), d_ns, ns.size() * 8, cudaMemcpyDeviceToHost));
-        CUDA_TRY(cudaMemcpy(c0.data(), B->d_cta_chunk0, c0.size() * 4, cudaMemcpyDeviceToHost));
-        CUDA_TRY(cudaMemcpy(b0.data(), B->d_bin_chunk0, b0.size() * 4, cudaMemcpyDeviceToHost));
-        vglb_dev_free(d_ns);
-        fprintf(stderr, "pr bins: %d bins + cold, %d chunks (cold from %d), rows %d (long %d), row chunks %d\n", B->nb, B->nkchunks, B->cold_chunk0,
-                B->rows, B->long_rows, B->nch);
-        for (int b = 0; b < B->grid; b++)
-        {
-            int bin = 0;
-            while (bin < B->nb + 1 && b0[bin + 1] <= c0[b]) bin++;
-            fprintf(stderr, "pr bins: CTA %3d chunks [%6d, %6d) first bin %2d: %7.1f us\n", b, c0[b], c0[b + 1], bin, ns[b] * 1e-3);
-        }
-    }
     return VGLB_OK;
 }

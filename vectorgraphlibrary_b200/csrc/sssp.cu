@@ -247,63 +247,26 @@ static int sssp_partitioned_dense(vglb_ctx *ctx, vglb_graph *g, const float *d_w
 #ifndef SSSP_FLAT_UNROLL
 #define SSSP_FLAT_UNROLL 4
 #endif
-// the gathered distance: kept in L2 ahead of the streamed adjacency / weights (evict-last hint), or a plain load
-#ifndef SSSP_GATHER_KEEP
-#define SSSP_GATHER_KEEP 1
-#endif
-#if SSSP_GATHER_KEEP
-#define SSSP_GATHER(p) sssp_ld_keep((p), pol_keep)
-#else
-#define SSSP_GATHER(p) (*(p))
-#endif
+// the gathered distance: kept in L2 ahead of the streamed adjacency / weights (evict-last hint)
 __device__ __forceinline__ uint32_t sssp_ld_keep(const uint32_t *p, uint64_t pol)
 {
     uint32_t r;
     asm volatile("ld.global.L2::cache_hint.u32 %0, [%1], %2;" : "=r"(r) : "l"(p), "l"(pol));
     return r;
 }
-#ifndef SSSP_FIRE_AND_FORGET
-#define SSSP_FIRE_AND_FORGET 1
-#endif
 #define SSSP_BIG_CHUNK 8192
 #define SSSP_BIG_DEGREE 512  // rows with at least this many edges are relaxed by CTAs (the graph-wide tier border is 4096)
 #ifndef SSSP_WARP_EDGES
 #define SSSP_WARP_EDGES 1280
 #endif
 
-// relax one edge: atomicMin on the uint32 view after a plain read that filters the losers; the winner marks the vertex
-// as due in the near (new distance below the threshold) or the far bitmap
-__device__ __forceinline__ void sssp_relax_one(uint32_t *__restrict__ dist, uint32_t *__restrict__ near_bm,
-                                               uint32_t *__restrict__ far_bm, uint32_t *__restrict__ changed_bm, int32_t col0,
-                                               int32_t vp, uint32_t threshold_bits, int32_t v, uint32_t c)
-{
-    if (c < dist[v])
-    {
-        const uint32_t old = atomicMin(&dist[v], c);
-        if (c < old)
-        {
-            // a vertex of this rank's slice (every vertex on one GPU) becomes due here; a vertex owned by a peer is
-            // flagged in the changed bitmap, whose slices go to the owners after the round
-            const uint32_t r = (uint32_t)(v - col0);
-            const bool local = r < (uint32_t)vp;
-            uint32_t *bm = local ? (c < threshold_bits ? near_bm : far_bm) : changed_bm;
-            const uint32_t i = local ? r : (uint32_t)v;
-            const uint32_t bit = 1u << (i & 31);
-            if (!(bm[i >> 5] & bit)) atomicOr(&bm[i >> 5], bit);
-        }
-    }
-}
-
-// relax SSSP_FLAT_UNROLL edges whose destination distances have been gathered, in PHASES: all atomicMin of the step (they
-// return the old value, so each is a full round trip), then the due-bitmap words of the winners, then the atomicOr marks.
-// Edge by edge the winners of a step paid up to 2 x SSSP_FLAT_UNROLL dependent round trips; in phases two. (The gathers are
-// issued together before any atomic for the same reason: an atomic orders the loads behind it.)
+// relax SSSP_FLAT_UNROLL edges whose destination distances have been gathered (together, before any atomic: an atomic orders
+// the loads behind it)
 template <int N>
 __device__ __forceinline__ void sssp_relax_batch(uint32_t *__restrict__ dist, uint32_t *__restrict__ near_bm, uint32_t *__restrict__ far_bm,
                                                  uint32_t *__restrict__ changed_bm, int32_t col0, int32_t vp, uint32_t threshold_bits,
                                                  const int32_t (&v)[N], const uint32_t (&c)[N], const uint32_t (&seen)[N])
 {
-#if SSSP_FIRE_AND_FORGET
     // Every candidate that beats the distance it saw lowers the distance AND marks the vertex due, both as reductions that
     // return nothing: no round trip left in the step after the gathers. A vertex may be marked by a candidate that lost to a
     // smaller one — it is due anyway (its distance dropped) — or, rarely, marked far by the loser and near by the winner: the far
@@ -319,35 +282,6 @@ __device__ __forceinline__ void sssp_relax_batch(uint32_t *__restrict__ dist, ui
             const uint32_t i = local ? r : (uint32_t)v[k];
             atomicOr(bm + (i >> 5), 1u << (i & 31));
         }
-#else
-    uint32_t old[N];
-#pragma unroll
-    for (int k = 0; k < N; k++) old[k] = (v[k] >= 0 && c[k] < seen[k]) ? atomicMin(&dist[v[k]], c[k]) : 0u;
-    uint32_t *word_ptr[N];
-    uint32_t word[N], bit[N];
-#pragma unroll
-    for (int k = 0; k < N; k++)
-    {
-        word_ptr[k] = NULL;
-        word[k] = 0xffffffffu;
-        bit[k] = 0;
-        if (c[k] < old[k]) // (old is 0 for the edges that did not try)
-        {
-            // a vertex of this rank's slice (every vertex on one GPU) becomes due here; a vertex owned by a peer is flagged in
-            // the changed bitmap, whose slices go to the owners after the round
-            const uint32_t r = (uint32_t)(v[k] - col0);
-            const bool local = r < (uint32_t)vp;
-            uint32_t *bm = local ? (c[k] < threshold_bits ? near_bm : far_bm) : changed_bm;
-            const uint32_t i = local ? r : (uint32_t)v[k];
-            word_ptr[k] = bm + (i >> 5);
-            bit[k] = 1u << (i & 31);
-            word[k] = *word_ptr[k];
-        }
-    }
-#pragma unroll
-    for (int k = 0; k < N; k++)
-        if (bit[k] && !(word[k] & bit[k])) atomicOr(word_ptr[k], bit[k]);
-#endif
 }
 
 __global__ void __launch_bounds__(SSSP_THREADS)
@@ -360,7 +294,6 @@ sssp_relax_flat_kernel(const int64_t *__restrict__ ptr, const int32_t *__restric
     const unsigned FULL = 0xffffffffu;
     const uint64_t pol = l2_policy_evict_first();
     const uint64_t pol_keep = l2_policy_evict_last();
-    (void)pol_keep;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     long long edges = 0;
     const int big_blocks = n_big * big_chunks;
@@ -391,7 +324,7 @@ sssp_relax_flat_kernel(const int64_t *__restrict__ ptr, const int32_t *__restric
             }
             uint32_t seen[SSSP_FLAT_UNROLL];
 #pragma unroll
-            for (int k = 0; k < SSSP_FLAT_UNROLL; k++) seen[k] = v[k] >= 0 ? SSSP_GATHER(dist + v[k]) : 0u;
+            for (int k = 0; k < SSSP_FLAT_UNROLL; k++) seen[k] = v[k] >= 0 ? sssp_ld_keep(dist + v[k], pol_keep) : 0u;
             sssp_relax_batch<SSSP_FLAT_UNROLL>(dist, near_bm, far_bm, changed_bm, col0, vp, threshold_bits, v, c, seen);
         }
     }
@@ -460,7 +393,7 @@ sssp_relax_flat_kernel(const int64_t *__restrict__ ptr, const int32_t *__restric
                     }
                 }
 #pragma unroll
-                for (int k = 0; k < SSSP_FLAT_UNROLL; k++) seen[k] = v[k] >= 0 ? SSSP_GATHER(dist + v[k]) : 0u;
+                for (int k = 0; k < SSSP_FLAT_UNROLL; k++) seen[k] = v[k] >= 0 ? sssp_ld_keep(dist + v[k], pol_keep) : 0u;
                 sssp_relax_batch<SSSP_FLAT_UNROLL>(dist, near_bm, far_bm, changed_bm, col0, vp, threshold_bits, v, c, seen);
             }
         }

@@ -170,16 +170,10 @@ class SingleGpuRunner:
             h_fwd, _ = pinned_array(vgl, g.V, np.int32)
             h_ptr[:], h_adj[:], h_fwd[:] = ptr, adj, g.orig_to_sorted()
             h_out, _ = pinned_array(vgl, g.V, np.float32 if self.dtype == "f32" else np.int32)
-            host = {"ptr": h_ptr, "adj": h_adj, "fwd": h_fwd, "out": h_out, "in_ptr": None, "in_adj": None, "w": None}
+            host = {"ptr": h_ptr, "adj": h_adj, "fwd": h_fwd, "out": h_out, "w": None}
             del ptr, adj
-            # BFS: the bottom-up levels need the incoming CSR. By default only the outgoing direction goes up and vglb_bfs derives
-            # the incoming one on the device (a sort of the edges beats a second PCIe upload of the same size);
-            # VGLB_E2E_UPLOAD_INCOMING=1 uploads the caller's incoming arrays instead (A/B).
-            if self.workload == "bfs" and self.bfs_direction_optimising and os.environ.get("VGLB_E2E_UPLOAD_INCOMING"):
-                iptr, iadj = g.layout(incoming=True)
-                host["in_ptr"], _ = pinned_array(vgl, g.V + 1, np.int64)
-                host["in_adj"], _ = pinned_array(vgl, g.E, np.int32)
-                host["in_ptr"][:], host["in_adj"][:] = iptr, iadj
+            # BFS: the bottom-up levels need the incoming CSR. Only the outgoing direction goes up and vglb_bfs derives the
+            # incoming one on the device (a sort of the edges beats a second PCIe upload of the same size).
             if self.workload == "sssp":
                 host["w"], _ = pinned_array(vgl, g.E, np.float32)
                 host["w"][:] = self.weights.to_numpy()
@@ -191,9 +185,8 @@ class SingleGpuRunner:
         H = self._host_arrays()
         L = vgl.lib()
         h2d = H["ptr"].nbytes + H["adj"].nbytes + H["fwd"].nbytes
-        for k in ("in_ptr", "in_adj", "w"):
-            if H[k] is not None:
-                h2d += H[k].nbytes
+        if H["w"] is not None:
+            h2d += H["w"].nbytes
         d2h = H["out"].nbytes
         times = []
         # (the caller says what it is going to run: PageRank's preparation then happens behind the upload)
@@ -201,7 +194,7 @@ class SingleGpuRunner:
         for i in range(steps + 1):
             ctx.synchronize()
             t0 = time.perf_counter()
-            g = vgl.Graph.from_csr(ctx, H["ptr"], H["adj"], H["fwd"], H["in_ptr"], H["in_adj"])
+            g = vgl.Graph.from_csr(ctx, H["ptr"], H["adj"], H["fwd"])
             out = ctx.empty(g.V, H["out"].dtype)
             if self.workload == "pr":
                 g.pagerank(self.pr_iters, 0.85, out)
