@@ -32,14 +32,8 @@ static double trace_now()
     return (double)ts.tv_sec + 1e-9 * (double)ts.tv_nsec;
 }
 
-// direction heuristic of the reference (gpu_change_state, change_state.hpp:5-6,100-141): ALPHA 15, BETA 18
-#define BFS_DEFAULT_ALPHA 15
-#define BFS_DEFAULT_BETA 18
-#define BFS_THREADS 256
-#define BFS_SMALL_LANES 8
 #define BFS_BU_PROBE 4       // in-neighbours probed per batch by one lane
 #define BFS_BU_PROBE_MAX 16  // lane-private probes before the warp takes the row over
-#define BFS_BIG_CHUNK 8192 // a "big" row is expanded by CTAs, one per chunk of this many edges
 
 // NT threads (a CTA, a warp or an 8-lane group) expand the out-row [s,e) of one frontier vertex.
 // Every thread of the warp must call this together (ballots inside); `e <= s` for idle groups.
@@ -159,6 +153,7 @@ __device__ __forceinline__ void td_expand(const int64_t *__restrict__ ptr, const
     }
 }
 
+// one top-down level: td_schedule (frontier.cuh) hands the queued rows to td_expand
 template <int MODE>
 __global__ void __launch_bounds__(BFS_THREADS)
 bfs_td_kernel(const int64_t *__restrict__ ptr, const int32_t *__restrict__ adj, TierQueues cq, int32_t n_big, int32_t hub_ctas,
@@ -166,102 +161,13 @@ bfs_td_kernel(const int64_t *__restrict__ ptr, const int32_t *__restrict__ adj, 
               int32_t *__restrict__ levels, int32_t next_level, int32_t b0, int32_t b1, TierQueues nq,
               unsigned long long *counters, PartArgs A)
 {
-    const int b = blockIdx.x;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int lane = threadIdx.x & 31;
     long long edges = 0, mf = 0;
     int found = 0;
-    // hubs (>= 4096 edges; the largest rows of a scale-26 Kronecker graph have > 10^6): the queued hub rows are cut into
-    // BFS_BIG_CHUNK-edge chunks and the chunks are dealt round-robin to `hub_ctas` CTAs. Every CTA stages 256 row ranges at a
-    // time in shared memory, scans their chunk counts (block prefix sum) and binary-searches the rows of the chunks it owns —
-    // no CTA is launched for a chunk that does not exist (one CTA per (row, chunk slot of the LONGEST row) launched
-    // hundreds of thousands of empty CTAs: 0.78 ms for an 18 M-edge level) and no CTA walks rows it has no chunk of.
-    const int big_blocks = hub_ctas;
-    if (b < big_blocks)
-    {
-        __shared__ int64_t s_row_start[BFS_THREADS], s_row_end[BFS_THREADS];
-        __shared__ int s_chunk_prefix[BFS_THREADS + 1];
-        __shared__ int s_warp_chunks[BFS_THREADS / 32];
-        long long chunk_base = 0; // chunks of the batches before this one
-        for (int base = 0; base < n_big; base += BFS_THREADS)
-        {
-            __syncthreads();
-            int nch = 0;
-            if (base + (int)threadIdx.x < n_big)
-            {
-                const int32_t u = cq.q[0][base + threadIdx.x];
-                const int64_t rs = ptr[u], re = ptr[u + 1];
-                s_row_start[threadIdx.x] = rs;
-                s_row_end[threadIdx.x] = re;
-                nch = (int)((re - rs + BFS_BIG_CHUNK - 1) / BFS_BIG_CHUNK);
-            }
-            int incl = nch;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1)
-            {
-                const int t = __shfl_up_sync(0xffffffffu, incl, o);
-                if (lane >= o) incl += t;
-            }
-            if (lane == 31) s_warp_chunks[warp] = incl;
-            __syncthreads();
-            int wbase = 0;
-#pragma unroll
-            for (int w = 0; w < BFS_THREADS / 32; w++)
-                if (w < warp) wbase += s_warp_chunks[w];
-            s_chunk_prefix[threadIdx.x + 1] = wbase + incl;
-            if (threadIdx.x == 0) s_chunk_prefix[0] = 0;
-            __syncthreads();
-            const int cnt = min(BFS_THREADS, n_big - base);
-            const int total = s_chunk_prefix[cnt];
-            int first = (int)((b - chunk_base % hub_ctas + hub_ctas) % hub_ctas);
-            for (int c = first; c < total; c += hub_ctas)
-            {
-                int lo = 0, hi = cnt; // row k with prefix[k] <= c < prefix[k + 1]
-                while (hi - lo > 1)
-                {
-                    const int mid = (lo + hi) >> 1;
-                    if (s_chunk_prefix[mid] <= c) lo = mid;
-                    else hi = mid;
-                }
-                const int64_t s = s_row_start[lo] + (int64_t)(c - s_chunk_prefix[lo]) * BFS_BIG_CHUNK, e = min(s_row_end[lo], s + BFS_BIG_CHUNK);
-                if (threadIdx.x == 0) edges += e - s;
-                td_expand<BFS_THREADS, MODE>(ptr, adj, s, e, threadIdx.x, visited, levels, next_level, b0, b1, nq, counters, mf, A, found);
-            }
-            chunk_base += total;
-        }
-    }
-    else if (b < big_blocks + blocks_mid)
-    {
-        const int nwarps = blocks_mid * (BFS_THREADS / 32);
-        for (int i = (b - big_blocks) * (BFS_THREADS / 32) + warp; i < n_mid; i += nwarps)
-        {
-            const int32_t u = cq.q[1][i];
-            const int64_t s = ptr[u], e = ptr[u + 1];
-            if (lane == 0) edges += e - s;
-            td_expand<32, MODE>(ptr, adj, s, e, lane, visited, levels, next_level, b0, b1, nq, counters, mf, A, found);
-        }
-    }
-    else
-    {
-        constexpr int G = BFS_SMALL_LANES;
-        constexpr int GROUPS = BFS_THREADS / G;
-        const int ngroups = blocks_small * GROUPS;
-        const int gid = threadIdx.x / G, gl = threadIdx.x % G;
-        // all groups of a warp iterate together (ballots in td_expand): pad the trip count to a multiple of the stride
-        const int first = (b - big_blocks - blocks_mid) * GROUPS + gid;
-        for (int base = first - gid; base < n_small; base += ngroups)
-        {
-            const int i = base + gid;
-            int64_t s = 0, e = 0;
-            if (i < n_small)
-            {
-                const int32_t u = cq.q[2][i];
-                s = ptr[u];
-                e = ptr[u + 1];
-                if (gl == 0) edges += e - s;
-            }
-            td_expand<G, MODE>(ptr, adj, s, e, gl, visited, levels, next_level, b0, b1, nq, counters, mf, A, found);
-        }
-    }
+    const TdGrid L = {n_big, hub_ctas, n_mid, n_small, blocks_mid, blocks_small};
+    td_schedule<long long>(ptr, cq, L, edges, [&](auto nt, int32_t, int64_t s, int64_t e, int tid) {
+        td_expand<decltype(nt)::value, MODE>(ptr, adj, s, e, tid, visited, levels, next_level, b0, b1, nq, counters, mf, A, found);
+    });
     edges = warp_sum_i64(edges);
     mf = warp_sum_i64(mf);
     if (lane == 0 && edges) atomicAdd(&counters[C_EDGES], (unsigned long long)edges);
@@ -664,25 +570,10 @@ __global__ void bfs_or_kernel(uint32_t *__restrict__ visited, const uint32_t *__
     }
 }
 
-__global__ void bfs_copy_counters_kernel(unsigned long long *c)
-{
-    if (threadIdx.x < C_COUNT) c[C_COUNT + threadIdx.x] = c[threadIdx.x];
-}
-
 static int bfs_partitioned_bitmaps(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t *d_levels, const vglb_bfs_opts *opts,
                                    vglb_stats *stats)
 {
-    VGLB_REQUIRE(source >= 0 && source < g->cols, "vglb_bfs: source column out of range");
-    const bool dopt = opts && opts->direction_optimising;
-    if (dopt && !g->d_in_ptr)
-    {
-        vglb_set_error("vglb_bfs: direction-optimising BFS needs a graph built with VGLB_GRAPH_WITH_INCOMING");
-        return VGLB_EINVAL;
-    }
-    const long long alpha = (opts && opts->alpha > 0) ? opts->alpha : 15;
-    const long long beta = (opts && opts->beta > 0) ? opts->beta : 18;
-    CUDA_TRY(cudaSetDevice(ctx->device));
-    int rc0;
+    const BfsDirection dir = bfs_direction(opts, g->E_global, g->V_orig);
     vglb_comm *comm = g->comm;
     const int32_t P = g->part_world, rank = g->part_rank, vp = g->vp, rows = g->V;
     const int32_t wslice = vp / 32;
@@ -691,17 +582,14 @@ static int bfs_partitioned_bitmaps(vglb_ctx *ctx, vglb_graph *g, int32_t source,
         if (!g->d_part_bm[i]) CUDA_TRY(vglb_dev_alloc(&g->d_part_bm[i], (size_t)(words + 32) * 4));
     if (!g->d_part_stage) CUDA_TRY(vglb_dev_alloc(&g->d_part_stage, (size_t)(words + 32) * 4));
     if (!g->d_queue[0]) CUDA_TRY(vglb_dev_alloc(&g->d_queue[0], ((size_t)vp + 3) * 4));
-    rc0 = bfs_prepare_no_in_edges(ctx, g);
-    if (rc0 != VGLB_OK) return rc0;
+    int rc = bfs_prepare_no_in_edges(ctx, g);
+    if (rc != VGLB_OK) return rc;
     const int64_t launches0 = ctx->launches;
     const int32_t b0 = g->tier_border[0], b1 = g->tier_border[1];
     unsigned long long *d_cnt = (unsigned long long *)ctx->d_counters;
     unsigned long long *h_cnt = (unsigned long long *)ctx->h_counters;
     cudaStream_t st = ctx->stream;
-    TierQueues cq;
-    cq.q[0] = g->d_queue[0];
-    cq.q[1] = g->d_queue[0] + b0;
-    cq.q[2] = g->d_queue[0] + b1;
+    TierQueues cq = tier_regions(g->d_queue[0], b0, b1);
     uint32_t *visited = g->d_part_bm[0], *cur_bm = g->d_part_bm[1], *next_bm = g->d_part_bm[2];
 
     CUDA_TRY(cudaEventRecord(ctx->ev_start, st));
@@ -725,10 +613,7 @@ static int bfs_partitioned_bitmaps(vglb_ctx *ctx, vglb_graph *g, int32_t source,
     int64_t tot_edges = 0, tot_rows = 0, tot_frontier_bytes = 0, levels_run = 0;
     int32_t bu_levels = 0;
     const long long Vg = g->V_orig;
-    const long long factor = (g->E_global / (Vg > 0 ? Vg : 1)) / 2 > 0 ? (g->E_global / Vg) / 2 : 1;
     const int max_blocks = ctx->sm_count * 16;
-    const int big_chunks = (int)ceil_div64(g->max_degree > 0 ? g->max_degree : 1, BFS_BIG_CHUNK);
-    int rc;
     const bool trace = getenv("VGLB_BFS_TRACE") != NULL;
     double trace_t = 0.0;
     if (trace)
@@ -742,15 +627,12 @@ static int bfs_partitioned_bitmaps(vglb_ctx *ctx, vglb_graph *g, int32_t source,
         if (!bottom_up)
         {
             CUDA_TRY(cudaMemsetAsync(next_bm, 0, (size_t)words * 4, st)); // candidates
-            const int blocks_mid = (int)min((int64_t)max_blocks, ceil_div64(n[1], BFS_THREADS / 32));
-            const int blocks_small = (int)min((int64_t)max_blocks, ceil_div64(n[2], BFS_THREADS / BFS_SMALL_LANES));
-            const int hub_ctas = (int)min((int64_t)n[0] * big_chunks, (int64_t)ctx->sm_count * 4); // CTAs that share the queued hub rows
-            const int64_t grid = (int64_t)hub_ctas + blocks_mid + blocks_small;
-            if (grid > 0)
+            const TdGrid L = td_grid(ctx, g, n);
+            if (L.ctas() > 0)
             {
-                bfs_td_kernel<1><<<(unsigned)grid, BFS_THREADS, 0, st>>>(g->d_out_ptr, g->d_out_adj, cq, n[0], hub_ctas, n[1], n[2], blocks_mid,
-                                                                       blocks_small, visited, (int32_t *)next_bm, level + 1, b0, b1,
-                                                                       cq, d_cnt, PartArgs());
+                bfs_td_kernel<1><<<(unsigned)L.ctas(), BFS_THREADS, 0, st>>>(g->d_out_ptr, g->d_out_adj, cq, L.n_big, L.hub_ctas, L.n_mid,
+                                                                           L.n_small, L.blocks_mid, L.blocks_small, visited,
+                                                                           (int32_t *)next_bm, level + 1, b0, b1, cq, d_cnt, PartArgs());
                 KERNEL_TRY();
                 ctx->launches++;
             }
@@ -776,9 +658,9 @@ static int bfs_partitioned_bitmaps(vglb_ctx *ctx, vglb_graph *g, int32_t source,
         if (rc != VGLB_OK) return rc;
         bfs_or_kernel<<<(unsigned)min((int64_t)max_blocks, ceil_div64(words, 256)), 256, 0, st>>>(visited, next_bm, words);
         KERNEL_TRY();
-        bfs_copy_counters_kernel<<<1, 32, 0, st>>>(d_cnt);
-        KERNEL_TRY();
-        ctx->launches += 2;
+        ctx->launches++;
+        rc = vglb_stage_counters(ctx);
+        if (rc != VGLB_OK) return rc;
         rc = vglb_comm_allreduce_async(comm, d_cnt + C_COUNT, C_COUNT, VGLB_DT_I64, VGLB_OP_SUM);
         if (rc != VGLB_OK) return rc;
         CUDA_TRY(cudaMemcpyAsync(h_cnt, d_cnt, 2 * C_COUNT * 8, cudaMemcpyDeviceToHost, st));
@@ -800,19 +682,7 @@ static int bfs_partitioned_bitmaps(vglb_ctx *ctx, vglb_graph *g, int32_t source,
         visited_total += n_next;
         if (n_next == 0) break;
 
-        bool next_bu = bottom_up;
-        if (dopt)
-        {
-            const long long unvisited = Vg - visited_total;
-            if (!bottom_up && n_cur < n_next)
-            {
-                if ((long long)gl[C_MF] >= (unvisited * factor + Vg) / alpha) next_bu = true;
-            }
-            else if (bottom_up && n_cur >= n_next)
-            {
-                if (n_next < (unvisited * factor + Vg) / (factor * beta)) next_bu = false;
-            }
-        }
+        const bool next_bu = next_direction(dir, bottom_up, n_cur, n_next, (long long)gl[C_MF], Vg - visited_total, Vg);
         if (!next_bu)
         {
             if (!bottom_up)
@@ -836,22 +706,14 @@ static int bfs_partitioned_bitmaps(vglb_ctx *ctx, vglb_graph *g, int32_t source,
         n_cur = n_next;
         level++;
     }
-    CUDA_TRY(cudaEventRecord(ctx->ev_stop, st));
-    CUDA_TRY(cudaEventSynchronize(ctx->ev_stop));
-    if (stats)
-    {
-        float ms = 0.f;
-        CUDA_TRY(cudaEventElapsedTime(&ms, ctx->ev_start, ctx->ev_stop));
-        memset(stats, 0, sizeof(*stats));
-        stats->seconds = ms * 1e-3;
-        stats->iterations = levels_run;
-        stats->edges_inspected = tot_edges;      // this rank's
-        stats->vertices_processed = tot_rows;
-        stats->frontier_bytes = tot_frontier_bytes;
-        stats->algorithmic_bytes = 8 * tot_edges + 12 * tot_rows + tot_frontier_bytes;
-        stats->kernel_launches = ctx->launches - launches0;
-        stats->bottom_up_levels = bu_levels;
-    }
+    rc = vglb_finish_run(ctx, launches0, stats);
+    if (rc != VGLB_OK || !stats) return rc;
+    stats->iterations = levels_run;
+    stats->edges_inspected = tot_edges; // this rank's
+    stats->vertices_processed = tot_rows;
+    stats->frontier_bytes = tot_frontier_bytes;
+    stats->algorithmic_bytes = 8 * tot_edges + 12 * tot_rows + tot_frontier_bytes;
+    stats->bottom_up_levels = bu_levels;
     return VGLB_OK;
 }
 
@@ -867,16 +729,7 @@ static int bfs_partitioned_bitmaps(vglb_ctx *ctx, vglb_graph *g, int32_t source,
 static int bfs_partitioned(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t *d_levels, const vglb_bfs_opts *opts,
                            vglb_stats *stats)
 {
-    VGLB_REQUIRE(source >= 0 && source < g->cols, "vglb_bfs: source column out of range");
-    const bool dopt = opts && opts->direction_optimising;
-    if (dopt && !g->d_in_ptr)
-    {
-        vglb_set_error("vglb_bfs: direction-optimising BFS needs a graph built with VGLB_GRAPH_WITH_INCOMING");
-        return VGLB_EINVAL;
-    }
-    const long long alpha = (opts && opts->alpha > 0) ? opts->alpha : 15;
-    const long long beta = (opts && opts->beta > 0) ? opts->beta : 18;
-    CUDA_TRY(cudaSetDevice(ctx->device));
+    const BfsDirection dir = bfs_direction(opts, g->E_global, g->V_orig);
     vglb_comm *comm = g->comm;
     const int32_t P = g->part_world, rank = g->part_rank, vp = g->vp, rows = g->V;
     const int32_t wslice = vp / 32;
@@ -892,14 +745,7 @@ static int bfs_partitioned(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t
     unsigned long long *d_cnt = (unsigned long long *)ctx->d_counters;
     unsigned long long *h_cnt = (unsigned long long *)ctx->h_counters;
     cudaStream_t st = ctx->stream;
-    auto regions = [&](int32_t *base) {
-        TierQueues q;
-        q.q[0] = base;
-        q.q[1] = base + b0;
-        q.q[2] = base + b1;
-        return q;
-    };
-    TierQueues cq = regions(g->d_queue[0]), nq = regions(g->d_queue[1]);
+    TierQueues cq = tier_regions(g->d_queue[0], b0, b1), nq = tier_regions(g->d_queue[1], b0, b1);
     uint32_t *visited = g->d_part_bm[0], *cur_bm = g->d_part_bm[1], *next_bm = g->d_part_bm[2];
     PartArgs A;
     A.col0 = g->col_of_row0;
@@ -931,9 +777,7 @@ static int bfs_partitioned(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t
     int64_t tot_edges = 0, tot_rows = 0, tot_frontier_bytes = 0, levels_run = 0;
     int32_t bu_levels = 0;
     const long long Vg = g->V_orig;
-    const long long factor = (g->E_global / (Vg > 0 ? Vg : 1)) / 2 > 0 ? (g->E_global / Vg) / 2 : 1;
     const int max_blocks = ctx->sm_count * 16;
-    const int big_chunks = (int)ceil_div64(g->max_degree > 0 ? g->max_degree : 1, BFS_BIG_CHUNK);
     const bool trace = getenv("VGLB_BFS_TRACE") != NULL;
     double trace_t = 0.0;
     if (trace)
@@ -947,14 +791,12 @@ static int bfs_partitioned(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t
         if (!bottom_up)
         {
             CUDA_TRY(cudaMemsetAsync(A.lists, 0, (size_t)P * 8, st)); // list lengths (the peers finished reading them: see below)
-            const int blocks_mid = (int)min((int64_t)max_blocks, ceil_div64(n[1], BFS_THREADS / 32));
-            const int blocks_small = (int)min((int64_t)max_blocks, ceil_div64(n[2], BFS_THREADS / BFS_SMALL_LANES));
-            const int hub_ctas = (int)min((int64_t)n[0] * big_chunks, (int64_t)ctx->sm_count * 4); // CTAs that share the queued hub rows
-            const int64_t grid = (int64_t)hub_ctas + blocks_mid + blocks_small;
-            if (grid > 0)
+            const TdGrid L = td_grid(ctx, g, n);
+            if (L.ctas() > 0)
             {
-                bfs_td_kernel<2><<<(unsigned)grid, BFS_THREADS, 0, st>>>(g->d_out_ptr, g->d_out_adj, cq, n[0], hub_ctas, n[1], n[2], blocks_mid,
-                                                                       blocks_small, visited, d_levels, level + 1, b0, b1, nq, d_cnt, A);
+                bfs_td_kernel<2><<<(unsigned)L.ctas(), BFS_THREADS, 0, st>>>(g->d_out_ptr, g->d_out_adj, cq, L.n_big, L.hub_ctas, L.n_mid,
+                                                                           L.n_small, L.blocks_mid, L.blocks_small, visited, d_levels,
+                                                                           level + 1, b0, b1, nq, d_cnt, A);
                 KERNEL_TRY();
                 ctx->launches++;
             }
@@ -980,9 +822,8 @@ static int bfs_partitioned(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t
             bu_levels++;
             tot_frontier_bytes += (int64_t)wslice * 4 * 3 + words * 4 * 3;
         }
-        bfs_copy_counters_kernel<<<1, 32, 0, st>>>(d_cnt);
-        KERNEL_TRY();
-        ctx->launches++;
+        rc = vglb_stage_counters(ctx);
+        if (rc != VGLB_OK) return rc;
         rc = vglb_comm_allreduce_async(comm, d_cnt + C_COUNT, C_COUNT, VGLB_DT_I64, VGLB_OP_SUM);
         if (rc != VGLB_OK) return rc;
         CUDA_TRY(cudaMemcpyAsync(h_cnt, d_cnt, 2 * C_COUNT * 8, cudaMemcpyDeviceToHost, st));
@@ -1005,19 +846,7 @@ static int bfs_partitioned(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t
         visited_total += n_next;
         if (n_next == 0) break;
 
-        bool next_bu = bottom_up;
-        if (dopt)
-        {
-            const long long unvisited = Vg - visited_total;
-            if (!bottom_up && n_cur < n_next)
-            {
-                if ((long long)gl[C_MF] >= (unvisited * factor + Vg) / alpha) next_bu = true;
-            }
-            else if (bottom_up && n_cur >= n_next)
-            {
-                if (n_next < (unvisited * factor + Vg) / (factor * beta)) next_bu = false;
-            }
-        }
+        const bool next_bu = next_direction(dir, bottom_up, n_cur, n_next, (long long)gl[C_MF], Vg - visited_total, Vg);
         if (!bottom_up && !next_bu)
         {
             TierQueues t = cq; cq = nq; nq = t;
@@ -1059,38 +888,30 @@ static int bfs_partitioned(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t
         n_cur = n_next;
         level++;
     }
-    CUDA_TRY(cudaEventRecord(ctx->ev_stop, st));
-    CUDA_TRY(cudaEventSynchronize(ctx->ev_stop));
-    if (stats)
-    {
-        float ms = 0.f;
-        CUDA_TRY(cudaEventElapsedTime(&ms, ctx->ev_start, ctx->ev_stop));
-        memset(stats, 0, sizeof(*stats));
-        stats->seconds = ms * 1e-3;
-        stats->iterations = levels_run;
-        stats->edges_inspected = tot_edges;      // this rank's
-        stats->vertices_processed = tot_rows;
-        stats->frontier_bytes = tot_frontier_bytes;
-        stats->algorithmic_bytes = 8 * tot_edges + 12 * tot_rows + tot_frontier_bytes;
-        stats->kernel_launches = ctx->launches - launches0;
-        stats->bottom_up_levels = bu_levels;
-    }
+    rc = vglb_finish_run(ctx, launches0, stats);
+    if (rc != VGLB_OK || !stats) return rc;
+    stats->iterations = levels_run;
+    stats->edges_inspected = tot_edges; // this rank's
+    stats->vertices_processed = tot_rows;
+    stats->frontier_bytes = tot_frontier_bytes;
+    stats->algorithmic_bytes = 8 * tot_edges + 12 * tot_rows + tot_frontier_bytes;
+    stats->bottom_up_levels = bu_levels;
     return VGLB_OK;
 }
 
-static int bfs_prepare(vglb_ctx *ctx, vglb_graph *g)
+// the scratch is shared with SSSP and vglb_bfs_multi (each allocates the same fields, same sizes, on first use): never
+// overwrite a pointer another algorithm has already filled in
+int bfs_prepare_queues(vglb_ctx *ctx, vglb_graph *g)
 {
-    if (g->bfs_ready) return VGLB_OK;
-    // the scratch is shared with SSSP (sssp.cu allocates the same fields, same sizes, on first use): never overwrite
-    // a pointer another algorithm has already filled in
-    const size_t words = ((size_t)g->V + 31) / 32 + 32;
-    if (!g->d_visited) CUDA_TRY(vglb_dev_alloc(&g->d_visited, words * 4));
-    if (!g->d_front_bm[0]) CUDA_TRY(vglb_dev_alloc(&g->d_front_bm[0], words * 4));
-    if (!g->d_front_bm[1]) CUDA_TRY(vglb_dev_alloc(&g->d_front_bm[1], words * 4));
-    if (!g->d_queue[0]) CUDA_TRY(vglb_dev_alloc(&g->d_queue[0], ((size_t)g->V + 3) * 4));
-    if (!g->d_queue[1]) CUDA_TRY(vglb_dev_alloc(&g->d_queue[1], ((size_t)g->V + 3) * 4));
-    g->bfs_ready = 1;
-    return bfs_prepare_no_in_edges(ctx, g);
+    for (int i = 0; i < 2; i++)
+        if (!g->d_queue[i]) CUDA_TRY(vglb_dev_alloc(&g->d_queue[i], ((size_t)g->V + 3) * 4));
+    int rc = bfs_prepare_no_in_edges(ctx, g);
+    if (rc != VGLB_OK || g->bfs_big_border_plus1 != 0) return rc;
+    int32_t border = 0; // first id with fewer than BFS_BIG_DEGREE edges (ids are degree-sorted), once per graph
+    rc = vglb_graph_threshold_vertex(ctx, g, BFS_BIG_DEGREE, &border);
+    if (rc != VGLB_OK) return rc;
+    g->bfs_big_border_plus1 = border + 1;
+    return VGLB_OK;
 }
 
 extern "C" int vglb_bfs(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t *d_levels, const vglb_bfs_opts *opts,
@@ -1102,12 +923,18 @@ extern "C" int vglb_bfs(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t *d
         CUDA_TRY(cudaSetDevice(ctx->device));
         int rc = vglb_part_map_lists(ctx, g); // per-owner discovery lists, mapped into the peers once per graph
         if (rc != VGLB_OK) return rc;
+        VGLB_REQUIRE(source >= 0 && source < g->cols, "vglb_bfs: source column out of range");
+        if (opts && opts->direction_optimising && !g->d_in_ptr)
+        {
+            vglb_set_error("vglb_bfs: direction-optimising BFS needs a graph built with VGLB_GRAPH_WITH_INCOMING");
+            return VGLB_EINVAL;
+        }
         return g->vec_peers_mapped > 0 ? bfs_partitioned(ctx, g, source, d_levels, opts, stats)
                                        : bfs_partitioned_bitmaps(ctx, g, source, d_levels, opts, stats);
     }
     VGLB_REQUIRE(source >= 0 && source < g->V, "vglb_bfs: source out of range");
-    const bool dopt = opts && opts->direction_optimising;
-    if (dopt && !g->d_in_ptr)
+    const BfsDirection dir = bfs_direction(opts, g->E, g->V);
+    if (dir.dopt && !g->d_in_ptr)
     {
         // The bottom-up levels need the incoming CSR. A graph uploaded without it (vglb_graph_from_csr with NULL incoming arrays)
         // gets it here, once, from the outgoing one: a device sort of the edges is cheaper than a second 4.8 GB PCIe upload
@@ -1115,35 +942,21 @@ extern "C" int vglb_bfs(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t *d
         int rc_in = vglb_graph_derive_incoming(ctx, g);
         if (rc_in != VGLB_OK) return rc_in;
     }
-    const long long alpha = (opts && opts->alpha > 0) ? opts->alpha : BFS_DEFAULT_ALPHA;
-    const long long beta = (opts && opts->beta > 0) ? opts->beta : BFS_DEFAULT_BETA;
     CUDA_TRY(cudaSetDevice(ctx->device));
-    int rc = bfs_prepare(ctx, g);
+    const size_t bm_bytes = (((size_t)g->V + 31) / 32 + 32) * 4;
+    if (!g->d_visited) CUDA_TRY(vglb_dev_alloc(&g->d_visited, bm_bytes));
+    for (int i = 0; i < 2; i++)
+        if (!g->d_front_bm[i]) CUDA_TRY(vglb_dev_alloc(&g->d_front_bm[i], bm_bytes));
+    int rc = bfs_prepare_queues(ctx, g);
     if (rc != VGLB_OK) return rc;
     const int64_t launches0 = ctx->launches;
     const int32_t V = g->V;
-    if (g->bfs_big_border_plus1 == 0) // first id with fewer than BFS_BIG_DEGREE edges (ids are degree-sorted), once per graph
-    {
-        int32_t border = 0;
-        rc = vglb_graph_threshold_vertex(ctx, g, BFS_BIG_DEGREE, &border);
-        if (rc != VGLB_OK) return rc;
-        g->bfs_big_border_plus1 = border + 1;
-    }
     const int32_t b0 = g->bfs_big_border_plus1 - 1, b1 = g->tier_border[1] > b0 ? g->tier_border[1] : b0;
     const size_t words = ((size_t)V + 31) / 32;
     unsigned long long *d_cnt = (unsigned long long *)ctx->d_counters;
     unsigned long long *h_cnt = (unsigned long long *)ctx->h_counters;
     cudaStream_t st = ctx->stream;
-
-    // queue regions: capacity of a tier's queue = population of the tier
-    auto regions = [&](int32_t *base) {
-        TierQueues q;
-        q.q[0] = base;
-        q.q[1] = base + b0;
-        q.q[2] = base + b1;
-        return q;
-    };
-    TierQueues cq = regions(g->d_queue[0]), nq = regions(g->d_queue[1]);
+    TierQueues cq = tier_regions(g->d_queue[0], b0, b1), nq = tier_regions(g->d_queue[1], b0, b1);
     uint32_t *cur_bm = g->d_front_bm[0], *next_bm = g->d_front_bm[1];
 
     CUDA_TRY(cudaEventRecord(ctx->ev_start, st));
@@ -1162,9 +975,7 @@ extern "C" int vglb_bfs(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t *d
     int32_t level = VGLB_FIRST_LEVEL_VERTEX;
     int64_t tot_edges = 0, tot_rows = 0, tot_frontier_bytes = 0, levels_run = 0;
     int32_t bu_levels = 0;
-    const long long factor = (g->E / (V > 0 ? V : 1)) / 2 > 0 ? (g->E / V) / 2 : 1; // change_state.hpp:104
     const int max_blocks = ctx->sm_count * 16;
-    const int big_chunks = (int)ceil_div64(g->max_degree > 0 ? g->max_degree : 1, BFS_BIG_CHUNK);
     const bool trace = getenv("VGLB_BFS_TRACE") != NULL; // developer aid: one line per level on stderr
     double trace_t = 0.0;
     if (trace)
@@ -1180,27 +991,22 @@ extern "C" int vglb_bfs(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t *d
         const bool bitmap_out = !bottom_up && m_f_cur > (1LL << 20);
         if (!bottom_up)
         {
-            const int blocks_mid = (int)min((int64_t)max_blocks, ceil_div64(n[1], BFS_THREADS / 32));
-            const int blocks_small = (int)min((int64_t)max_blocks, ceil_div64(n[2], BFS_THREADS / BFS_SMALL_LANES));
-            const int hub_ctas = (int)min((int64_t)n[0] * big_chunks, (int64_t)ctx->sm_count * 4); // CTAs that share the queued hub rows
-            const int64_t grid = (int64_t)hub_ctas + blocks_mid + blocks_small;
+            const TdGrid L = td_grid(ctx, g, n);
+            PartArgs out;
+            memset(&out, 0, sizeof(out));
             if (bitmap_out)
             {
-                PartArgs out;
-                memset(&out, 0, sizeof(out));
                 out.lists = reinterpret_cast<unsigned long long *>(next_bm);
                 CUDA_TRY(cudaMemsetAsync(next_bm, 0, words * 4, st));
-                bfs_td_kernel<3><<<(unsigned)grid, BFS_THREADS, 0, st>>>(g->d_out_ptr, g->d_out_adj, cq, n[0], hub_ctas, n[1], n[2], blocks_mid,
-                                                                       blocks_small, g->d_visited, d_levels, level + 1, b0, b1, nq, d_cnt, out);
+                bfs_td_kernel<3><<<(unsigned)L.ctas(), BFS_THREADS, 0, st>>>(g->d_out_ptr, g->d_out_adj, cq, L.n_big, L.hub_ctas, L.n_mid,
+                                                                           L.n_small, L.blocks_mid, L.blocks_small, g->d_visited,
+                                                                           d_levels, level + 1, b0, b1, nq, d_cnt, out);
                 tot_frontier_bytes += (int64_t)words * 4;
             }
             else
-            {
-                PartArgs none;
-                memset(&none, 0, sizeof(none));
-                bfs_td_kernel<0><<<(unsigned)grid, BFS_THREADS, 0, st>>>(g->d_out_ptr, g->d_out_adj, cq, n[0], hub_ctas, n[1], n[2], blocks_mid,
-                                                                       blocks_small, g->d_visited, d_levels, level + 1, b0, b1, nq, d_cnt, none);
-            }
+                bfs_td_kernel<0><<<(unsigned)L.ctas(), BFS_THREADS, 0, st>>>(g->d_out_ptr, g->d_out_adj, cq, L.n_big, L.hub_ctas, L.n_mid,
+                                                                           L.n_small, L.blocks_mid, L.blocks_small, g->d_visited,
+                                                                           d_levels, level + 1, b0, b1, nq, d_cnt, out);
             KERNEL_TRY();
             ctx->launches++;
             tot_rows += n_cur;
@@ -1235,21 +1041,7 @@ extern "C" int vglb_bfs(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t *d
         }
         if (n_next == 0) break;
 
-        // direction switch — gpu_change_state (change_state.hpp:100-141) evaluated on the device counters; the
-        // top-down test uses the edges the NEXT top-down level would inspect (m_f) instead of the level just done
-        bool next_bu = bottom_up;
-        if (dopt)
-        {
-            const long long unvisited = (long long)V - visited_total;
-            if (!bottom_up && n_cur < n_next)
-            {
-                if (m_f_next >= (unvisited * factor + V) / alpha) next_bu = true;
-            }
-            else if (bottom_up && n_cur >= n_next)
-            {
-                if (n_next < (unvisited * factor + V) / (factor * beta)) next_bu = false;
-            }
-        }
+        const bool next_bu = next_direction(dir, bottom_up, n_cur, n_next, m_f_next, (long long)V - visited_total, V);
         CUDA_TRY(cudaMemsetAsync(d_cnt, 0, C_COUNT * 8, st));
         if (!out_is_bitmap && !next_bu)
         {
@@ -1288,22 +1080,14 @@ extern "C" int vglb_bfs(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t *d
         n_cur = n_next;
         level++;
     }
-    CUDA_TRY(cudaEventRecord(ctx->ev_stop, st));
-    CUDA_TRY(cudaEventSynchronize(ctx->ev_stop));
-    if (stats)
-    {
-        float ms = 0.f;
-        CUDA_TRY(cudaEventElapsedTime(&ms, ctx->ev_start, ctx->ev_stop));
-        memset(stats, 0, sizeof(*stats));
-        stats->seconds = ms * 1e-3;
-        stats->iterations = levels_run;
-        stats->edges_inspected = tot_edges;
-        stats->vertices_processed = tot_rows;
-        stats->frontier_bytes = tot_frontier_bytes;
-        // SURVEY §8(d): B = sum_levels [ 8 e_l + 12 f_l + g_l ]
-        stats->algorithmic_bytes = 8 * tot_edges + 12 * tot_rows + tot_frontier_bytes;
-        stats->kernel_launches = ctx->launches - launches0;
-        stats->bottom_up_levels = bu_levels;
-    }
+    rc = vglb_finish_run(ctx, launches0, stats);
+    if (rc != VGLB_OK || !stats) return rc;
+    stats->iterations = levels_run;
+    stats->edges_inspected = tot_edges;
+    stats->vertices_processed = tot_rows;
+    stats->frontier_bytes = tot_frontier_bytes;
+    // SURVEY §8(d): B = sum_levels [ 8 e_l + 12 f_l + g_l ]
+    stats->algorithmic_bytes = 8 * tot_edges + 12 * tot_rows + tot_frontier_bytes;
+    stats->bottom_up_levels = bu_levels;
     return VGLB_OK;
 }

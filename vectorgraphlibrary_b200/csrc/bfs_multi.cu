@@ -23,9 +23,6 @@
 #include "common.cuh"
 #include "frontier.cuh"
 
-#define BFS_MS_THREADS 256
-#define BFS_MS_SMALL_LANES 8
-#define BFS_MS_BIG_CHUNK 8192 // a queued big row is expanded by CTAs, one per chunk of this many edges
 #define BFS_MS_PROBE 4        // in-neighbours loaded per step by one lane (bottom-up)
 #define BFS_MS_PROBE_MAX 16   // lane-private in-neighbours before the warp takes the row over
 #define BFS_MS_LONG_UNROLL 8  // in-neighbours per lane and round trip when the warp scans one row
@@ -124,113 +121,25 @@ __device__ __forceinline__ void ms_td_expand(const int64_t *__restrict__ ptr, co
     }
 }
 
+// one top-down level: td_schedule (frontier.cuh) hands the queued rows to ms_td_expand
 template <class W>
-__global__ void __launch_bounds__(BFS_MS_THREADS)
+__global__ void __launch_bounds__(BFS_THREADS)
 bfs_multi_td_kernel(const int64_t *__restrict__ ptr, const int32_t *__restrict__ adj, TierQueues cq, int32_t n_big, int32_t hub_ctas,
                     int32_t n_mid, int32_t n_small, int32_t blocks_mid, int32_t blocks_small, const W *__restrict__ front, W full,
                     W *__restrict__ seen, W *__restrict__ next, int32_t *__restrict__ levels, int32_t V, int32_t next_level,
                     int32_t b0, int32_t b1, TierQueues nq, unsigned long long *counters)
 {
-    const int b = blockIdx.x;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     MsCounts c = {0, 0, 0, 0, 0, 0};
-    if (b < hub_ctas)
-    {
-        // queued big rows cut into BFS_MS_BIG_CHUNK-edge chunks dealt round-robin to `hub_ctas` CTAs (bfs_td_kernel's scheme)
-        __shared__ int64_t s_row_start[BFS_MS_THREADS], s_row_end[BFS_MS_THREADS];
-        __shared__ W s_word[BFS_MS_THREADS];
-        __shared__ int s_chunk_prefix[BFS_MS_THREADS + 1];
-        __shared__ int s_warp_chunks[BFS_MS_THREADS / 32];
-        int chunk_base = 0; // chunks of the batches before this one
-        for (int base = 0; base < n_big; base += BFS_MS_THREADS)
-        {
-            __syncthreads();
-            int nch = 0;
-            if (base + (int)threadIdx.x < n_big)
-            {
-                const int32_t u = cq.q[0][base + threadIdx.x];
-                const int64_t rs = ptr[u], re = ptr[u + 1];
-                s_row_start[threadIdx.x] = rs;
-                s_row_end[threadIdx.x] = re;
-                s_word[threadIdx.x] = front[u];
-                nch = (int)((re - rs + BFS_MS_BIG_CHUNK - 1) / BFS_MS_BIG_CHUNK);
-            }
-            int incl = nch;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1)
-            {
-                const int t = __shfl_up_sync(0xffffffffu, incl, o);
-                if (lane >= o) incl += t;
-            }
-            if (lane == 31) s_warp_chunks[warp] = incl;
-            __syncthreads();
-            int wbase = 0;
-#pragma unroll
-            for (int w = 0; w < BFS_MS_THREADS / 32; w++)
-                if (w < warp) wbase += s_warp_chunks[w];
-            s_chunk_prefix[threadIdx.x + 1] = wbase + incl;
-            if (threadIdx.x == 0) s_chunk_prefix[0] = 0;
-            __syncthreads();
-            const int cnt = min(BFS_MS_THREADS, n_big - base);
-            const int total = s_chunk_prefix[cnt];
-            const int first = (int)((b - chunk_base % hub_ctas + hub_ctas) % hub_ctas);
-            for (int ch = first; ch < total; ch += hub_ctas)
-            {
-                int lo = 0, hi = cnt;
-                while (hi - lo > 1)
-                {
-                    const int mid = (lo + hi) >> 1;
-                    if (s_chunk_prefix[mid] <= ch) lo = mid;
-                    else hi = mid;
-                }
-                const int64_t s = s_row_start[lo] + (int64_t)(ch - s_chunk_prefix[lo]) * BFS_MS_BIG_CHUNK;
-                const int64_t e = min(s_row_end[lo], s + BFS_MS_BIG_CHUNK);
-                if (threadIdx.x == 0) c.edges += e - s;
-                ms_td_expand<BFS_MS_THREADS, W>(ptr, adj, s, e, threadIdx.x, s_word[lo], full, seen, next, levels, V, next_level, b0, b1,
-                                                nq, counters, c);
-            }
-            chunk_base += total;
-        }
-    }
-    else if (b < hub_ctas + blocks_mid)
-    {
-        const int nwarps = blocks_mid * (BFS_MS_THREADS / 32);
-        for (int i = (b - hub_ctas) * (BFS_MS_THREADS / 32) + warp; i < n_mid; i += nwarps)
-        {
-            const int32_t u = cq.q[1][i];
-            const int64_t s = ptr[u], e = ptr[u + 1];
-            if (lane == 0) c.edges += e - s;
-            ms_td_expand<32, W>(ptr, adj, s, e, lane, front[u], full, seen, next, levels, V, next_level, b0, b1, nq, counters, c);
-        }
-    }
-    else
-    {
-        constexpr int G = BFS_MS_SMALL_LANES;
-        constexpr int GROUPS = BFS_MS_THREADS / G;
-        const int ngroups = blocks_small * GROUPS;
-        const int gid = threadIdx.x / G, gl = threadIdx.x % G;
-        const int first = (b - hub_ctas - blocks_mid) * GROUPS + gid;
-        for (int base = first - gid; base < n_small; base += ngroups) // trip count uniform over the warp (ballots inside)
-        {
-            const int i = base + gid;
-            int64_t s = 0, e = 0;
-            W fu = 0;
-            if (i < n_small)
-            {
-                const int32_t u = cq.q[2][i];
-                s = ptr[u];
-                e = ptr[u + 1];
-                fu = front[u];
-                if (gl == 0) c.edges += e - s;
-            }
-            ms_td_expand<G, W>(ptr, adj, s, e, gl, fu, full, seen, next, levels, V, next_level, b0, b1, nq, counters, c);
-        }
-    }
+    const TdGrid L = {n_big, hub_ctas, n_mid, n_small, blocks_mid, blocks_small};
+    td_schedule<int>(ptr, cq, L, c.edges, [&](auto nt, int32_t u, int64_t s, int64_t e, int tid) {
+        const W fu = u >= 0 ? front[u] : (W)0;
+        ms_td_expand<decltype(nt)::value, W>(ptr, adj, s, e, tid, fu, full, seen, next, levels, V, next_level, b0, b1, nq, counters, c);
+    });
     ms_counts_flush(c, counters);
 }
 
 template <class W>
-__global__ void __launch_bounds__(BFS_MS_THREADS)
+__global__ void __launch_bounds__(BFS_THREADS)
 bfs_multi_bu_kernel(const int64_t *__restrict__ in_ptr, const int32_t *__restrict__ in_adj, int32_t V, const uint32_t *__restrict__ no_in_edges,
                     const W *__restrict__ front, W full, W *__restrict__ seen, W *__restrict__ next, int32_t *__restrict__ levels,
                     int32_t next_level, unsigned long long *counters)
@@ -373,8 +282,8 @@ __global__ void bfs_multi_init_kernel(MsSources S, int32_t V, int32_t *__restric
 }
 
 template <class W>
-static int bfs_multi_run(vglb_ctx *ctx, vglb_graph *g, const int32_t *h_sources, int32_t k, int32_t *d_levels, bool dopt,
-                         long long alpha, long long beta, W *seen, W *front_a, W *front_b, vglb_stats *stats)
+static int bfs_multi_run(vglb_ctx *ctx, vglb_graph *g, const int32_t *h_sources, int32_t k, int32_t *d_levels, const BfsDirection &dir,
+                         W *seen, W *front_a, W *front_b, vglb_stats *stats)
 {
     const int32_t V = g->V;
     const int32_t b0 = g->bfs_big_border_plus1 - 1, b1 = g->tier_border[1] > b0 ? g->tier_border[1] : b0;
@@ -383,14 +292,7 @@ static int bfs_multi_run(vglb_ctx *ctx, vglb_graph *g, const int32_t *h_sources,
     unsigned long long *d_cnt = (unsigned long long *)ctx->d_counters;
     unsigned long long *h_cnt = (unsigned long long *)ctx->h_counters;
     cudaStream_t st = ctx->stream;
-    auto regions = [&](int32_t *base) {
-        TierQueues q;
-        q.q[0] = base;
-        q.q[1] = base + b0;
-        q.q[2] = base + b1;
-        return q;
-    };
-    TierQueues cq = regions(g->d_queue[0]), nq = regions(g->d_queue[1]);
+    TierQueues cq = tier_regions(g->d_queue[0], b0, b1), nq = tier_regions(g->d_queue[1], b0, b1);
 
     // the sources: distinct vertices ascending, binned by tier; a vertex that is every row's source starts out full
     MsSources S;
@@ -436,27 +338,22 @@ static int bfs_multi_run(vglb_ctx *ctx, vglb_graph *g, const int32_t *h_sources,
     int64_t tot_edges = 0, tot_rows = 0, tot_frontier_bytes = 0, tot_pairs = k, levels_run = 0;
     int32_t bu_levels = 0;
     const int64_t w = sizeof(W);
-    const long long factor = (g->E / (V > 0 ? V : 1)) / 2 > 0 ? (g->E / V) / 2 : 1; // change_state.hpp:104
     const int max_blocks = ctx->sm_count * 16;
-    const int big_chunks = (int)ceil_div64(g->max_degree > 0 ? g->max_degree : 1, BFS_MS_BIG_CHUNK);
     int rc;
     while (n_cur > 0)
     {
         if (!bottom_up)
         {
-            const int blocks_mid = (int)min((int64_t)max_blocks, ceil_div64(n[1], BFS_MS_THREADS / 32));
-            const int blocks_small = (int)min((int64_t)max_blocks, ceil_div64(n[2], BFS_MS_THREADS / BFS_MS_SMALL_LANES));
-            const int hub_ctas = (int)min((int64_t)n[0] * big_chunks, (int64_t)ctx->sm_count * 4);
-            const int64_t grid = (int64_t)hub_ctas + blocks_mid + blocks_small;
-            bfs_multi_td_kernel<W><<<(unsigned)grid, BFS_MS_THREADS, 0, st>>>(g->d_out_ptr, g->d_out_adj, cq, n[0], hub_ctas, n[1], n[2],
-                                                                             blocks_mid, blocks_small, cur, full, seen, nxt, d_levels, V,
-                                                                             level + 1, b0, b1, nq, d_cnt);
+            const TdGrid L = td_grid(ctx, g, n);
+            bfs_multi_td_kernel<W><<<(unsigned)L.ctas(), BFS_THREADS, 0, st>>>(g->d_out_ptr, g->d_out_adj, cq, L.n_big, L.hub_ctas, L.n_mid,
+                                                                              L.n_small, L.blocks_mid, L.blocks_small, cur, full, seen, nxt,
+                                                                              d_levels, V, level + 1, b0, b1, nq, d_cnt);
             KERNEL_TRY();
             ctx->launches++;
         }
         else
         {
-            bfs_multi_bu_kernel<W><<<ctx->sm_count * 8, BFS_MS_THREADS, 0, st>>>(g->d_in_ptr, g->d_in_adj, V, (const uint32_t *)g->d_scratch_i32,
+            bfs_multi_bu_kernel<W><<<ctx->sm_count * 8, BFS_THREADS, 0, st>>>(g->d_in_ptr, g->d_in_adj, V, (const uint32_t *)g->d_scratch_i32,
                                                                                 cur, full, seen, nxt, d_levels, level + 1, d_cnt);
             KERNEL_TRY();
             ctx->launches++;
@@ -483,19 +380,7 @@ static int bfs_multi_run(vglb_ctx *ctx, vglb_graph *g, const int32_t *h_sources,
         m_f_next = (long long)h_cnt[C_MF];
         if (n_next == 0) break;
 
-        bool next_bu = bottom_up;
-        if (dopt)
-        {
-            const long long unvisited = (long long)V - full_total;
-            if (!bottom_up && n_cur < n_next)
-            {
-                if (m_f_next >= (unvisited * factor + V) / alpha) next_bu = true;
-            }
-            else if (bottom_up && n_cur >= n_next)
-            {
-                if (n_next < (unvisited * factor + V) / (factor * beta)) next_bu = false;
-            }
-        }
+        const bool next_bu = next_direction(dir, bottom_up, n_cur, n_next, m_f_next, (long long)V - full_total, V);
         CUDA_TRY(cudaMemsetAsync(d_cnt, 0, M_COUNT * 8, st));
         // Before a top-down level the target array must be all zero; a bottom-up level writes every word of its target.
         if (!bottom_up && !next_bu)
@@ -526,23 +411,15 @@ static int bfs_multi_run(vglb_ctx *ctx, vglb_graph *g, const int32_t *h_sources,
         n_cur = n_next;
         level++;
     }
-    CUDA_TRY(cudaEventRecord(ctx->ev_stop, st));
-    CUDA_TRY(cudaEventSynchronize(ctx->ev_stop));
-    if (stats)
-    {
-        float ms = 0.f;
-        CUDA_TRY(cudaEventElapsedTime(&ms, ctx->ev_start, ctx->ev_stop));
-        memset(stats, 0, sizeof(*stats));
-        stats->seconds = ms * 1e-3;
-        stats->iterations = levels_run;
-        stats->edges_inspected = tot_edges;
-        stats->vertices_processed = tot_rows;
-        stats->frontier_bytes = tot_frontier_bytes;
-        // the formula of include/vgl_b200.h (vglb_bfs_multi)
-        stats->algorithmic_bytes = (4 + w) * tot_edges + (12 + w) * tot_rows + tot_frontier_bytes + 4LL * k * V + 4 * tot_pairs;
-        stats->kernel_launches = ctx->launches - launches0;
-        stats->bottom_up_levels = bu_levels;
-    }
+    rc = vglb_finish_run(ctx, launches0, stats);
+    if (rc != VGLB_OK || !stats) return rc;
+    stats->iterations = levels_run;
+    stats->edges_inspected = tot_edges;
+    stats->vertices_processed = tot_rows;
+    stats->frontier_bytes = tot_frontier_bytes;
+    // the formula of include/vgl_b200.h (vglb_bfs_multi)
+    stats->algorithmic_bytes = (4 + w) * tot_edges + (12 + w) * tot_rows + tot_frontier_bytes + 4LL * k * V + 4 * tot_pairs;
+    stats->bottom_up_levels = bu_levels;
     return VGLB_OK;
 }
 
@@ -554,27 +431,15 @@ extern "C" int vglb_bfs_multi(vglb_ctx *ctx, vglb_graph *g, int32_t num_sources,
     VGLB_REQUIRE(g->comm == NULL, "vglb_bfs_multi: partitioned graphs are not supported");
     for (int i = 0; i < num_sources; i++)
         VGLB_REQUIRE(h_sources_sorted[i] >= 0 && h_sources_sorted[i] < g->V, "vglb_bfs_multi: source out of range");
-    const bool dopt = opts && opts->direction_optimising;
+    const BfsDirection dir = bfs_direction(opts, g->E, g->V);
     CUDA_TRY(cudaSetDevice(ctx->device));
-    if (dopt && !g->d_in_ptr)
+    if (dir.dopt && !g->d_in_ptr)
     {
         int rc_in = vglb_graph_derive_incoming(ctx, g); // as vglb_bfs: the bottom-up levels need the incoming CSR
         if (rc_in != VGLB_OK) return rc_in;
     }
-    const long long alpha = (opts && opts->alpha > 0) ? opts->alpha : 15;
-    const long long beta = (opts && opts->beta > 0) ? opts->beta : 18;
-    // the graph's BFS scratch, shared with vglb_bfs / vglb_sssp: only what is missing is allocated
-    for (int i = 0; i < 2; i++)
-        if (!g->d_queue[i]) CUDA_TRY(vglb_dev_alloc(&g->d_queue[i], ((size_t)g->V + 3) * 4));
-    int rc = bfs_prepare_no_in_edges(ctx, g);
+    int rc = bfs_prepare_queues(ctx, g);
     if (rc != VGLB_OK) return rc;
-    if (g->bfs_big_border_plus1 == 0) // first id with fewer than BFS_BIG_DEGREE edges, once per graph (shared with vglb_bfs)
-    {
-        int32_t border = 0;
-        rc = vglb_graph_threshold_vertex(ctx, g, BFS_BIG_DEGREE, &border);
-        if (rc != VGLB_OK) return rc;
-        g->bfs_big_border_plus1 = border + 1;
-    }
     // per-call word arrays from the context's allocation cache: seen | front_a | front_b, V words each
     const bool wide = num_sources > 32;
     const size_t wbytes = wide ? 8 : 4;
@@ -583,12 +448,12 @@ extern "C" int vglb_bfs_multi(vglb_ctx *ctx, vglb_graph *g, int32_t num_sources,
     if (wide)
     {
         unsigned long long *p = (unsigned long long *)words;
-        rc = bfs_multi_run<unsigned long long>(ctx, g, h_sources_sorted, num_sources, d_levels, dopt, alpha, beta, p, p + g->V, p + 2 * (size_t)g->V, stats);
+        rc = bfs_multi_run<unsigned long long>(ctx, g, h_sources_sorted, num_sources, d_levels, dir, p, p + g->V, p + 2 * (size_t)g->V, stats);
     }
     else
     {
         uint32_t *p = (uint32_t *)words;
-        rc = bfs_multi_run<uint32_t>(ctx, g, h_sources_sorted, num_sources, d_levels, dopt, alpha, beta, p, p + g->V, p + 2 * (size_t)g->V, stats);
+        rc = bfs_multi_run<uint32_t>(ctx, g, h_sources_sorted, num_sources, d_levels, dir, p, p + g->V, p + 2 * (size_t)g->V, stats);
     }
     if (rc != VGLB_OK) cudaStreamSynchronize(ctx->stream); // nothing may still use the block when it goes back to the cache
     vglb_dev_free(words);

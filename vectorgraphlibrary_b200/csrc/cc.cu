@@ -262,21 +262,13 @@ static int cc_partitioned(vglb_ctx *ctx, vglb_graph *g, int32_t *d_labels, vglb_
         ctx->launches++;
     }
     if (rows > 0) CUDA_TRY(cudaMemcpyAsync(d_labels, comp + g->col_of_row0, (size_t)rows * 4, cudaMemcpyDeviceToDevice, st));
-    CUDA_TRY(cudaEventRecord(ctx->ev_stop, st));
-    CUDA_TRY(cudaEventSynchronize(ctx->ev_stop));
-    if (stats)
-    {
-        float ms = 0.f;
-        CUDA_TRY(cudaEventElapsedTime(&ms, ctx->ev_start, ctx->ev_stop));
-        memset(stats, 0, sizeof(*stats));
-        stats->seconds = ms * 1e-3;
-        stats->iterations = hook_rounds;
-        stats->edges_inspected = hook_rounds * g->E;
-        stats->vertices_processed = hook_rounds * (int64_t)rows;
-        stats->frontier_bytes = hook_rounds * g->cols * 4 * 2; // the allreduced label vector
-        stats->algorithmic_bytes = hook_rounds * (8 * g->E + 12 * (int64_t)rows) + (hook_rounds - 1) * 8 * g->cols + stats->frontier_bytes;
-        stats->kernel_launches = ctx->launches - launches0;
-    }
+    rc = vglb_finish_run(ctx, launches0, stats);
+    if (rc != VGLB_OK || !stats) return rc;
+    stats->iterations = hook_rounds;
+    stats->edges_inspected = hook_rounds * g->E;
+    stats->vertices_processed = hook_rounds * (int64_t)rows;
+    stats->frontier_bytes = hook_rounds * g->cols * 4 * 2; // the allreduced label vector
+    stats->algorithmic_bytes = hook_rounds * (8 * g->E + 12 * (int64_t)rows) + (hook_rounds - 1) * 8 * g->cols + stats->frontier_bytes;
     return VGLB_OK;
 }
 
@@ -310,19 +302,11 @@ extern "C" int vglb_cc(vglb_ctx *ctx, vglb_graph *g, int32_t *d_labels, vglb_sta
         KERNEL_TRY();
         ctx->launches++;
     }
-    CUDA_TRY(cudaEventRecord(ctx->ev_stop, st));
-    CUDA_TRY(cudaEventSynchronize(ctx->ev_stop));
-    if (stats)
-    {
-        float ms = 0.f;
-        CUDA_TRY(cudaEventElapsedTime(&ms, ctx->ev_start, ctx->ev_stop));
-        memset(stats, 0, sizeof(*stats));
-        stats->seconds = ms * 1e-3;
-        stats->iterations = hook_rounds;
-        stats->edges_inspected = hook_rounds * g->E;
-        stats->vertices_processed = hook_rounds * (int64_t)V;
-        stats->algorithmic_bytes = hook_rounds * (8 * g->E + 12 * (int64_t)V) + (hook_rounds - 1) * 8 * (int64_t)V;
-        stats->kernel_launches = ctx->launches - launches0;
-    }
+    int rc = vglb_finish_run(ctx, launches0, stats);
+    if (rc != VGLB_OK || !stats) return rc;
+    stats->iterations = hook_rounds;
+    stats->edges_inspected = hook_rounds * g->E;
+    stats->vertices_processed = hook_rounds * (int64_t)V;
+    stats->algorithmic_bytes = hook_rounds * (8 * g->E + 12 * (int64_t)V) + (hook_rounds - 1) * 8 * (int64_t)V;
     return VGLB_OK;
 }

@@ -134,7 +134,6 @@ struct vglb_graph
     uint32_t *d_visited, *d_front_bm[2];
     int32_t *d_queue[2];
     int32_t *d_scratch_i32;
-    int bfs_ready;
     int32_t sssp_mid_rows_per_warp; // queue entries of the mid tier per warp (~2048 edges), set with the border
     int64_t cc_hub_edges_plus1;    // 0 = not read yet; else 1 + row pointer at tier_border[0] (cc.cu)
     int32_t bfs_big_border_plus1;  // 0 = not computed yet; else 1 + first id with fewer than BFS_BIG_DEGREE edges (bfs.cu)
@@ -175,6 +174,9 @@ constexpr int32_t vglb_tier_degree(int t)
 
 // copy `words` (<= 56) 8-byte counters from device memory to ctx->h_counters, ordered after everything enqueued on ctx->stream
 int vglb_counters_fetch(vglb_ctx *ctx, const void *d_src, int words);
+// end of a run timed from ctx->ev_start: records ev_stop on ctx->stream and waits for it; with stats, zeroes *stats and fills in
+// seconds and kernel_launches (launches since launches0). The algorithm fills in its own fields.
+int vglb_finish_run(vglb_ctx *ctx, int64_t launches0, vglb_stats *stats);
 int vglb_graph_compute_tiers(vglb_ctx *ctx, vglb_graph *g);
 void vglb_graph_set_unpartitioned(vglb_graph *g);
 int vglb_graph_derive_incoming(vglb_ctx *ctx, vglb_graph *g);

@@ -252,6 +252,19 @@ int vglb_counters_fetch(vglb_ctx *ctx, const void *d_src, int words)
     return VGLB_OK;
 }
 
+int vglb_finish_run(vglb_ctx *ctx, int64_t launches0, vglb_stats *stats)
+{
+    CUDA_TRY(cudaEventRecord(ctx->ev_stop, ctx->stream));
+    CUDA_TRY(cudaEventSynchronize(ctx->ev_stop));
+    if (!stats) return VGLB_OK;
+    float ms = 0.f;
+    CUDA_TRY(cudaEventElapsedTime(&ms, ctx->ev_start, ctx->ev_stop));
+    memset(stats, 0, sizeof(*stats));
+    stats->seconds = ms * 1e-3;
+    stats->kernel_launches = ctx->launches - launches0;
+    return VGLB_OK;
+}
+
 extern "C" void *vglb_stream(vglb_ctx *ctx) { return ctx ? (void *)ctx->stream : NULL; }
 
 extern "C" int vglb_malloc(vglb_ctx *ctx, size_t bytes, void **d_ptr)

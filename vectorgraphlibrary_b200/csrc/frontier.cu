@@ -530,3 +530,18 @@ extern "C" int vglb_reduce_max_i32(vglb_ctx *ctx, vglb_frontier *f, const int32_
     if (rc == VGLB_OK) *out = (int32_t)r;
     return rc;
 }
+
+// ---- the per-level counters of the partitioned BFS / SSSP drivers, staged for their allreduce -------------------------
+__global__ void stage_counters_kernel(unsigned long long *c)
+{
+    if (threadIdx.x < C_COUNT) c[C_COUNT + threadIdx.x] = c[threadIdx.x];
+    if (threadIdx.x == 0) c[2 * C_COUNT] = c[C_MF];
+}
+
+int vglb_stage_counters(vglb_ctx *ctx)
+{
+    stage_counters_kernel<<<1, 32, 0, ctx->stream>>>((unsigned long long *)ctx->d_counters);
+    KERNEL_TRY();
+    ctx->launches++;
+    return VGLB_OK;
+}

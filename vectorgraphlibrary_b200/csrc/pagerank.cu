@@ -1065,22 +1065,15 @@ extern "C" int vglb_pagerank_ex(vglb_ctx *ctx, vglb_graph *g, int iters, float d
             if (rc != VGLB_OK) return rc;
         }
     }
-    CUDA_TRY(cudaEventRecord(ctx->ev_stop, ctx->stream));
-    CUDA_TRY(cudaEventSynchronize(ctx->ev_stop));
+    rc = vglb_finish_run(ctx, launches0, stats);
+    if (rc != VGLB_OK) return rc;
     vglb_dev_free(d_ref_partial);
-    if (stats)
-    {
-        float ms = 0.f;
-        CUDA_TRY(cudaEventElapsedTime(&ms, ctx->ev_start, ctx->ev_stop));
-        memset(stats, 0, sizeof(*stats));
-        stats->seconds = ms * 1e-3;
-        stats->iterations = iters;
-        stats->edges_inspected = (int64_t)iters * g->E;
-        stats->vertices_processed = (int64_t)iters * V;
-        stats->algorithmic_bytes = (int64_t)iters * (8 * g->E + 16 * (int64_t)V) + (iters > 0 ? 4 * (int64_t)V : 0);
-        if (comm) stats->frontier_bytes = (int64_t)iters * g->cols * 4; // bytes of the vector every rank receives + sends
-        stats->kernel_launches = ctx->launches - launches0;
-    }
+    if (!stats) return VGLB_OK;
+    stats->iterations = iters;
+    stats->edges_inspected = (int64_t)iters * g->E;
+    stats->vertices_processed = (int64_t)iters * V;
+    stats->algorithmic_bytes = (int64_t)iters * (8 * g->E + 16 * (int64_t)V) + (iters > 0 ? 4 * (int64_t)V : 0);
+    if (comm) stats->frontier_bytes = (int64_t)iters * g->cols * 4; // bytes of the vector every rank receives + sends
     return VGLB_OK;
 }
 

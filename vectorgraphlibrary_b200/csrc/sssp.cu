@@ -133,11 +133,6 @@ sssp_part_frontier_kernel(const uint32_t *__restrict__ dist_slice, uint32_t *__r
     }
 }
 
-__global__ void sssp_copy_counters_kernel(unsigned long long *c)
-{
-    if (threadIdx.x < C_COUNT) c[C_COUNT + threadIdx.x] = c[threadIdx.x];
-}
-
 static int sssp_partitioned_dense(vglb_ctx *ctx, vglb_graph *g, const float *d_weights, int32_t source, float *d_dist,
                             vglb_stats *stats)
 {
@@ -155,14 +150,7 @@ static int sssp_partitioned_dense(vglb_ctx *ctx, vglb_graph *g, const float *d_w
     unsigned long long *h_cnt = (unsigned long long *)ctx->h_counters;
     cudaStream_t st = ctx->stream;
     uint32_t *dist = g->d_part_vec;
-    auto regions = [&](int32_t *base) {
-        TierQueues q;
-        q.q[0] = base;
-        q.q[1] = base + b0;
-        q.q[2] = base + b1;
-        return q;
-    };
-    TierQueues cq = regions(g->d_queue[0]), nq = regions(g->d_queue[1]);
+    TierQueues cq = tier_regions(g->d_queue[0], b0, b1), nq = tier_regions(g->d_queue[1], b0, b1);
 
     CUDA_TRY(cudaEventRecord(ctx->ev_start, st));
     const bool own_source = source / vp == rank;
@@ -199,9 +187,9 @@ static int sssp_partitioned_dense(vglb_ctx *ctx, vglb_graph *g, const float *d_w
                 dist + col0, g->d_part_prev, rows, b0, b1, nq, d_cnt);
             KERNEL_TRY();
         }
-        sssp_copy_counters_kernel<<<1, 32, 0, st>>>(d_cnt);
-        KERNEL_TRY();
-        ctx->launches += 2;
+        ctx->launches++;
+        rc = vglb_stage_counters(ctx);
+        if (rc != VGLB_OK) return rc;
         rc = vglb_comm_allreduce_async(comm, d_cnt + C_COUNT, C_COUNT, VGLB_DT_I64, VGLB_OP_SUM);
         if (rc != VGLB_OK) return rc;
         CUDA_TRY(cudaMemcpyAsync(h_cnt, d_cnt, 2 * C_COUNT * 8, cudaMemcpyDeviceToHost, st));
@@ -219,21 +207,13 @@ static int sssp_partitioned_dense(vglb_ctx *ctx, vglb_graph *g, const float *d_w
         TierQueues t = cq; cq = nq; nq = t;
     }
     if (rows > 0) CUDA_TRY(cudaMemcpyAsync(d_dist, dist + col0, (size_t)rows * 4, cudaMemcpyDeviceToDevice, st));
-    CUDA_TRY(cudaEventRecord(ctx->ev_stop, st));
-    CUDA_TRY(cudaEventSynchronize(ctx->ev_stop));
-    if (stats)
-    {
-        float ms = 0.f;
-        CUDA_TRY(cudaEventElapsedTime(&ms, ctx->ev_start, ctx->ev_stop));
-        memset(stats, 0, sizeof(*stats));
-        stats->seconds = ms * 1e-3;
-        stats->iterations = rounds;
-        stats->edges_inspected = tot_edges; // this rank's
-        stats->vertices_processed = tot_rows;
-        stats->frontier_bytes = 8 * tot_next + rounds * g->cols * 4 * 2; // queues + the allreduced vector (read + written)
-        stats->algorithmic_bytes = 12 * tot_edges + 24 * tot_rows + stats->frontier_bytes;
-        stats->kernel_launches = ctx->launches - launches0;
-    }
+    rc = vglb_finish_run(ctx, launches0, stats);
+    if (rc != VGLB_OK || !stats) return rc;
+    stats->iterations = rounds;
+    stats->edges_inspected = tot_edges; // this rank's
+    stats->vertices_processed = tot_rows;
+    stats->frontier_bytes = 8 * tot_next + rounds * g->cols * 4 * 2; // queues + the allreduced vector (read + written)
+    stats->algorithmic_bytes = 12 * tot_edges + 24 * tot_rows + stats->frontier_bytes;
     return VGLB_OK;
 }
 
@@ -774,13 +754,6 @@ __global__ void sssp_part_seed_kernel(uint32_t *__restrict__ dist, int64_t cols,
     if (blockIdx.x == 0 && threadIdx.x == 0 && src_row >= 0) near_bm[src_row >> 5] = 1u << (src_row & 31);
 }
 
-// counters [0, C_COUNT) -> [C_COUNT, 2 C_COUNT) (summed over ranks) and the pending minimum -> slot 2 C_COUNT (max over ranks)
-__global__ void sssp_stage_counters_kernel(unsigned long long *c)
-{
-    if (threadIdx.x < C_COUNT) c[C_COUNT + threadIdx.x] = c[threadIdx.x];
-    if (threadIdx.x == 0) c[2 * C_COUNT] = c[C_MF];
-}
-
 // Schedule. The reference relaxes the out-edges of EVERY vertex whose distance changed in the previous round
 // (shortest_paths.hpp:40-66); on the BASELINE graph that re-relaxes each edge ~5.8 times. The fixed point does not
 // depend on the schedule, so the frontier is split near/far: only due vertices with dist < threshold are relaxed; when
@@ -845,10 +818,7 @@ static int sssp_run(vglb_ctx *ctx, vglb_graph *g, const float *d_weights, int32_
     unsigned long long *h_cnt = (unsigned long long *)ctx->h_counters;
     cudaStream_t st = ctx->stream;
     uint32_t *near_bm = g->d_visited, *far_bm = g->d_front_bm[0];
-    TierQueues cq;
-    cq.q[0] = g->d_queue[0];
-    cq.q[1] = g->d_queue[0] + b0;
-    cq.q[2] = g->d_queue[0] + b1;
+    TierQueues cq = tier_regions(g->d_queue[0], b0, b1);
     int rc;
 
     CUDA_TRY(cudaEventRecord(ctx->ev_start, st));
@@ -924,9 +894,8 @@ static int sssp_run(vglb_ctx *ctx, vglb_graph *g, const float *d_weights, int32_
         far_selects += from_far;
         if (part)
         {
-            sssp_stage_counters_kernel<<<1, 32, 0, st>>>(d_cnt);
-            KERNEL_TRY();
-            ctx->launches++;
+            rc = vglb_stage_counters(ctx);
+            if (rc != VGLB_OK) return rc;
             rc = vglb_comm_allreduce_async(comm, d_cnt + C_COUNT, C_COUNT, VGLB_DT_I64, VGLB_OP_SUM);
             if (rc != VGLB_OK) return rc;
         }
@@ -1058,24 +1027,16 @@ static int sssp_run(vglb_ctx *ctx, vglb_graph *g, const float *d_weights, int32_
         tot_next += n_local;
     }
     if (part && rows > 0) CUDA_TRY(cudaMemcpyAsync(d_dist, dist + col0, (size_t)rows * 4, cudaMemcpyDeviceToDevice, st));
-    CUDA_TRY(cudaEventRecord(ctx->ev_stop, st));
-    CUDA_TRY(cudaEventSynchronize(ctx->ev_stop));
-    if (stats)
-    {
-        float ms = 0.f;
-        CUDA_TRY(cudaEventElapsedTime(&ms, ctx->ev_start, ctx->ev_stop));
-        memset(stats, 0, sizeof(*stats));
-        stats->seconds = ms * 1e-3;
-        stats->iterations = rounds;
-        stats->edges_inspected = tot_edges;
-        stats->vertices_processed = tot_rows;
-        // queues, bitmap scans, far-pile distance reads; partitioned: + the changed-bitmap scan of every round and, per
-        // update received, 8 bytes written by the sender + 8 read over NVLink + the owner's 12-byte read-modify-write
-        stats->frontier_bytes = 8 * tot_next + selects * (int64_t)words * 4 + far_selects * 4 * (int64_t)rows
-                                + (part ? rounds * (int64_t)words_full * 4 + 28 * tot_pulled : 0);
-        stats->algorithmic_bytes = 12 * tot_edges + 24 * tot_rows + stats->frontier_bytes; // SURVEY §8(d)
-        stats->kernel_launches = ctx->launches - launches0;
-    }
+    rc = vglb_finish_run(ctx, launches0, stats);
+    if (rc != VGLB_OK || !stats) return rc;
+    stats->iterations = rounds;
+    stats->edges_inspected = tot_edges;
+    stats->vertices_processed = tot_rows;
+    // queues, bitmap scans, far-pile distance reads; partitioned: + the changed-bitmap scan of every round and, per
+    // update received, 8 bytes written by the sender + 8 read over NVLink + the owner's 12-byte read-modify-write
+    stats->frontier_bytes = 8 * tot_next + selects * (int64_t)words * 4 + far_selects * 4 * (int64_t)rows
+                            + (part ? rounds * (int64_t)words_full * 4 + 28 * tot_pulled : 0);
+    stats->algorithmic_bytes = 12 * tot_edges + 24 * tot_rows + stats->frontier_bytes; // SURVEY §8(d)
     return VGLB_OK;
 }
 
