@@ -128,6 +128,33 @@ def test_partitioned_drivers_single_rank_nccl(vgl, ctx, oracle, golden):
     comm.close()
 
 
+def test_partitioned_csr_upload_rejects_bad_part(vgl, ctx, oracle):
+    """The upload checks the caller's part on the device and rejects it before anything indexes with it; the verdict and
+    the edge count come out of the same allreduce."""
+    scale, ef = 10, 8
+    V = 1 << scale
+    src, dst = oracle.generate_edges(oracle.GEN_RMAT, scale, ef)
+    comm = vgl.Comm(ctx, 0, 1)
+    G = vgl.Graph.from_edges_partitioned(ctx, comm, V, src, dst)
+    ptr, adj = G.layout()
+    fwd = G.orig_to_sorted()
+    assert ptr[1] < ptr[2]
+    bad_ptr = ptr.copy()
+    bad_ptr[1], bad_ptr[2] = ptr[2], ptr[1]
+    bad_adj = adj.copy()
+    bad_adj[0] = G.cols
+    bad_fwd = fwd.copy()
+    bad_fwd[1] = fwd[0]
+    for p, a, f in ((bad_ptr, adj, fwd), (ptr, bad_adj, fwd), (ptr, adj, bad_fwd)):
+        with pytest.raises(vgl.VglbError, match="this rank's part is not a CSR"):
+            vgl.Graph.from_csr_partitioned(ctx, comm, V, p, a, f)
+    H = vgl.Graph.from_csr_partitioned(ctx, comm, V, ptr, adj, fwd)
+    assert H.E_global == G.E_global == len(src)
+    H.free()
+    G.free()
+    comm.close()
+
+
 @pytest.mark.parametrize("world,dense", [(2, False), (2, True)])
 def test_partitioned_drivers_multi_gpu(vgl, world, dense):
     """torchrun, one process per GPU; every rank checks the whole result against the golden fixtures — with the CUDA IPC

@@ -659,15 +659,11 @@ static int bfs_partitioned_bitmaps(vglb_ctx *ctx, vglb_graph *g, int32_t source,
         bfs_or_kernel<<<(unsigned)min((int64_t)max_blocks, ceil_div64(words, 256)), 256, 0, st>>>(visited, next_bm, words);
         KERNEL_TRY();
         ctx->launches++;
-        rc = vglb_stage_counters(ctx);
+        rc = vglb_part_round_counters(ctx, comm, 2 * C_COUNT);
         if (rc != VGLB_OK) return rc;
-        rc = vglb_comm_allreduce_async(comm, d_cnt + C_COUNT, C_COUNT, VGLB_DT_I64, VGLB_OP_SUM);
-        if (rc != VGLB_OK) return rc;
-        CUDA_TRY(cudaMemcpyAsync(h_cnt, d_cnt, 2 * C_COUNT * 8, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
         CUDA_TRY(cudaMemsetAsync(d_cnt, 0, 2 * C_COUNT * 8, st));
         levels_run++;
-        const unsigned long long *gl = h_cnt + C_COUNT; // global sums
+        const unsigned long long *gl = h_cnt + C_STAGED; // global sums
         const long long n_next = (long long)gl[C_FOUND];
         if (trace)
         {
@@ -697,7 +693,7 @@ static int bfs_partitioned_bitmaps(vglb_ctx *ctx, vglb_graph *g, int32_t source,
                 ctx->launches++;
                 CUDA_TRY(cudaMemcpyAsync(h_cnt, d_cnt, 3 * 8, cudaMemcpyDeviceToHost, st));
                 CUDA_TRY(cudaStreamSynchronize(st));
-                n[0] = (int32_t)h_cnt[0]; n[1] = (int32_t)h_cnt[1]; n[2] = (int32_t)h_cnt[2];
+                n[0] = (int32_t)h_cnt[C_NEXT_BIG]; n[1] = (int32_t)h_cnt[C_NEXT_MID]; n[2] = (int32_t)h_cnt[C_NEXT_SMALL];
                 CUDA_TRY(cudaMemsetAsync(d_cnt, 0, 2 * C_COUNT * 8, st));
             }
         }
@@ -753,7 +749,7 @@ static int bfs_partitioned(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t
     A.P = P;
     A.rank = rank;
     A.lists = (unsigned long long *)g->d_part_lists;
-    const unsigned long long **d_peer_table = (const unsigned long long **)(ctx->d_counters + 24); // 8 device pointers
+    const unsigned long long **d_peer_table = (const unsigned long long **)(ctx->d_counters + CTR_PEER_TABLE);
     CUDA_TRY(cudaMemcpyAsync(d_peer_table, g->d_vec_peer, sizeof(g->d_vec_peer), cudaMemcpyHostToDevice, st));
 
     CUDA_TRY(cudaEventRecord(ctx->ev_start, st));
@@ -802,7 +798,7 @@ static int bfs_partitioned(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t
             }
             // barrier: every rank's lists are complete before anybody reads them; they are not reset before every rank has
             // passed this level's counter allreduce, i.e. finished reading
-            rc = vglb_comm_allreduce_async(comm, d_cnt + 2 * C_COUNT + 2, 1, VGLB_DT_I64, VGLB_OP_SUM);
+            rc = vglb_comm_allreduce_async(comm, d_cnt + CTR_LIST_BARRIER, 1, VGLB_DT_I64, VGLB_OP_SUM);
             if (rc != VGLB_OK) return rc;
             bfs_apply_lists_kernel<<<ctx->sm_count * 4, 256, 0, st>>>(d_peer_table, A, g->d_out_ptr, visited, d_levels, level + 1, b0, b1, nq, d_cnt);
             KERNEL_TRY();
@@ -822,15 +818,11 @@ static int bfs_partitioned(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t
             bu_levels++;
             tot_frontier_bytes += (int64_t)wslice * 4 * 3 + words * 4 * 3;
         }
-        rc = vglb_stage_counters(ctx);
+        rc = vglb_part_round_counters(ctx, comm, 2 * C_COUNT);
         if (rc != VGLB_OK) return rc;
-        rc = vglb_comm_allreduce_async(comm, d_cnt + C_COUNT, C_COUNT, VGLB_DT_I64, VGLB_OP_SUM);
-        if (rc != VGLB_OK) return rc;
-        CUDA_TRY(cudaMemcpyAsync(h_cnt, d_cnt, 2 * C_COUNT * 8, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
         CUDA_TRY(cudaMemsetAsync(d_cnt, 0, 2 * C_COUNT * 8, st));
         levels_run++;
-        const unsigned long long *gl = h_cnt + C_COUNT; // whole-job sums
+        const unsigned long long *gl = h_cnt + C_STAGED; // whole-job sums
         const int32_t nn[3] = {(int32_t)h_cnt[C_NEXT_BIG], (int32_t)h_cnt[C_NEXT_MID], (int32_t)h_cnt[C_NEXT_SMALL]};
         const long long n_next = bottom_up ? (long long)gl[C_FOUND] : (long long)(gl[C_NEXT_BIG] + gl[C_NEXT_MID] + gl[C_NEXT_SMALL]);
         if (trace)
@@ -881,7 +873,7 @@ static int bfs_partitioned(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t
             ctx->launches++;
             CUDA_TRY(cudaMemcpyAsync(h_cnt, d_cnt, 3 * 8, cudaMemcpyDeviceToHost, st));
             CUDA_TRY(cudaStreamSynchronize(st));
-            n[0] = (int32_t)h_cnt[0]; n[1] = (int32_t)h_cnt[1]; n[2] = (int32_t)h_cnt[2];
+            n[0] = (int32_t)h_cnt[C_NEXT_BIG]; n[1] = (int32_t)h_cnt[C_NEXT_MID]; n[2] = (int32_t)h_cnt[C_NEXT_SMALL];
             CUDA_TRY(cudaMemsetAsync(d_cnt, 0, 2 * C_COUNT * 8, st));
         }
         bottom_up = next_bu;
@@ -1069,7 +1061,7 @@ extern "C" int vglb_bfs(vglb_ctx *ctx, vglb_graph *g, int32_t source, int32_t *d
             ctx->launches++;
             rc = vglb_counters_fetch(ctx, d_cnt, 3);
             if (rc != VGLB_OK) return rc;
-            n[0] = (int32_t)h_cnt[0]; n[1] = (int32_t)h_cnt[1]; n[2] = (int32_t)h_cnt[2];
+            n[0] = (int32_t)h_cnt[C_NEXT_BIG]; n[1] = (int32_t)h_cnt[C_NEXT_MID]; n[2] = (int32_t)h_cnt[C_NEXT_SMALL];
             CUDA_TRY(cudaMemsetAsync(d_cnt, 0, C_COUNT * 8, st));
             tot_frontier_bytes += (int64_t)words * 4 + 4 * n_next;
         }

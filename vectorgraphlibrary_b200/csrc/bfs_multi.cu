@@ -27,14 +27,6 @@
 #define BFS_MS_PROBE_MAX 16   // lane-private in-neighbours before the warp takes the row over
 #define BFS_MS_LONG_UNROLL 8  // in-neighbours per lane and round trip when the warp scans one row
 
-// counter slots: the vglb_bfs slots of frontier.cuh, then two of this file
-enum
-{
-    M_PAIRS = C_COUNT,  // (vertex, source) pairs reached this level = level stores
-    M_FULL = C_COUNT + 1, // vertices whose seen word became full this level
-    M_COUNT = C_COUNT + 2
-};
-
 template <class W> __device__ __forceinline__ int word_popc(W x);
 template <> __device__ __forceinline__ int word_popc<uint32_t>(uint32_t x) { return __popc(x); }
 template <> __device__ __forceinline__ int word_popc<unsigned long long>(unsigned long long x) { return __popcll(x); }
@@ -399,7 +391,7 @@ static int bfs_multi_run(vglb_ctx *ctx, vglb_graph *g, const int32_t *h_sources,
             ctx->launches++;
             rc = vglb_counters_fetch(ctx, d_cnt, 3);
             if (rc != VGLB_OK) return rc;
-            n[0] = (int32_t)h_cnt[0]; n[1] = (int32_t)h_cnt[1]; n[2] = (int32_t)h_cnt[2];
+            n[0] = (int32_t)h_cnt[C_NEXT_BIG]; n[1] = (int32_t)h_cnt[C_NEXT_MID]; n[2] = (int32_t)h_cnt[C_NEXT_SMALL];
             CUDA_TRY(cudaMemsetAsync(d_cnt, 0, M_COUNT * 8, st));
             CUDA_TRY(cudaMemsetAsync(cur, 0, (size_t)V * w, st));
             tot_frontier_bytes += (int64_t)V * 2 * w + 4 * n_next;

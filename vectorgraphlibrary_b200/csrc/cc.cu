@@ -233,8 +233,8 @@ static int cc_partitioned(vglb_ctx *ctx, vglb_graph *g, int32_t *d_labels, vglb_
     const int64_t launches0 = ctx->launches;
     const int32_t rows = g->V, P = g->part_world, vp = g->vp;
     cudaStream_t st = ctx->stream;
-    int *d_changed = (int *)(ctx->d_counters + 40);
-    int *h_changed = (int *)(ctx->h_counters + 40);
+    int *d_changed = (int *)(ctx->d_counters + CTR_CC_CHANGED);
+    int *h_changed = (int *)(ctx->h_counters + CTR_CC_CHANGED);
     if (!g->d_part_vec) CUDA_TRY(vglb_dev_alloc(&g->d_part_vec, (size_t)g->cols * 4));
     int32_t *comp = (int32_t *)g->d_part_vec;
 
@@ -280,8 +280,8 @@ extern "C" int vglb_cc(vglb_ctx *ctx, vglb_graph *g, int32_t *d_labels, vglb_sta
     const int64_t launches0 = ctx->launches;
     const int32_t V = g->V;
     cudaStream_t st = ctx->stream;
-    int *d_changed = (int *)(ctx->d_counters + 40);
-    int *h_changed = (int *)(ctx->h_counters + 40);
+    int *d_changed = (int *)(ctx->d_counters + CTR_CC_CHANGED);
+    int *h_changed = (int *)(ctx->h_counters + CTR_CC_CHANGED);
 
 
     CUDA_TRY(cudaEventRecord(ctx->ev_start, st));

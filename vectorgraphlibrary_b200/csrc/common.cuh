@@ -58,21 +58,76 @@ struct vglb_ctx
     cudaStream_t copy_stream;   // host -> device uploads that overlap kernels on `stream` (vglb_graph_from_csr)
     cudaEvent_t ev_chunk[8];
     cudaEvent_t ev_start, ev_stop;
-    // host-visible scratch for counters read back once per level / round
-    int64_t *h_counters;   // pinned, 64 x int64
-    int64_t *d_counters;   // device, 64 x int64
+    // host-visible scratch for counters read back once per level / round (layout: CTR_* below)
+    int64_t *h_counters;   // pinned, CTR_WORDS x int64
+    int64_t *d_counters;   // device, CTR_WORDS x int64
     void *d_flush;         // L2 flush buffer
     size_t flush_bytes;
     int64_t launches;      // kernels launched since the last reset (gpu_launches evidence)
     // counter mailbox: pinned host memory mapped into the device; a 1-warp kernel at the end of a round copies the round's
     // counters there and raises a sequence number the host spins on (vglb_counters_fetch) — a level / round boundary costs a
     // PCIe write instead of cudaMemcpyAsync + cudaStreamSynchronize
-    unsigned long long *h_mailbox; // 64 words, word 63 = sequence number
+    unsigned long long *h_mailbox; // CTR_WORDS words, word MAILBOX_SEQ = sequence number
     unsigned long long mailbox_seq;
     int pr_carveout_set;   // the PageRank sweep kernels' shared-memory carve-out preferences have been set on this device
     int upload_hint;       // VGLB_HINT_* (vglb_set_upload_hint)
     int prb_smem_set;      // pr_bin_kernel's dynamic shared-memory limit has been raised on this device
 };
+
+// The words (8 bytes each) of the counter block ctx->d_counters and its pinned host copy ctx->h_counters. Every user of the
+// block names its words here; a word without a name is free. Two names on one word are users that never run together.
+enum
+{
+    // level / round counters of BFS, multi-source BFS and SSSP (u64): the level's kernels add to them, the driver clears
+    // them before the first level and again after each read-back
+    C_NEXT_BIG = 0,   // rows queued for the next level, per tier
+    C_NEXT_MID = 1,
+    C_NEXT_SMALL = 2,
+    C_EDGES = 3,      // edges inspected this level
+    C_FOUND = 4,      // vertices discovered this level
+    C_MF = 5,         // sum of out-degrees of the next frontier
+    C_ROWS = 6,       // rows whose pointer pair was read this level
+    C_COUNT = 8,
+    // int32 scratch of graph set-up (the tier borders of vglb_graph_compute_tiers, the vertex of
+    // vglb_graph_threshold_vertex): used outside any run only, so it shares the level counters; both zero it again
+    // afterwards, because a run expects its counters at 0
+    CTR_SCRATCH_I32 = 0,
+    // a partitioned level's counters, copied by the staging kernel and summed over the ranks (vglb_part_round_counters)
+    C_STAGED = C_COUNT,
+    // multi-source BFS level counters (u64). vglb_bfs_multi rejects partitioned graphs, so they share the staged copy
+    M_PAIRS = C_STAGED,     // (vertex, source) pairs reached this level = level stores
+    M_FULL = M_PAIRS + 1,   // vertices whose seen word became full this level
+    M_COUNT = M_FULL + 1,
+    // SSSP: complement of this rank's smallest pending distance (u64), C_MF copied by the staging kernel every round
+    CTR_PENDING_MIN = C_STAGED + C_COUNT,
+    CTR_SSSP_ROUND = CTR_PENDING_MIN + 1, // words an SSSP round reads back
+    // partitioned BFS / SSSP: one-word allreduce that is the barrier of the discovery / update list exchange (value unused)
+    CTR_LIST_BARRIER = CTR_PENDING_MIN + 2,
+    // SSSP drain results (u64, written by sssp_drain_kernel). The drain never runs on a partitioned graph, so DR_REASON
+    // shares the list barrier
+    DR_REASON = CTR_LIST_BARRIER,
+    DR_ROUNDS,
+    DR_ROWS,
+    DR_END,
+    // partitioned BFS / SSSP: the peers' update lists (g->d_vec_peer, 8 device pointers), copied in before the run
+    CTR_PEER_TABLE = 24,
+    CTR_REDUCE = 32,         // vglb_reduce_*: the frontier reduce result (i64 or f64)
+    CTR_CC_CHANGED = 40,     // CC: a hook changed a label this round (int32, device and host)
+    CTR_HOST_ALLREDUCE = 52, // vglb_comm_allreduce_host: up to two 8-byte host values on their way through the allreduce
+    CTR_BAD = 56,            // CSR / label validation: a check failed (int32)
+    CTR_VERIFY_COUNT = 57,   // vglb_verify_*: mismatches (u64)
+    CTR_VERIFY_SUMS = 58,    // vglb_verify_ranking_f32: two f64 sums
+    CTR_SSSP_WMAX = 60,      // SSSP: the largest sampled weight (u32 bits of a float)
+    CTR_WORDS = 64,          // size of the block, and of the mailbox
+    MAILBOX_WORDS = 56,      // vglb_counters_fetch copies at most this many words
+    MAILBOX_SEQ = 63         // mailbox word that carries the sequence number
+};
+static_assert(DR_END <= CTR_PEER_TABLE && CTR_REDUCE < CTR_CC_CHANGED && CTR_CC_CHANGED < CTR_HOST_ALLREDUCE &&
+                  CTR_HOST_ALLREDUCE + 2 <= CTR_BAD && CTR_VERIFY_SUMS + 2 <= CTR_SSSP_WMAX && CTR_SSSP_WMAX < CTR_WORDS &&
+                  MAILBOX_WORDS < MAILBOX_SEQ && MAILBOX_SEQ < CTR_WORDS,
+              "counter slots in order, each inside the block");
+static_assert(C_COUNT <= MAILBOX_WORDS && CTR_SSSP_ROUND <= MAILBOX_WORDS && DR_END <= MAILBOX_WORDS && M_COUNT <= MAILBOX_WORDS,
+              "every run read through the mailbox fits it");
 
 struct vglb_graph
 {
@@ -139,6 +194,7 @@ struct vglb_graph
     int32_t bfs_big_border_plus1;  // 0 = not computed yet; else 1 + first id with fewer than BFS_BIG_DEGREE edges (bfs.cu)
     int32_t sssp_big_border_plus1; // 0 = not computed yet; else 1 + first id with fewer than 512 edges (sssp.cu)
 };
+static_assert(sizeof(vglb_graph::d_vec_peer) <= (CTR_REDUCE - CTR_PEER_TABLE) * 8, "the peer table holds d_vec_peer");
 
 // NCCL communicator of one rank (partition.cu); the library dlopen()s libnccl.so.2 on first use
 struct vglb_comm
@@ -172,7 +228,7 @@ constexpr int32_t vglb_tier_degree(int t)
     return t == 0 ? 4096 : t == 1 ? 32 : t == 2 ? 16 : t == 3 ? 8 : t == 4 ? 4 : t == 5 ? 2 : t == 6 ? 1 : 0;
 }
 
-// copy `words` (<= 56) 8-byte counters from device memory to ctx->h_counters, ordered after everything enqueued on ctx->stream
+// copy `words` (<= MAILBOX_WORDS) 8-byte counters from device memory to ctx->h_counters, ordered after everything enqueued on ctx->stream
 int vglb_counters_fetch(vglb_ctx *ctx, const void *d_src, int words);
 // end of a run timed from ctx->ev_start: records ev_stop on ctx->stream and waits for it; with stats, zeroes *stats and fills in
 // seconds and kernel_launches (launches since launches0). The algorithm fills in its own fields.
@@ -191,6 +247,8 @@ enum { VGLB_DT_I32 = 0, VGLB_DT_U32 = 1, VGLB_DT_I64 = 2, VGLB_DT_F64 = 3 };
 enum { VGLB_OP_SUM = 0, VGLB_OP_MIN = 1, VGLB_OP_MAX = 2 };
 int vglb_comm_allgather_async(vglb_comm *comm, void *d_buf, size_t bytes_per_rank);
 int vglb_comm_allreduce_async(vglb_comm *comm, void *d_buf, size_t count, int dtype, int op);
+// allreduce of `count` host values (at most 16 bytes) through CTR_HOST_ALLREDUCE; waits, and leaves the result in h_inout
+int vglb_comm_allreduce_host(vglb_comm *comm, void *h_inout, int count, int dtype, int op);
 int vglb_comm_alltoall_async(vglb_comm *comm, const void *d_send, void *d_recv, size_t bytes_per_rank);
 int vglb_comm_ipc_map(vglb_comm *comm, void *d_local, void **peers /* [world] */);
 int vglb_part_map_lists(vglb_ctx *ctx, vglb_graph *g);

@@ -180,12 +180,12 @@ extern "C" int vglb_init(int device, vglb_ctx **out_ctx)
     for (int i = 0; i < 8; i++) CUDA_TRY(cudaEventCreateWithFlags(&ctx->ev_chunk[i], cudaEventDisableTiming));
     CUDA_TRY(cudaEventCreate(&ctx->ev_start));
     CUDA_TRY(cudaEventCreate(&ctx->ev_stop));
-    CUDA_TRY(cudaMallocHost((void **)&ctx->h_counters, 64 * sizeof(int64_t)));
-    CUDA_TRY(cudaHostAlloc((void **)&ctx->h_mailbox, 64 * sizeof(unsigned long long), cudaHostAllocMapped));
-    memset(ctx->h_mailbox, 0, 64 * sizeof(unsigned long long));
+    CUDA_TRY(cudaMallocHost((void **)&ctx->h_counters, CTR_WORDS * sizeof(int64_t)));
+    CUDA_TRY(cudaHostAlloc((void **)&ctx->h_mailbox, CTR_WORDS * sizeof(unsigned long long), cudaHostAllocMapped));
+    memset(ctx->h_mailbox, 0, CTR_WORDS * sizeof(unsigned long long));
     ctx->mailbox_seq = 0;
-    CUDA_TRY(vglb_dev_alloc((void **)&ctx->d_counters, 64 * sizeof(int64_t)));
-    CUDA_TRY(cudaMemset(ctx->d_counters, 0, 64 * sizeof(int64_t)));
+    CUDA_TRY(vglb_dev_alloc((void **)&ctx->d_counters, CTR_WORDS * sizeof(int64_t)));
+    CUDA_TRY(cudaMemset(ctx->d_counters, 0, CTR_WORDS * sizeof(int64_t)));
     ctx->flush_bytes = ctx->l2_bytes * 2 > (size_t)(256u << 20) ? ctx->l2_bytes * 2 : (size_t)(256u << 20);
     ctx->d_flush = NULL;
     *out_ctx = ctx;
@@ -225,16 +225,16 @@ __global__ void counters_publish_kernel(const unsigned long long *__restrict__ s
     if ((int)threadIdx.x < words) mailbox[threadIdx.x] = src[threadIdx.x];
     __threadfence_system();
     __syncthreads();
-    if (threadIdx.x == 0) mailbox[63] = seq;
+    if (threadIdx.x == 0) mailbox[MAILBOX_SEQ] = seq;
 }
 
 int vglb_counters_fetch(vglb_ctx *ctx, const void *d_src, int words)
 {
-    VGLB_REQUIRE(words > 0 && words <= 56, "vglb_counters_fetch: at most 56 counters");
+    VGLB_REQUIRE(words > 0 && words <= MAILBOX_WORDS, "vglb_counters_fetch: at most 56 counters");
     const unsigned long long seq = ++ctx->mailbox_seq;
-    counters_publish_kernel<<<1, 64, 0, ctx->stream>>>((const unsigned long long *)d_src, words, ctx->h_mailbox, seq);
+    counters_publish_kernel<<<1, CTR_WORDS, 0, ctx->stream>>>((const unsigned long long *)d_src, words, ctx->h_mailbox, seq);
     KERNEL_TRY();
-    volatile unsigned long long *flag = ctx->h_mailbox + 63;
+    volatile unsigned long long *flag = ctx->h_mailbox + MAILBOX_SEQ;
     for (unsigned spins = 1;; spins++)
     {
         if (*flag == seq) break;

@@ -42,6 +42,7 @@ enum
     G_TIER2 = 5,
     G_COUNT = 8
 };
+static_assert((int)G_COUNT <= (int)MAILBOX_WORDS, "gnf_run reads its counters through the mailbox");
 
 struct PredFlags
 {
@@ -491,7 +492,7 @@ template <int OP>
 static int reduce_run(vglb_ctx *ctx, vglb_frontier *f, const void *d_values, void *h_out8)
 {
     CUDA_TRY(cudaSetDevice(ctx->device));
-    unsigned long long *d_out = (unsigned long long *)ctx->d_counters + 32;
+    unsigned long long *d_out = (unsigned long long *)ctx->d_counters + CTR_REDUCE;
     long long init = OP == RED_MAX_I32 ? (long long)INT32_MIN : 0;
     double initf = 0.0;
     CUDA_TRY(cudaMemcpyAsync(d_out, OP == RED_SUM_F32 ? (void *)&initf : (void *)&init, 8, cudaMemcpyHostToDevice, ctx->stream));
@@ -534,14 +535,18 @@ extern "C" int vglb_reduce_max_i32(vglb_ctx *ctx, vglb_frontier *f, const int32_
 // ---- the per-level counters of the partitioned BFS / SSSP drivers, staged for their allreduce -------------------------
 __global__ void stage_counters_kernel(unsigned long long *c)
 {
-    if (threadIdx.x < C_COUNT) c[C_COUNT + threadIdx.x] = c[threadIdx.x];
-    if (threadIdx.x == 0) c[2 * C_COUNT] = c[C_MF];
+    if (threadIdx.x < C_COUNT) c[C_STAGED + threadIdx.x] = c[threadIdx.x];
+    if (threadIdx.x == 0) c[CTR_PENDING_MIN] = c[C_MF];
 }
 
-int vglb_stage_counters(vglb_ctx *ctx)
+int vglb_part_round_counters(vglb_ctx *ctx, vglb_comm *comm, int words)
 {
     stage_counters_kernel<<<1, 32, 0, ctx->stream>>>((unsigned long long *)ctx->d_counters);
     KERNEL_TRY();
     ctx->launches++;
+    int rc = vglb_comm_allreduce_async(comm, ctx->d_counters + C_STAGED, C_COUNT, VGLB_DT_I64, VGLB_OP_SUM);
+    if (rc != VGLB_OK) return rc;
+    CUDA_TRY(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, (size_t)words * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return VGLB_OK;
 }

@@ -6,19 +6,6 @@
 
 #include "common.cuh"
 
-// counter slots (unsigned long long) in ctx->d_counters
-enum
-{
-    C_NEXT_BIG = 0,
-    C_NEXT_MID = 1,
-    C_NEXT_SMALL = 2,
-    C_EDGES = 3,   // edges inspected this level
-    C_FOUND = 4,   // vertices discovered this level
-    C_MF = 5,      // sum of out-degrees of the next frontier
-    C_ROWS = 6,    // rows whose pointer pair was read this level
-    C_COUNT = 8
-};
-
 struct TierQueues
 {
     int32_t *q[3];       // big / mid / small regions
@@ -276,6 +263,7 @@ int bfs_prepare_no_in_edges(vglb_ctx *ctx, vglb_graph *g);
 // mask and g->bfs_big_border_plus1 (bfs.cu)
 int bfs_prepare_queues(vglb_ctx *ctx, vglb_graph *g);
 
-// one kernel: counters [0, C_COUNT) -> [C_COUNT, 2 C_COUNT), the copy a partitioned level allreduces (sum over ranks), and
-// C_MF -> slot 2 C_COUNT (partitioned SSSP allreduces its pending minimum there with MAX) (frontier.cu)
-int vglb_stage_counters(vglb_ctx *ctx);
+// read-back of a partitioned level or round (frontier.cu): stages the counters [0, C_COUNT) at C_STAGED and C_MF at
+// CTR_PENDING_MIN (one kernel), sums the staged copy over the ranks, copies `words` counters to ctx->h_counters and waits
+// for them. [0, C_COUNT) stay this rank's own counts.
+int vglb_part_round_counters(vglb_ctx *ctx, vglb_comm *comm, int words);

@@ -224,7 +224,7 @@ static int bits_for(int32_t V)
 
 int vglb_graph_compute_tiers(vglb_ctx *ctx, vglb_graph *g)
 {
-    int32_t *d_out = (int32_t *)ctx->d_counters; // reuse the counter block
+    int32_t *d_out = (int32_t *)(ctx->d_counters + CTR_SCRATCH_I32);
     CUDA_TRY(cudaMemsetAsync(d_out, 0, (VGLB_NUM_TIERS + 2) * sizeof(int32_t), ctx->stream));
     if (g->V > 0)
     {
@@ -546,7 +546,7 @@ extern "C" int vglb_graph_from_csr(vglb_ctx *ctx, int32_t V, int64_t E, const in
         clock_gettime(CLOCK_MONOTONIC, &ts);
         fprintf(stderr, "from_csr: %-44s %8.2f ms\n", what, 1e3 * (double)(ts.tv_sec - ts0.tv_sec) + 1e-6 * (double)(ts.tv_nsec - ts0.tv_nsec));
     };
-    int *d_bad = (int *)(ctx->d_counters + 56);
+    int *d_bad = (int *)(ctx->d_counters + CTR_BAD);
     BUILD_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int), ctx->stream));
     const size_t eb = (size_t)(E ? E : 1) * 4;
     BUILD_CUDA(vglb_dev_alloc(&g->d_out_ptr, ((size_t)V + 2) * 8));
@@ -768,7 +768,7 @@ extern "C" int vglb_graph_borrow_csr(vglb_ctx *ctx, int32_t V, int64_t E, const 
 
 int vglb_csr_validate_device(vglb_ctx *ctx, const int64_t *d_ptr, int32_t rows, int64_t E, const int32_t *d_adj, int64_t id_limit)
 {
-    int *d_bad = (int *)(ctx->d_counters + 56);
+    int *d_bad = (int *)(ctx->d_counters + CTR_BAD);
     CUDA_TRY(cudaMemsetAsync(d_bad, 0, sizeof(int), ctx->stream));
     csr_ptr_check_kernel<<<(unsigned)ceil_div64((int64_t)rows + 1, 256), 256, 0, ctx->stream>>>(d_ptr, rows, E, d_bad);
     KERNEL_TRY();
@@ -882,7 +882,7 @@ __global__ void threshold_vertex_kernel(const int64_t *__restrict__ ptr, int32_t
 extern "C" int vglb_graph_threshold_vertex(vglb_ctx *ctx, vglb_graph *g, int32_t degree_threshold, int32_t *out_vertex)
 {
     VGLB_REQUIRE(ctx != NULL && g != NULL && out_vertex != NULL, "vglb_graph_threshold_vertex: NULL argument");
-    int32_t *d_out = (int32_t *)ctx->d_counters;
+    int32_t *d_out = (int32_t *)(ctx->d_counters + CTR_SCRATCH_I32);
     CUDA_TRY(cudaMemsetAsync(d_out, 0, 4, ctx->stream));
     threshold_vertex_kernel<<<(unsigned)ceil_div64(g->V, 256), 256, 0, ctx->stream>>>(g->d_out_ptr, g->V, degree_threshold, d_out);
     KERNEL_TRY();

@@ -182,6 +182,8 @@ int vglb_comm_allgather_async(vglb_comm *comm, void *d_buf, size_t bytes_per_ran
     return VGLB_OK;
 }
 
+static inline size_t dtype_bytes(int dtype) { return dtype == VGLB_DT_I64 || dtype == VGLB_DT_F64 ? 8 : 4; }
+
 int vglb_comm_allreduce_async(vglb_comm *comm, void *d_buf, size_t count, int dtype, int op)
 {
     NcclApi *N = nccl_api();
@@ -190,6 +192,23 @@ int vglb_comm_allreduce_async(vglb_comm *comm, void *d_buf, size_t count, int dt
     const ncclDataType_t t = dtype == VGLB_DT_I64 ? ncclInt64 : dtype == VGLB_DT_F64 ? ncclFloat64 : dtype == VGLB_DT_U32 ? ncclUint32 : ncclInt32;
     const ncclRedOp_t o = op == VGLB_OP_MIN ? ncclMin : op == VGLB_OP_MAX ? ncclMax : ncclSum;
     NCCL_TRY(N->AllReduce(d_buf, d_buf, count, t, o, (ncclComm_t)comm->nccl, comm->ctx->stream));
+    return VGLB_OK;
+}
+
+// the host side of the slot is pinned (ctx->h_counters), so both copies are plain asynchronous DMA on the context stream
+int vglb_comm_allreduce_host(vglb_comm *comm, void *h_inout, int count, int dtype, int op)
+{
+    const size_t bytes = (size_t)count * dtype_bytes(dtype);
+    VGLB_REQUIRE(count > 0 && bytes <= 16, "vglb_comm_allreduce_host: at most 16 bytes");
+    vglb_ctx *ctx = comm->ctx;
+    void *h = ctx->h_counters + CTR_HOST_ALLREDUCE, *d = ctx->d_counters + CTR_HOST_ALLREDUCE;
+    memcpy(h, h_inout, bytes);
+    CUDA_TRY(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    int rc = vglb_comm_allreduce_async(comm, d, (size_t)count, dtype, op);
+    if (rc != VGLB_OK) return rc;
+    CUDA_TRY(cudaMemcpyAsync(h, d, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    memcpy(h_inout, h, bytes);
     return VGLB_OK;
 }
 
@@ -315,12 +334,8 @@ int vglb_part_map_lists(vglb_ctx *ctx, vglb_graph *g)
         g->ipc_exported = 1;
         if (vglb_comm_ipc_map(g->comm, g->d_part_lists, (void **)g->d_vec_peer) != VGLB_OK) ok = 0;
     }
-    int *d_ok = (int *)(ctx->d_counters + 62);
-    CUDA_TRY(cudaMemcpyAsync(d_ok, &ok, 4, cudaMemcpyHostToDevice, ctx->stream));
-    int rc = vglb_comm_allreduce_async(g->comm, d_ok, 1, VGLB_DT_I32, VGLB_OP_MIN);
+    int rc = vglb_comm_allreduce_host(g->comm, &ok, 1, VGLB_DT_I32, VGLB_OP_MIN);
     if (rc != VGLB_OK) return rc;
-    CUDA_TRY(cudaMemcpyAsync(&ok, d_ok, 4, cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     g->vec_peers_mapped = ok ? 1 : -1;
     return VGLB_OK;
 }
@@ -340,14 +355,7 @@ extern "C" int vglb_comm_allreduce_sum_i64(vglb_comm *comm, int64_t *d_buf, int 
 extern "C" int vglb_comm_allreduce_max_f64(vglb_comm *comm, double *h_value)
 {
     VGLB_REQUIRE(comm != NULL && h_value != NULL, "vglb_comm_allreduce_max_f64: NULL argument");
-    vglb_ctx *ctx = comm->ctx;
-    double *d = (double *)(ctx->d_counters + 48);
-    CUDA_TRY(cudaMemcpyAsync(d, h_value, 8, cudaMemcpyHostToDevice, ctx->stream));
-    int rc = vglb_comm_allreduce_async(comm, d, 1, VGLB_DT_F64, VGLB_OP_MAX);
-    if (rc != VGLB_OK) return rc;
-    CUDA_TRY(cudaMemcpyAsync(h_value, d, 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    return VGLB_OK;
+    return vglb_comm_allreduce_host(comm, h_value, 1, VGLB_DT_F64, VGLB_OP_MAX);
 }
 
 extern "C" int vglb_comm_barrier(vglb_comm *comm)
@@ -848,7 +856,7 @@ extern "C" int vglb_graph_from_csr_partitioned(vglb_ctx *ctx, vglb_comm *comm, i
     // caller-supplied arrays are checked on the device before anything indexes with them (row pointers non-decreasing
     // from 0 to E, column ids in [0, cols), the map injective); the verdict travels with the edge count so that a
     // rank with a bad part takes every rank out of the call together instead of leaving the others in a collective
-    int *d_bad = (int *)(ctx->d_counters + 56);
+    int *d_bad = (int *)(ctx->d_counters + CTR_BAD);
     PBUILD_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int), st));
     part_invert_map_kernel<<<(unsigned)ceil_div64(V, 256), 256, 0, st>>>(g->d_fwd, V, g->cols, g->d_bwd, d_bad);
     PBUILD_CUDA(cudaGetLastError());
@@ -869,14 +877,9 @@ extern "C" int vglb_graph_from_csr_partitioned(vglb_ctx *ctx, vglb_comm *comm, i
     int64_t bad_ranks = bad ? 1 : 0;
     if (comm->nccl && P > 1)
     {
-        int64_t *d = ctx->d_counters + 50;
-        const int64_t h2[2] = {E, bad_ranks};
-        int64_t r2[2] = {0, 0};
-        PBUILD_CUDA(cudaMemcpyAsync(d, h2, 16, cudaMemcpyHostToDevice, st));
-        int rc = vglb_comm_allreduce_async(comm, d, 2, VGLB_DT_I64, VGLB_OP_SUM);
+        int64_t r2[2] = {E, bad_ranks};
+        int rc = vglb_comm_allreduce_host(comm, r2, 2, VGLB_DT_I64, VGLB_OP_SUM);
         if (rc != VGLB_OK) { cleanup(); return rc; }
-        PBUILD_CUDA(cudaMemcpyAsync(r2, d, 16, cudaMemcpyDeviceToHost, st));
-        PBUILD_CUDA(cudaStreamSynchronize(st));
         g->E_global = r2[0];
         bad_ranks = r2[1];
     }

@@ -188,12 +188,8 @@ static int sssp_partitioned_dense(vglb_ctx *ctx, vglb_graph *g, const float *d_w
             KERNEL_TRY();
         }
         ctx->launches++;
-        rc = vglb_stage_counters(ctx);
+        rc = vglb_part_round_counters(ctx, comm, 2 * C_COUNT);
         if (rc != VGLB_OK) return rc;
-        rc = vglb_comm_allreduce_async(comm, d_cnt + C_COUNT, C_COUNT, VGLB_DT_I64, VGLB_OP_SUM);
-        if (rc != VGLB_OK) return rc;
-        CUDA_TRY(cudaMemcpyAsync(h_cnt, d_cnt, 2 * C_COUNT * 8, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
         CUDA_TRY(cudaMemsetAsync(d_cnt, 0, 2 * C_COUNT * 8, st));
         rounds++;
         tot_rows += (int64_t)n[0] + n[1] + n[2];
@@ -201,7 +197,7 @@ static int sssp_partitioned_dense(vglb_ctx *ctx, vglb_graph *g, const float *d_w
         n[0] = (int32_t)h_cnt[C_NEXT_BIG];
         n[1] = (int32_t)h_cnt[C_NEXT_MID];
         n[2] = (int32_t)h_cnt[C_NEXT_SMALL];
-        const unsigned long long *gl = h_cnt + C_COUNT;
+        const unsigned long long *gl = h_cnt + C_STAGED;
         n_cur = (long long)(gl[C_NEXT_BIG] + gl[C_NEXT_MID] + gl[C_NEXT_SMALL]);
         tot_next += (int64_t)n[0] + n[1] + n[2];
         TierQueues t = cq; cq = nq; nq = t;
@@ -396,8 +392,6 @@ sssp_relax_flat_kernel(const int64_t *__restrict__ ptr, const int32_t *__restric
 #define SSSP_DRAIN_MAX_EDGES 65536 // edges one CTA relaxes per round
 #define SSSP_DRAIN_LIST 2048
 enum { DRAIN_NOT_STARTED = 0, DRAIN_EMPTY = 1, DRAIN_PENDING = 2 };
-// result slots in the counter block (after the 2 * C_COUNT + 1 words the host loop reads)
-enum { DR_REASON = 2 * C_COUNT + 2, DR_ROUNDS, DR_ROWS, DR_END };
 
 __global__ void __launch_bounds__(SSSP_DRAIN_THREADS)
 sssp_drain_kernel(const int64_t *__restrict__ ptr, const int32_t *__restrict__ adj, const float *__restrict__ wgt, TierQueues cq,
@@ -810,7 +804,7 @@ static int sssp_run(vglb_ctx *ctx, vglb_graph *g, const float *d_weights, int32_
         if (!g->d_part_bm[0]) CUDA_TRY(vglb_dev_alloc(&g->d_part_bm[0], (words_full + 32) * 4));
         dist = g->d_part_vec;
         changed_bm = g->d_part_bm[0];
-        d_peer_table = (const unsigned long long **)(ctx->d_counters + 24); // 8 device pointers
+        d_peer_table = (const unsigned long long **)(ctx->d_counters + CTR_PEER_TABLE);
         CUDA_TRY(cudaMemcpyAsync(d_peer_table, g->d_vec_peer, sizeof(g->d_vec_peer), cudaMemcpyHostToDevice, ctx->stream));
     }
     const int64_t launches0 = ctx->launches;
@@ -828,7 +822,7 @@ static int sssp_run(vglb_ctx *ctx, vglb_graph *g, const float *d_weights, int32_
     float delta = 0.f; // 0 = plain schedule
     if (scale > 0.0 && g->E_global > 0)
     {
-        unsigned int *d_max = (unsigned int *)(d_cnt + 60);
+        unsigned int *d_max = (unsigned int *)(d_cnt + CTR_SSSP_WMAX);
         CUDA_TRY(cudaMemsetAsync(d_max, 0, 4, st));
         if (g->E > 0)
         {
@@ -862,7 +856,7 @@ static int sssp_run(vglb_ctx *ctx, vglb_graph *g, const float *d_weights, int32_
     sssp_part_seed_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(dist, part ? g->cols : (int64_t)rows, source, near_bm,
                                                             (src_row >= 0 && src_row < rows) ? src_row : -1);
     KERNEL_TRY();
-    CUDA_TRY(cudaMemsetAsync(d_cnt, 0, (2 * C_COUNT + 1) * 8, st));
+    CUDA_TRY(cudaMemsetAsync(d_cnt, 0, CTR_SSSP_ROUND * 8, st));
     ctx->launches++;
     int64_t tot_edges = 0, tot_rows = 0, tot_next = 0, rounds = 0, selects = 0, far_selects = 0, tot_pulled = 0;
     const unsigned select_grid = (unsigned)ceil_div64((int64_t)words, 256);
@@ -892,26 +886,11 @@ static int sssp_run(vglb_ctx *ctx, vglb_graph *g, const float *d_weights, int32_
         ctx->launches++;
         selects++;
         far_selects += from_far;
-        if (part)
-        {
-            rc = vglb_stage_counters(ctx);
-            if (rc != VGLB_OK) return rc;
-            rc = vglb_comm_allreduce_async(comm, d_cnt + C_COUNT, C_COUNT, VGLB_DT_I64, VGLB_OP_SUM);
-            if (rc != VGLB_OK) return rc;
-        }
-        if (part)
-        {
-            CUDA_TRY(cudaMemcpyAsync(h_cnt, d_cnt, (2 * C_COUNT + 1) * 8, cudaMemcpyDeviceToHost, st));
-            CUDA_TRY(cudaStreamSynchronize(st));
-        }
-        else
-        {
-            rc = vglb_counters_fetch(ctx, d_cnt, 2 * C_COUNT + 1);
-            if (rc != VGLB_OK) return rc;
-        }
-        CUDA_TRY(cudaMemsetAsync(d_cnt, 0, (2 * C_COUNT + 1) * 8, st));
+        rc = part ? vglb_part_round_counters(ctx, comm, CTR_SSSP_ROUND) : vglb_counters_fetch(ctx, d_cnt, CTR_SSSP_ROUND);
+        if (rc != VGLB_OK) return rc;
+        CUDA_TRY(cudaMemsetAsync(d_cnt, 0, CTR_SSSP_ROUND * 8, st));
         const int32_t n[3] = {(int32_t)h_cnt[C_NEXT_BIG], (int32_t)h_cnt[C_NEXT_MID], (int32_t)h_cnt[C_NEXT_SMALL]};
-        const unsigned long long *gl = part ? h_cnt + C_COUNT : h_cnt; // whole-job sums drive the schedule
+        const unsigned long long *gl = part ? h_cnt + C_STAGED : h_cnt; // whole-job sums drive the schedule
         const long long n_local = (long long)n[0] + n[1] + n[2];
         const long long n_cur = (long long)(gl[C_NEXT_BIG] + gl[C_NEXT_MID] + gl[C_NEXT_SMALL]), pending = (long long)gl[C_FOUND];
         tot_edges += (int64_t)h_cnt[C_EDGES]; // relaxed by the previous round (this rank)
@@ -948,15 +927,10 @@ static int sssp_run(vglb_ctx *ctx, vglb_graph *g, const float *d_weights, int32_
             if (part)
             {
                 // the smallest pending distance of the whole job (every rank takes this branch: same allreduced counters)
-                unsigned long long *d_min = d_cnt + 2 * C_COUNT;
-                CUDA_TRY(cudaMemcpyAsync(d_min, h_cnt + 2 * C_COUNT, 8, cudaMemcpyHostToDevice, st));
-                rc = vglb_comm_allreduce_async(comm, d_min, 1, VGLB_DT_I64, VGLB_OP_MAX);
+                rc = vglb_comm_allreduce_host(comm, h_cnt + CTR_PENDING_MIN, 1, VGLB_DT_I64, VGLB_OP_MAX);
                 if (rc != VGLB_OK) return rc;
-                CUDA_TRY(cudaMemcpyAsync(h_cnt + 2 * C_COUNT, d_min, 8, cudaMemcpyDeviceToHost, st));
-                CUDA_TRY(cudaStreamSynchronize(st));
-                CUDA_TRY(cudaMemsetAsync(d_min, 0, 8, st));
             }
-            const uint32_t min_bits = 0xffffffffu - (uint32_t)(part ? h_cnt[2 * C_COUNT] : h_cnt[C_MF]);
+            const uint32_t min_bits = 0xffffffffu - (uint32_t)(part ? h_cnt[CTR_PENDING_MIN] : h_cnt[C_MF]);
             float min_pending;
             memcpy(&min_pending, &min_bits, 4);
             // nothing below the moved threshold: jump. The far select takes d < threshold, so the new threshold must lie
@@ -1016,7 +990,7 @@ static int sssp_run(vglb_ctx *ctx, vglb_graph *g, const float *d_weights, int32_
             KERNEL_TRY();
             // barrier: every rank's lists are complete before anybody reads them; the NEXT round's lists are not touched
             // before every rank has passed the next counter allreduce, i.e. finished reading these
-            rc = vglb_comm_allreduce_async(comm, d_cnt + 2 * C_COUNT + 2, 1, VGLB_DT_I64, VGLB_OP_SUM);
+            rc = vglb_comm_allreduce_async(comm, d_cnt + CTR_LIST_BARRIER, 1, VGLB_DT_I64, VGLB_OP_SUM);
             if (rc != VGLB_OK) return rc;
             sssp_apply_updates_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(d_peer_table, P, rank, vp, col0, dist, near_bm, far_bm, tbits, d_cnt);
             KERNEL_TRY();

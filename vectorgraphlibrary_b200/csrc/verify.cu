@@ -113,7 +113,7 @@ int fetch_count(vglb_ctx *ctx, unsigned long long *d_out, int64_t *out)
 extern "C" int vglb_verify_i32(vglb_ctx *ctx, const int32_t *d_a, const int32_t *d_b, int64_t n, int64_t *error_count)
 {
     VGLB_REQUIRE(ctx != NULL && d_a != NULL && d_b != NULL && error_count != NULL && n >= 0, "vglb_verify_i32: bad argument");
-    unsigned long long *d_out = (unsigned long long *)(ctx->d_counters + 57);
+    unsigned long long *d_out = (unsigned long long *)(ctx->d_counters + CTR_VERIFY_COUNT);
     CUDA_TRY(cudaMemsetAsync(d_out, 0, 8, ctx->stream));
     if (n > 0)
     {
@@ -127,7 +127,7 @@ extern "C" int vglb_verify_i32(vglb_ctx *ctx, const int32_t *d_a, const int32_t 
 extern "C" int vglb_verify_f32(vglb_ctx *ctx, const float *d_a, const float *d_b, int64_t n, int64_t *error_count)
 {
     VGLB_REQUIRE(ctx != NULL && d_a != NULL && d_b != NULL && error_count != NULL && n >= 0, "vglb_verify_f32: bad argument");
-    unsigned long long *d_out = (unsigned long long *)(ctx->d_counters + 57);
+    unsigned long long *d_out = (unsigned long long *)(ctx->d_counters + CTR_VERIFY_COUNT);
     CUDA_TRY(cudaMemsetAsync(d_out, 0, 8, ctx->stream));
     if (n > 0)
     {
@@ -142,7 +142,7 @@ extern "C" int vglb_verify_ranking_f32(vglb_ctx *ctx, const float *d_a, const fl
                                        double *relative_l1, int64_t *error_count)
 {
     VGLB_REQUIRE(ctx != NULL && d_a != NULL && d_ref != NULL && n >= 0, "vglb_verify_ranking_f32: bad argument");
-    double *d_out = (double *)(ctx->d_counters + 58);
+    double *d_out = (double *)(ctx->d_counters + CTR_VERIFY_SUMS);
     CUDA_TRY(cudaMemsetAsync(d_out, 0, 16, ctx->stream));
     if (n > 0)
     {
@@ -167,8 +167,8 @@ extern "C" int vglb_verify_components_i32(vglb_ctx *ctx, const int32_t *d_a, con
     int32_t *last = NULL;
     CUDA_TRY(vglb_dev_alloc(&last, 2 * ((size_t)n + 2) * 4));
     int32_t *last_a = last, *last_b = last + n + 2;
-    unsigned long long *d_out = (unsigned long long *)(ctx->d_counters + 57);
-    int *d_bad = (int *)(ctx->d_counters + 56);
+    unsigned long long *d_out = (unsigned long long *)(ctx->d_counters + CTR_VERIFY_COUNT);
+    int *d_bad = (int *)(ctx->d_counters + CTR_BAD);
     CUDA_TRY(cudaMemsetAsync(last, 0xFF, 2 * ((size_t)n + 2) * 4, ctx->stream));
     CUDA_TRY(cudaMemsetAsync(d_out, 0, 8, ctx->stream));
     CUDA_TRY(cudaMemsetAsync(d_bad, 0, 4, ctx->stream));
