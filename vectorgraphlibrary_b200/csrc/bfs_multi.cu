@@ -425,29 +425,18 @@ extern "C" int vglb_bfs_multi(vglb_ctx *ctx, vglb_graph *g, int32_t num_sources,
         VGLB_REQUIRE(h_sources_sorted[i] >= 0 && h_sources_sorted[i] < g->V, "vglb_bfs_multi: source out of range");
     const BfsDirection dir = bfs_direction(opts, g->E, g->V);
     CUDA_TRY(cudaSetDevice(ctx->device));
-    if (dir.dopt && !g->d_in_ptr)
-    {
-        int rc_in = vglb_graph_derive_incoming(ctx, g); // as vglb_bfs: the bottom-up levels need the incoming CSR
-        if (rc_in != VGLB_OK) return rc_in;
-    }
-    int rc = bfs_prepare_queues(ctx, g);
-    if (rc != VGLB_OK) return rc;
+    if (dir.dopt && !g->d_in_ptr) VGLB_TRY(vglb_graph_derive_incoming(ctx, g)); // as vglb_bfs: the bottom-up levels need the incoming CSR
+    VGLB_TRY(bfs_prepare_queues(ctx, g));
     // per-call word arrays from the context's allocation cache: seen | front_a | front_b, V words each
     const bool wide = num_sources > 32;
     const size_t wbytes = wide ? 8 : 4;
-    void *words = NULL;
-    CUDA_TRY(vglb_dev_alloc(&words, (size_t)3 * ((size_t)g->V > 0 ? g->V : 1) * wbytes));
+    dev_ptr<void> words;
+    CUDA_TRY(vglb_dev_alloc(words, (size_t)3 * ((size_t)g->V > 0 ? g->V : 1) * wbytes));
     if (wide)
     {
-        unsigned long long *p = (unsigned long long *)words;
-        rc = bfs_multi_run<unsigned long long>(ctx, g, h_sources_sorted, num_sources, d_levels, dir, p, p + g->V, p + 2 * (size_t)g->V, stats);
+        unsigned long long *p = (unsigned long long *)words.get();
+        return bfs_multi_run<unsigned long long>(ctx, g, h_sources_sorted, num_sources, d_levels, dir, p, p + g->V, p + 2 * (size_t)g->V, stats);
     }
-    else
-    {
-        uint32_t *p = (uint32_t *)words;
-        rc = bfs_multi_run<uint32_t>(ctx, g, h_sources_sorted, num_sources, d_levels, dir, p, p + g->V, p + 2 * (size_t)g->V, stats);
-    }
-    if (rc != VGLB_OK) cudaStreamSynchronize(ctx->stream); // nothing may still use the block when it goes back to the cache
-    vglb_dev_free(words);
-    return rc;
+    uint32_t *p = (uint32_t *)words.get();
+    return bfs_multi_run<uint32_t>(ctx, g, h_sources_sorted, num_sources, d_levels, dir, p, p + g->V, p + 2 * (size_t)g->V, stats);
 }

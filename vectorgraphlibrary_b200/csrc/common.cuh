@@ -4,7 +4,10 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <stdlib.h>
 #include <string.h>
+
+#include <memory>
 
 #include "vgl_b200.h"
 #include "vglb_synth.h"
@@ -24,20 +27,69 @@ static inline cudaError_t vglb_dev_alloc(T **ptr, size_t bytes)
     return vglb_dev_alloc_bytes((void **)ptr, bytes);
 }
 
-// SAFE_CALL twin (cuda_error_handling.h:7-13): record the message and return an error code instead of throwing.
+// Owning handle of a block from the cache: the block goes back on every exit of the scope that holds it. release() hands it
+// over to a graph or PrBins field; reset() frees it early.
+struct vglb_dev_deleter
+{
+    void operator()(void *p) const { vglb_dev_free(p); }
+};
+template <class T>
+using dev_ptr = std::unique_ptr<T, vglb_dev_deleter>;
+// (a block the handle already holds goes back first, as a vglb_dev_free before the allocation would)
+template <class T>
+static inline cudaError_t vglb_dev_alloc(dev_ptr<T> &p, size_t bytes)
+{
+    p.reset();
+    T *raw = NULL;
+    const cudaError_t e = vglb_dev_alloc(&raw, bytes);
+    if (e == cudaSuccess) p.reset(raw);
+    return e;
+}
+
+// SAFE_CALL twin (cuda_error_handling.h:7-13): record the message and return an error code instead of throwing. The
+// runtime's last error is cleared, so a failed allocation is reported once, as VGLB_ENOMEM.
 #define CUDA_TRY(call)                                                                               \
     do                                                                                               \
     {                                                                                                \
         cudaError_t err__ = (call);                                                                  \
         if (err__ != cudaSuccess)                                                                    \
         {                                                                                            \
+            cudaGetLastError();                                                                      \
             vglb_set_error("CUDA error %s at %s:%d (%s)", cudaGetErrorString(err__), __FILE__,       \
                            __LINE__, #call);                                                         \
-            return VGLB_ECUDA;                                                                       \
+            return err__ == cudaErrorMemoryAllocation ? VGLB_ENOMEM : VGLB_ECUDA;                    \
         }                                                                                            \
     } while (0)
 
 #define KERNEL_TRY() CUDA_TRY(cudaGetLastError())
+
+// a library call that returns a VGLB_* code
+#define VGLB_TRY(call)                \
+    do                                \
+    {                                 \
+        const int rc__ = (call);      \
+        if (rc__ != VGLB_OK)          \
+            return rc__;              \
+    } while (0)
+
+// A two-phase CUB call run(d_temp, bytes): asks for the size of its temporary, takes that from the cache into `tmp` and runs
+// it. Nothing is synchronised; the caller decides when `tmp` goes back (the cache orders its re-use after the call).
+template <class Run>
+static inline cudaError_t vglb_cub(dev_ptr<void> &tmp, Run &&run)
+{
+    size_t bytes = 0;
+    cudaError_t e = run(nullptr, bytes);
+    if (e == cudaSuccess) e = vglb_dev_alloc(tmp, bytes);
+    return e == cudaSuccess ? run(tmp.get(), bytes) : e;
+}
+
+// bits of a radix-sort key that holds the values [0, n): at least 1, at most 32
+static inline int vglb_key_bits(int64_t n)
+{
+    int b = 1;
+    while (b < 32 && ((int64_t)1 << b) < n) b++;
+    return b;
+}
 
 #define VGLB_REQUIRE(cond, msg)                                       \
     do                                                                \
@@ -238,6 +290,33 @@ void vglb_graph_set_unpartitioned(vglb_graph *g);
 int vglb_graph_derive_incoming(vglb_ctx *ctx, vglb_graph *g);
 int vglb_pr_build_tasks_host(vglb_ctx *ctx, vglb_graph *g, const int64_t *h_ptr, int32_t heavy_rows, int32_t long_rows);
 void vglb_graph_free_fields(vglb_graph *g);
+// owner of a graph that is still being built: its fields and the struct go back unless it is released into *out_graph
+struct vglb_graph_deleter
+{
+    void operator()(vglb_graph *g) const
+    {
+        vglb_graph_free_fields(g);
+        free(g);
+    }
+};
+using graph_ptr = std::unique_ptr<vglb_graph, vglb_graph_deleter>;
+static inline graph_ptr vglb_graph_new() { return graph_ptr((vglb_graph *)calloc(1, sizeof(vglb_graph))); }
+
+// checks of caller-supplied construction input (graph_build.cu); a failed check sets the CTR_BAD word, which the caller
+// clears before and reads back after
+// row pointers d_ptr[0..rows] from 0 to E, non-decreasing, and the E ids of d_adj in [0, id_limit)
+int vglb_csr_validate_device(vglb_ctx *ctx, const int64_t *d_ptr, int32_t rows, int64_t E, const int32_t *d_adj, int64_t id_limit);
+// bwd[fwd[i]] = i for i in [0, n); bwd must be filled with -1, and every fwd[i] must be a distinct value in [0, limit)
+int vglb_invert_map_checked(vglb_ctx *ctx, const int32_t *d_fwd, int32_t n, int64_t limit, int32_t *d_bwd);
+// the ids [0, V) stably sorted by degree descending (ties by ascending id, the reference's std::stable_sort): `sorted`
+// points into ids[]. The buffers go back when the struct does.
+struct DegreeOrder
+{
+    dev_ptr<uint32_t> keys[2], ids[2];
+    dev_ptr<void> tmp;
+    const uint32_t *sorted = nullptr;
+};
+int vglb_degree_order(vglb_ctx *ctx, const int32_t *d_deg, int32_t V, DegreeOrder &order);
 void vglb_pr_bins_free(vglb_graph *g);   // pagerank_bins.cu
 int vglb_pr_bins_build_rows(vglb_ctx *ctx, vglb_graph *g, int32_t rows); // rows = ids with >= 32 edges (tier_border[1])
 int vglb_pr_bins_wanted(const vglb_graph *g); // 1: the PageRank sweep of this graph uses the column-binned heavy rows

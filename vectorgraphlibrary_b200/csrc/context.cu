@@ -146,6 +146,19 @@ void vglb_dev_cache_release(void)
     cache_release_all(C);
 }
 
+// Test hook, not part of the public header: the blocks of the current device's cache that are handed out and not yet freed.
+// A test compares it before and after a call to see that the call gave back every temporary.
+extern "C" int vglb_dev_live_blocks(int64_t *blocks, int64_t *bytes)
+{
+    DeviceCache &C = cache_of_current_device();
+    std::lock_guard<std::mutex> lock(C.mu);
+    size_t total = 0;
+    for (const auto &kv : C.live) total += kv.second;
+    if (blocks) *blocks = (int64_t)C.live.size();
+    if (bytes) *bytes = (int64_t)total;
+    return VGLB_OK;
+}
+
 
 extern "C" int vglb_device_count(void)
 {

@@ -35,12 +35,12 @@ __global__ void degree_histogram_kernel(const int32_t *__restrict__ ids, int64_t
     }
 }
 
-__global__ void range_check_kernel(const int32_t *__restrict__ ids, int64_t n, int32_t V, int *__restrict__ bad)
+__global__ void id_range_check_kernel(const int32_t *__restrict__ ids, int64_t n, int64_t limit, int *__restrict__ bad)
 {
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (; i < n; i += stride)
-        if (ids[i] < 0 || ids[i] >= V) *bad = 1;
+        if (ids[i] < 0 || ids[i] >= limit) *bad = 1;
 }
 
 __global__ void degree_sort_keys_kernel(const int32_t *__restrict__ deg, int32_t V, uint32_t *__restrict__ keys,
@@ -151,13 +151,15 @@ __global__ void csr_ptr_check_kernel(const int64_t *__restrict__ ptr, int32_t ro
     if (v < rows && ptr[v] > ptr[v + 1]) *bad = 1;
 }
 
-// ORIGINAL -> sorted map supplied by the caller: bwd was filled with -1; every slot must be hit exactly once
-__global__ void invert_perm_checked_kernel(const int32_t *__restrict__ fwd, int32_t *__restrict__ bwd, int32_t n, int *__restrict__ bad)
+// map supplied by the caller (ORIGINAL -> sorted, or ORIGINAL -> column of a partitioned graph): bwd was filled with -1; every
+// vertex must go to a distinct slot in [0, limit)
+__global__ void invert_map_checked_kernel(const int32_t *__restrict__ fwd, int32_t n, int64_t limit, int32_t *__restrict__ bwd,
+                                          int *__restrict__ bad)
 {
     int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const int32_t f = fwd[i];
-    if ((uint32_t)f >= (uint32_t)n) { *bad = 1; return; }
+    if (f < 0 || f >= limit) { *bad = 1; return; }
     if (atomicExch(&bwd[f], i) != -1) *bad = 1;
 }
 
@@ -174,12 +176,6 @@ __global__ void iota_kernel(int32_t *a, int32_t n)
 {
     int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) a[i] = i;
-}
-
-__global__ void invert_perm_kernel(const int32_t *__restrict__ fwd, int32_t *__restrict__ bwd, int32_t n)
-{
-    int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) bwd[fwd[i]] = i;
 }
 
 // tier borders: border[t] = first id whose degree < tier_degree[t]; also checks the rows are degree-sorted.
@@ -213,13 +209,6 @@ void vglb_graph_set_unpartitioned(vglb_graph *g)
     g->cols = g->V;
     g->E_global = g->E;
     g->col_of_row0 = 0;
-}
-
-static int bits_for(int32_t V)
-{
-    int b = 1;
-    while (b < 32 && ((int64_t)1 << b) < (int64_t)V) b++;
-    return b;
 }
 
 int vglb_graph_compute_tiers(vglb_ctx *ctx, vglb_graph *g)
@@ -310,57 +299,29 @@ extern "C" int vglb_graph_free(vglb_ctx *ctx, vglb_graph *g)
     return VGLB_OK;
 }
 
-#define BUILD_TRY(call)                   \
-    do                                    \
-    {                                     \
-        int rc__ = (call);                \
-        if (rc__ != VGLB_OK)              \
-        {                                 \
-            cleanup();                    \
-            return rc__;                  \
-        }                                 \
-    } while (0)
-
-#define BUILD_CUDA(call)                                                                                   \
-    do                                                                                                     \
-    {                                                                                                      \
-        cudaError_t err__ = (call);                                                                        \
-        if (err__ != cudaSuccess)                                                                          \
-        {                                                                                                  \
-            vglb_set_error("CUDA error %s at %s:%d (%s)", cudaGetErrorString(err__), __FILE__, __LINE__,   \
-                           #call);                                                                         \
-            cudaGetLastError();                                                                            \
-            cleanup();                                                                                     \
-            return err__ == cudaErrorMemoryAllocation ? VGLB_ENOMEM : VGLB_ECUDA;                          \
-        }                                                                                                  \
-    } while (0)
-
 // outgoing direction: stable sort of the edges by fwd[src]; adjacency = fwd[dst] in that order. When d_row_of_pos is
 // non-NULL it receives the (ascending) row id of every CSR position, which the incoming build reuses.
 static int build_outgoing(vglb_ctx *ctx, int32_t V, int64_t E, const int32_t *d_src, const int32_t *d_dst,
                           const int32_t *d_fwd, int32_t *d_adj, int64_t *d_edge_order, uint32_t *d_row_of_pos)
 {
-    uint32_t *k0 = NULL, *k1 = NULL, *v0 = NULL, *v1 = NULL;
-    void *tmp = NULL;
-    auto cleanup = [&]() { vglb_dev_free(k0); vglb_dev_free(k1); vglb_dev_free(v0); vglb_dev_free(v1); vglb_dev_free(tmp); };
     if (E == 0) return VGLB_OK;
     const size_t eb = (size_t)E * sizeof(uint32_t);
-    BUILD_CUDA(vglb_dev_alloc(&k0, eb)); BUILD_CUDA(vglb_dev_alloc(&k1, eb));
-    BUILD_CUDA(vglb_dev_alloc(&v0, eb)); BUILD_CUDA(vglb_dev_alloc(&v1, eb));
+    dev_ptr<uint32_t> k0, k1, v0, v1;
+    dev_ptr<void> tmp;
+    CUDA_TRY(vglb_dev_alloc(k0, eb)); CUDA_TRY(vglb_dev_alloc(k1, eb));
+    CUDA_TRY(vglb_dev_alloc(v0, eb)); CUDA_TRY(vglb_dev_alloc(v1, eb));
     const int grid = ctx->sm_count * 16;
-    edge_keys_kernel<<<grid, 256, 0, ctx->stream>>>(d_src, d_fwd, E, k0, v0);
-    BUILD_CUDA(cudaGetLastError());
-    cub::DoubleBuffer<uint32_t> keys(k0, k1), vals(v0, v1);
-    size_t tmp_bytes = 0;
-    BUILD_CUDA(cub::DeviceRadixSort::SortPairs(NULL, tmp_bytes, keys, vals, E, 0, bits_for(V), ctx->stream));
-    BUILD_CUDA(vglb_dev_alloc(&tmp, tmp_bytes ? tmp_bytes : 16));
-    BUILD_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, keys, vals, E, 0, bits_for(V), ctx->stream));
+    edge_keys_kernel<<<grid, 256, 0, ctx->stream>>>(d_src, d_fwd, E, k0.get(), v0.get());
+    KERNEL_TRY();
+    cub::DoubleBuffer<uint32_t> keys(k0.get(), k1.get()), vals(v0.get(), v1.get());
+    CUDA_TRY(vglb_cub(tmp, [&](void *t, size_t &bytes) {
+        return cub::DeviceRadixSort::SortPairs(t, bytes, keys, vals, E, 0, vglb_key_bits(V), ctx->stream);
+    }));
     gather_adj_kernel<<<grid, 256, 0, ctx->stream>>>(vals.Current(), d_dst, d_fwd, E, d_adj, d_edge_order);
-    BUILD_CUDA(cudaGetLastError());
+    KERNEL_TRY();
     if (d_row_of_pos)
-        BUILD_CUDA(cudaMemcpyAsync(d_row_of_pos, keys.Current(), eb, cudaMemcpyDeviceToDevice, ctx->stream));
-    BUILD_CUDA(cudaStreamSynchronize(ctx->stream));
-    cleanup();
+        CUDA_TRY(cudaMemcpyAsync(d_row_of_pos, keys.Current(), eb, cudaMemcpyDeviceToDevice, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return VGLB_OK;
 }
 
@@ -370,21 +331,52 @@ static int build_outgoing(vglb_ctx *ctx, int32_t V, int64_t E, const int32_t *d_
 static int build_incoming(vglb_ctx *ctx, int32_t V, int64_t E, const int32_t *d_out_adj, uint32_t *d_row_of_pos,
                           int32_t *d_in_adj)
 {
-    uint32_t *k0 = NULL, *k1 = NULL, *v1 = NULL;
-    void *tmp = NULL;
-    auto cleanup = [&]() { vglb_dev_free(k0); vglb_dev_free(k1); vglb_dev_free(v1); vglb_dev_free(tmp); };
     if (E == 0) return VGLB_OK;
     const size_t eb = (size_t)E * sizeof(uint32_t);
-    BUILD_CUDA(vglb_dev_alloc(&k0, eb)); BUILD_CUDA(vglb_dev_alloc(&k1, eb)); BUILD_CUDA(vglb_dev_alloc(&v1, eb));
-    BUILD_CUDA(cudaMemcpyAsync(k0, d_out_adj, eb, cudaMemcpyDeviceToDevice, ctx->stream));
-    cub::DoubleBuffer<uint32_t> keys(k0, k1), vals(d_row_of_pos, v1);
-    size_t tmp_bytes = 0;
-    BUILD_CUDA(cub::DeviceRadixSort::SortPairs(NULL, tmp_bytes, keys, vals, E, 0, bits_for(V), ctx->stream));
-    BUILD_CUDA(vglb_dev_alloc(&tmp, tmp_bytes ? tmp_bytes : 16));
-    BUILD_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, keys, vals, E, 0, bits_for(V), ctx->stream));
-    BUILD_CUDA(cudaMemcpyAsync(d_in_adj, vals.Current(), eb, cudaMemcpyDeviceToDevice, ctx->stream));
-    BUILD_CUDA(cudaStreamSynchronize(ctx->stream));
-    cleanup();
+    dev_ptr<uint32_t> k0, k1, v1;
+    dev_ptr<void> tmp;
+    CUDA_TRY(vglb_dev_alloc(k0, eb)); CUDA_TRY(vglb_dev_alloc(k1, eb)); CUDA_TRY(vglb_dev_alloc(v1, eb));
+    CUDA_TRY(cudaMemcpyAsync(k0.get(), d_out_adj, eb, cudaMemcpyDeviceToDevice, ctx->stream));
+    cub::DoubleBuffer<uint32_t> keys(k0.get(), k1.get()), vals(d_row_of_pos, v1.get());
+    CUDA_TRY(vglb_cub(tmp, [&](void *t, size_t &bytes) {
+        return cub::DeviceRadixSort::SortPairs(t, bytes, keys, vals, E, 0, vglb_key_bits(V), ctx->stream);
+    }));
+    CUDA_TRY(cudaMemcpyAsync(d_in_adj, vals.Current(), eb, cudaMemcpyDeviceToDevice, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    return VGLB_OK;
+}
+
+int vglb_degree_order(vglb_ctx *ctx, const int32_t *d_deg, int32_t V, DegreeOrder &order)
+{
+    for (auto *p : {&order.keys[0], &order.keys[1], &order.ids[0], &order.ids[1]}) CUDA_TRY(vglb_dev_alloc(*p, (size_t)V * 4));
+    degree_sort_keys_kernel<<<(unsigned)ceil_div64(V, 256), 256, 0, ctx->stream>>>(d_deg, V, order.keys[0].get(), order.ids[0].get());
+    KERNEL_TRY();
+    cub::DoubleBuffer<uint32_t> keys(order.keys[0].get(), order.keys[1].get()), vals(order.ids[0].get(), order.ids[1].get());
+    CUDA_TRY(vglb_cub(order.tmp, [&](void *t, size_t &bytes) {
+        return cub::DeviceRadixSort::SortPairs(t, bytes, keys, vals, V, 0, 32, ctx->stream);
+    }));
+    order.sorted = vals.Current();
+    return VGLB_OK;
+}
+
+int vglb_csr_validate_device(vglb_ctx *ctx, const int64_t *d_ptr, int32_t rows, int64_t E, const int32_t *d_adj, int64_t id_limit)
+{
+    int *d_bad = (int *)(ctx->d_counters + CTR_BAD);
+    csr_ptr_check_kernel<<<(unsigned)ceil_div64((int64_t)rows + 1, 256), 256, 0, ctx->stream>>>(d_ptr, rows, E, d_bad);
+    KERNEL_TRY();
+    if (E > 0)
+    {
+        id_range_check_kernel<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(d_adj, E, id_limit, d_bad);
+        KERNEL_TRY();
+    }
+    return VGLB_OK;
+}
+
+int vglb_invert_map_checked(vglb_ctx *ctx, const int32_t *d_fwd, int32_t n, int64_t limit, int32_t *d_bwd)
+{
+    invert_map_checked_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, ctx->stream>>>(d_fwd, n, limit, d_bwd,
+                                                                                     (int *)(ctx->d_counters + CTR_BAD));
+    KERNEL_TRY();
     return VGLB_OK;
 }
 
@@ -395,116 +387,97 @@ extern "C" int vglb_graph_from_edges(vglb_ctx *ctx, int32_t V, int64_t E, const 
     VGLB_REQUIRE(V > 0 && E >= 0 && E < 0xFFFFFFFFLL, "vglb_graph_from_edges: need V > 0 and 0 <= E < 2^32-1 per device");
     VGLB_REQUIRE(E == 0 || (src != NULL && dst != NULL), "vglb_graph_from_edges: NULL edge arrays");
     CUDA_TRY(cudaSetDevice(ctx->device));
-    vglb_graph *g = (vglb_graph *)calloc(1, sizeof(vglb_graph));
-    if (!g) return VGLB_ENOMEM;
+    graph_ptr owner = vglb_graph_new();
+    if (!owner) return VGLB_ENOMEM;
+    vglb_graph *g = owner.get();
     g->V = V;
     g->E = E;
-    int32_t *d_src_own = NULL, *d_dst_own = NULL, *d_deg = NULL;
-    uint32_t *dk0 = NULL, *dk1 = NULL, *dv0 = NULL, *dv1 = NULL, *d_row_of_pos = NULL;
-    int64_t *d_deg_sorted = NULL;
-    void *tmp = NULL;
-    int *d_bad = NULL;
-    auto cleanup = [&]() {
-        vglb_dev_free(d_src_own); vglb_dev_free(d_dst_own); vglb_dev_free(d_deg); vglb_dev_free(dk0); vglb_dev_free(dk1); vglb_dev_free(dv0);
-        vglb_dev_free(dv1); vglb_dev_free(d_deg_sorted); vglb_dev_free(tmp); vglb_dev_free(d_bad); vglb_dev_free(d_row_of_pos);
-        vglb_graph_free_fields(g);
-        free(g);
-    };
+    dev_ptr<int32_t> d_src_own, d_dst_own, d_deg;
+    dev_ptr<int64_t> d_deg_sorted;
+    dev_ptr<uint32_t> d_row_of_pos;
+    dev_ptr<int> d_bad;
     const int32_t *d_src = src, *d_dst = dst;
     const size_t eb = (size_t)(E ? E : 1) * sizeof(int32_t);
     if (!src_on_device)
     {
-        BUILD_CUDA(vglb_dev_alloc(&d_src_own, eb));
-        BUILD_CUDA(vglb_dev_alloc(&d_dst_own, eb));
-        BUILD_CUDA(cudaMemcpyAsync(d_src_own, src, (size_t)E * 4, cudaMemcpyHostToDevice, ctx->stream));
-        BUILD_CUDA(cudaMemcpyAsync(d_dst_own, dst, (size_t)E * 4, cudaMemcpyHostToDevice, ctx->stream));
-        d_src = d_src_own;
-        d_dst = d_dst_own;
+        CUDA_TRY(vglb_dev_alloc(d_src_own, eb));
+        CUDA_TRY(vglb_dev_alloc(d_dst_own, eb));
+        CUDA_TRY(cudaMemcpyAsync(d_src_own.get(), src, (size_t)E * 4, cudaMemcpyHostToDevice, ctx->stream));
+        CUDA_TRY(cudaMemcpyAsync(d_dst_own.get(), dst, (size_t)E * 4, cudaMemcpyHostToDevice, ctx->stream));
+        d_src = d_src_own.get();
+        d_dst = d_dst_own.get();
     }
     const int grid = ctx->sm_count * 16;
     const unsigned vgrid = (unsigned)ceil_div64((int64_t)V + 1, 256);
 
     // 1. out-degree histogram (extract_connection_count)
-    BUILD_CUDA(vglb_dev_alloc(&d_deg, (size_t)V * 4));
-    BUILD_CUDA(vglb_dev_alloc(&d_bad, 4));
-    BUILD_CUDA(cudaMemsetAsync(d_deg, 0, (size_t)V * 4, ctx->stream));
-    BUILD_CUDA(cudaMemsetAsync(d_bad, 0, 4, ctx->stream));
+    CUDA_TRY(vglb_dev_alloc(d_deg, (size_t)V * 4));
+    CUDA_TRY(vglb_dev_alloc(d_bad, 4));
+    CUDA_TRY(cudaMemsetAsync(d_deg.get(), 0, (size_t)V * 4, ctx->stream));
+    CUDA_TRY(cudaMemsetAsync(d_bad.get(), 0, 4, ctx->stream));
     if (E)
     {
-        degree_histogram_kernel<<<grid, 256, 0, ctx->stream>>>(d_src, E, V, d_deg, d_bad);
-        BUILD_CUDA(cudaGetLastError());
-        range_check_kernel<<<grid, 256, 0, ctx->stream>>>(d_dst, E, V, d_bad);
-        BUILD_CUDA(cudaGetLastError());
+        degree_histogram_kernel<<<grid, 256, 0, ctx->stream>>>(d_src, E, V, d_deg.get(), d_bad.get());
+        KERNEL_TRY();
+        id_range_check_kernel<<<grid, 256, 0, ctx->stream>>>(d_dst, E, V, d_bad.get());
+        KERNEL_TRY();
     }
     int bad = 0;
-    BUILD_CUDA(cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, ctx->stream));
-    BUILD_CUDA(cudaStreamSynchronize(ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(&bad, d_bad.get(), 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     if (bad)
     {
         vglb_set_error("vglb_graph_from_edges: vertex id out of range [0, V)");
-        cleanup();
         return VGLB_EINVAL;
     }
     // 2. stable sort of vertex ids by degree descending (sort_vertices_by_degree)
-    BUILD_CUDA(vglb_dev_alloc(&dk0, (size_t)V * 4)); BUILD_CUDA(vglb_dev_alloc(&dk1, (size_t)V * 4));
-    BUILD_CUDA(vglb_dev_alloc(&dv0, (size_t)V * 4)); BUILD_CUDA(vglb_dev_alloc(&dv1, (size_t)V * 4));
-    degree_sort_keys_kernel<<<vgrid, 256, 0, ctx->stream>>>(d_deg, V, dk0, dv0);
-    BUILD_CUDA(cudaGetLastError());
     {
-        cub::DoubleBuffer<uint32_t> keys(dk0, dk1), vals(dv0, dv1);
-        size_t tmp_bytes = 0;
-        BUILD_CUDA(cub::DeviceRadixSort::SortPairs(NULL, tmp_bytes, keys, vals, V, 0, 32, ctx->stream));
-        BUILD_CUDA(vglb_dev_alloc(&tmp, tmp_bytes ? tmp_bytes : 16));
-        BUILD_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, keys, vals, V, 0, 32, ctx->stream));
-        BUILD_CUDA(vglb_dev_alloc(&g->d_fwd, (size_t)V * 4));
-        BUILD_CUDA(vglb_dev_alloc(&g->d_bwd, (size_t)V * 4));
-        BUILD_CUDA(vglb_dev_alloc(&d_deg_sorted, ((size_t)V + 1) * 8));
-        conversions_kernel<<<vgrid, 256, 0, ctx->stream>>>(vals.Current(), d_deg, V, g->d_fwd, g->d_bwd, d_deg_sorted);
-        BUILD_CUDA(cudaGetLastError());
-        BUILD_CUDA(cudaStreamSynchronize(ctx->stream));
-        vglb_dev_free(tmp); tmp = NULL;
+        DegreeOrder order;
+        VGLB_TRY(vglb_degree_order(ctx, d_deg.get(), V, order));
+        CUDA_TRY(vglb_dev_alloc(&g->d_fwd, (size_t)V * 4));
+        CUDA_TRY(vglb_dev_alloc(&g->d_bwd, (size_t)V * 4));
+        CUDA_TRY(vglb_dev_alloc(d_deg_sorted, ((size_t)V + 1) * 8));
+        conversions_kernel<<<vgrid, 256, 0, ctx->stream>>>(order.sorted, d_deg.get(), V, g->d_fwd, g->d_bwd, d_deg_sorted.get());
+        KERNEL_TRY();
+        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     }
-    vglb_dev_free(dk0); vglb_dev_free(dk1); vglb_dev_free(dv0); vglb_dev_free(dv1);
-    dk0 = dk1 = dv0 = dv1 = NULL;
     // 3. row pointers (construct_CSR)
-    BUILD_CUDA(vglb_dev_alloc(&g->d_out_ptr, ((size_t)V + 2) * 8));
+    CUDA_TRY(vglb_dev_alloc(&g->d_out_ptr, ((size_t)V + 2) * 8));
     {
-        size_t tmp_bytes = 0;
-        BUILD_CUDA(cub::DeviceScan::ExclusiveSum(NULL, tmp_bytes, d_deg_sorted, g->d_out_ptr, V + 1, ctx->stream));
-        BUILD_CUDA(vglb_dev_alloc(&tmp, tmp_bytes ? tmp_bytes : 16));
-        BUILD_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, d_deg_sorted, g->d_out_ptr, V + 1, ctx->stream));
-        BUILD_CUDA(cudaStreamSynchronize(ctx->stream));
-        vglb_dev_free(tmp); tmp = NULL;
+        dev_ptr<void> tmp;
+        CUDA_TRY(vglb_cub(tmp, [&](void *t, size_t &bytes) {
+            return cub::DeviceScan::ExclusiveSum(t, bytes, d_deg_sorted.get(), g->d_out_ptr, V + 1, ctx->stream);
+        }));
+        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     }
     // 4. edges: stable sort by new src id, adjacency in new ids (renumber + preprocess_into_csr_based)
-    BUILD_CUDA(vglb_dev_alloc(&g->d_out_adj, eb + 16));
-    if (flags & VGLB_GRAPH_WITH_EDGE_ORDER) BUILD_CUDA(vglb_dev_alloc(&g->d_edge_order, (size_t)(E ? E : 1) * 8));
-    if ((flags & VGLB_GRAPH_WITH_INCOMING) && E) BUILD_CUDA(vglb_dev_alloc(&d_row_of_pos, eb));
-    BUILD_TRY(build_outgoing(ctx, V, E, d_src, d_dst, g->d_fwd, g->d_out_adj, g->d_edge_order, d_row_of_pos));
+    CUDA_TRY(vglb_dev_alloc(&g->d_out_adj, eb + 16));
+    if (flags & VGLB_GRAPH_WITH_EDGE_ORDER) CUDA_TRY(vglb_dev_alloc(&g->d_edge_order, (size_t)(E ? E : 1) * 8));
+    if ((flags & VGLB_GRAPH_WITH_INCOMING) && E) CUDA_TRY(vglb_dev_alloc(d_row_of_pos, eb));
+    VGLB_TRY(build_outgoing(ctx, V, E, d_src, d_dst, g->d_fwd, g->d_out_adj, g->d_edge_order, d_row_of_pos.get()));
     // 5. incoming CSR on the same numbering
     if (flags & VGLB_GRAPH_WITH_INCOMING)
     {
-        BUILD_CUDA(cudaMemsetAsync(d_deg_sorted, 0, ((size_t)V + 1) * 8, ctx->stream));
+        CUDA_TRY(cudaMemsetAsync(d_deg_sorted.get(), 0, ((size_t)V + 1) * 8, ctx->stream));
         if (E)
         {
-            indegree_sorted_kernel<<<grid, 256, 0, ctx->stream>>>(d_dst, g->d_fwd, E, (unsigned long long *)d_deg_sorted);
-            BUILD_CUDA(cudaGetLastError());
+            indegree_sorted_kernel<<<grid, 256, 0, ctx->stream>>>(d_dst, g->d_fwd, E, (unsigned long long *)d_deg_sorted.get());
+            KERNEL_TRY();
         }
-        BUILD_CUDA(vglb_dev_alloc(&g->d_in_ptr, ((size_t)V + 2) * 8));
-        size_t tmp_bytes = 0;
-        BUILD_CUDA(cub::DeviceScan::ExclusiveSum(NULL, tmp_bytes, d_deg_sorted, g->d_in_ptr, V + 1, ctx->stream));
-        BUILD_CUDA(vglb_dev_alloc(&tmp, tmp_bytes ? tmp_bytes : 16));
-        BUILD_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, d_deg_sorted, g->d_in_ptr, V + 1, ctx->stream));
-        BUILD_CUDA(cudaStreamSynchronize(ctx->stream));
-        vglb_dev_free(tmp); tmp = NULL;
-        BUILD_CUDA(vglb_dev_alloc(&g->d_in_adj, eb + 16));
-        BUILD_TRY(build_incoming(ctx, V, E, g->d_out_adj, d_row_of_pos, g->d_in_adj));
+        CUDA_TRY(vglb_dev_alloc(&g->d_in_ptr, ((size_t)V + 2) * 8));
+        {
+            dev_ptr<void> tmp;
+            CUDA_TRY(vglb_cub(tmp, [&](void *t, size_t &bytes) {
+                return cub::DeviceScan::ExclusiveSum(t, bytes, d_deg_sorted.get(), g->d_in_ptr, V + 1, ctx->stream);
+            }));
+            CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+        }
+        CUDA_TRY(vglb_dev_alloc(&g->d_in_adj, eb + 16));
+        VGLB_TRY(build_incoming(ctx, V, E, g->d_out_adj, d_row_of_pos.get(), g->d_in_adj));
     }
-    BUILD_TRY(vglb_graph_compute_tiers(ctx, g));
+    VGLB_TRY(vglb_graph_compute_tiers(ctx, g));
     vglb_graph_set_unpartitioned(g);
-    vglb_dev_free(d_src_own); vglb_dev_free(d_dst_own); vglb_dev_free(d_deg); vglb_dev_free(d_deg_sorted); vglb_dev_free(d_bad);
-    vglb_dev_free(d_row_of_pos);
-    *out_graph = g;
+    *out_graph = owner.release();
     return VGLB_OK;
 }
 
@@ -523,18 +496,17 @@ extern "C" int vglb_graph_from_csr(vglb_ctx *ctx, int32_t V, int64_t E, const in
     VGLB_REQUIRE(V > 0 && E >= 0 && (E == 0 || h_out_adj != NULL), "vglb_graph_from_csr: bad sizes");
     VGLB_REQUIRE((h_in_ptr == NULL) == (h_in_adj == NULL) || E == 0, "vglb_graph_from_csr: incoming arrays must come together");
     CUDA_TRY(cudaSetDevice(ctx->device));
-    vglb_graph *g = (vglb_graph *)calloc(1, sizeof(vglb_graph));
-    if (!g) return VGLB_ENOMEM;
+    graph_ptr owner = vglb_graph_new();
+    if (!owner) return VGLB_ENOMEM;
+    vglb_graph *g = owner.get();
     g->V = V;
     g->E = E;
-    auto cleanup = [&]() { vglb_graph_free_fields(g); free(g); };
     // The arrays come from the caller or straight from a .vgl file (vglb_graph_load_vgl): nothing below may index with
     // a value that has not been checked. Host side: the end points and every chunk border used for a copy; device side
-    // (csr_ptr_check_kernel, the guarded in-degree pass, range_check_kernel, invert_perm_checked_kernel): the rest.
+    // (csr_ptr_check_kernel, the guarded in-degree pass, vglb_csr_validate_device, vglb_invert_map_checked): the rest.
     if (h_out_ptr[0] != 0 || h_out_ptr[V] != E || (h_in_ptr && (h_in_ptr[0] != 0 || h_in_ptr[V] != E)))
     {
         vglb_set_error("vglb_graph_from_csr: row pointers must start at 0 and end at the edge count");
-        cleanup();
         return VGLB_EINVAL;
     }
     const bool csr_trace = getenv("VGLB_CSR_TRACE") != NULL; // developer aid: host timeline of the upload on stderr
@@ -547,21 +519,21 @@ extern "C" int vglb_graph_from_csr(vglb_ctx *ctx, int32_t V, int64_t E, const in
         fprintf(stderr, "from_csr: %-44s %8.2f ms\n", what, 1e3 * (double)(ts.tv_sec - ts0.tv_sec) + 1e-6 * (double)(ts.tv_nsec - ts0.tv_nsec));
     };
     int *d_bad = (int *)(ctx->d_counters + CTR_BAD);
-    BUILD_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int), ctx->stream));
+    CUDA_TRY(cudaMemsetAsync(d_bad, 0, sizeof(int), ctx->stream));
     const size_t eb = (size_t)(E ? E : 1) * 4;
-    BUILD_CUDA(vglb_dev_alloc(&g->d_out_ptr, ((size_t)V + 2) * 8));
+    CUDA_TRY(vglb_dev_alloc(&g->d_out_ptr, ((size_t)V + 2) * 8));
     stamp("first allocation");
-    BUILD_CUDA(vglb_dev_alloc(&g->d_out_adj, eb + 16));
+    CUDA_TRY(vglb_dev_alloc(&g->d_out_adj, eb + 16));
     // The upload is PCIe-bound (1.3 GB at ~55 GB/s for the BASELINE PageRank graph), so the device works while it runs: the
     // adjacency goes up in 8 row-aligned chunks on a second stream and the in-degrees without self loops — what PageRank's
     // preparation needs first (pr.hpp:28-73), a 7 ms pass of atomics — are counted chunk by chunk behind it.
-    BUILD_CUDA(cudaMemcpyAsync(g->d_out_ptr, h_out_ptr, ((size_t)V + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
-    BUILD_CUDA(vglb_dev_alloc(&g->d_indeg_noloops, (size_t)V * 4));
-    BUILD_CUDA(cudaMemsetAsync(g->d_indeg_noloops, 0, (size_t)V * 4, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(g->d_out_ptr, h_out_ptr, ((size_t)V + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(vglb_dev_alloc(&g->d_indeg_noloops, (size_t)V * 4));
+    CUDA_TRY(cudaMemsetAsync(g->d_indeg_noloops, 0, (size_t)V * 4, ctx->stream));
     csr_ptr_check_kernel<<<(unsigned)ceil_div64((int64_t)V + 1, 256), 256, 0, ctx->stream>>>(g->d_out_ptr, V, E, d_bad);
-    BUILD_CUDA(cudaGetLastError());
-    BUILD_CUDA(cudaEventRecord(ctx->ev_chunk[0], ctx->stream));
-    BUILD_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_chunk[0], 0)); // (orders the copy stream after earlier work on the buffers)
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaEventRecord(ctx->ev_chunk[0], ctx->stream));
+    CUDA_TRY(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_chunk[0], 0)); // (orders the copy stream after earlier work on the buffers)
     const int chunks = E >= (1 << 22) ? 8 : 1;
     // rows are degree-sorted: binary search the first row with fewer than d edges
     auto rows_with_degree_at_least = [&](int64_t d) {
@@ -621,17 +593,16 @@ extern "C" int vglb_graph_from_csr(vglb_ctx *ctx, int32_t V, int64_t E, const in
             cudaStreamSynchronize(ctx->copy_stream);
             cudaStreamSynchronize(ctx->stream);
             vglb_set_error("vglb_graph_from_csr: row pointers are not non-decreasing within [0, E]");
-            cleanup();
             return VGLB_EINVAL;
         }
     }
     // the other arrays of the caller: queued on the copy stream behind the adjacency (before the host waits for anything)
-    BUILD_CUDA(vglb_dev_alloc(&g->d_fwd, (size_t)V * 4));
-    BUILD_CUDA(vglb_dev_alloc(&g->d_bwd, (size_t)V * 4));
+    CUDA_TRY(vglb_dev_alloc(&g->d_fwd, (size_t)V * 4));
+    CUDA_TRY(vglb_dev_alloc(&g->d_bwd, (size_t)V * 4));
     if (h_in_ptr)
     {
-        BUILD_CUDA(vglb_dev_alloc(&g->d_in_ptr, ((size_t)V + 2) * 8));
-        BUILD_CUDA(vglb_dev_alloc(&g->d_in_adj, eb + 16));
+        CUDA_TRY(vglb_dev_alloc(&g->d_in_ptr, ((size_t)V + 2) * 8));
+        CUDA_TRY(vglb_dev_alloc(&g->d_in_adj, eb + 16));
     }
     bool others_queued = false;
     auto queue_others = [&]() -> cudaError_t {
@@ -648,10 +619,10 @@ extern "C" int vglb_graph_from_csr(vglb_ctx *ctx, int32_t V, int64_t E, const in
         {
             const int64_t e0 = h_out_ptr[border[k]], e1 = h_out_ptr[border[k + 1]];
             if (e1 > e0)
-                BUILD_CUDA(cudaMemcpyAsync(g->d_out_adj + e0, h_out_adj + e0, (size_t)(e1 - e0) * 4, cudaMemcpyHostToDevice, ctx->copy_stream));
-            BUILD_CUDA(cudaEventRecord(ctx->ev_chunk[k], ctx->copy_stream));
+                CUDA_TRY(cudaMemcpyAsync(g->d_out_adj + e0, h_out_adj + e0, (size_t)(e1 - e0) * 4, cudaMemcpyHostToDevice, ctx->copy_stream));
+            CUDA_TRY(cudaEventRecord(ctx->ev_chunk[k], ctx->copy_stream));
         }
-    if (heavy_chunk >= 0) BUILD_CUDA(queue_others());
+    if (heavy_chunk >= 0) CUDA_TRY(queue_others());
     for (int k = 0; k < chunks; k++)
     {
         const int32_t row0 = border[k], row1 = border[k + 1];
@@ -660,10 +631,10 @@ extern "C" int vglb_graph_from_csr(vglb_ctx *ctx, int32_t V, int64_t E, const in
         {
             if (heavy_chunk < 0)
             {
-                BUILD_CUDA(cudaMemcpyAsync(g->d_out_adj + e0, h_out_adj + e0, (size_t)(e1 - e0) * 4, cudaMemcpyHostToDevice, ctx->copy_stream));
-                BUILD_CUDA(cudaEventRecord(ctx->ev_chunk[k], ctx->copy_stream));
+                CUDA_TRY(cudaMemcpyAsync(g->d_out_adj + e0, h_out_adj + e0, (size_t)(e1 - e0) * 4, cudaMemcpyHostToDevice, ctx->copy_stream));
+                CUDA_TRY(cudaEventRecord(ctx->ev_chunk[k], ctx->copy_stream));
             }
-            BUILD_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_chunk[k], 0));
+            CUDA_TRY(cudaStreamWaitEvent(ctx->stream, ctx->ev_chunk[k], 0));
             // (rows are degree-sorted: a chunk that starts at or after the first row with fewer than 32 edges has only such rows)
             if (row0 >= short_rows_from)
                 indegree_noloops_short_rows_kernel<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(g->d_out_ptr, g->d_out_adj, row0, row1, e0, e1, V,
@@ -671,7 +642,7 @@ extern "C" int vglb_graph_from_csr(vglb_ctx *ctx, int32_t V, int64_t E, const in
             else
                 indegree_noloops_rows_kernel<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(g->d_out_ptr, g->d_out_adj, row0, row1, e0, e1, V,
                                                                                          g->d_indeg_noloops, d_bad);
-            BUILD_CUDA(cudaGetLastError());
+            CUDA_TRY(cudaGetLastError());
             ctx->launches++;
         }
         if (k == heavy_chunk)
@@ -679,63 +650,52 @@ extern "C" int vglb_graph_from_csr(vglb_ctx *ctx, int32_t V, int64_t E, const in
             // (the row pointers were checked by csr_ptr_check_kernel: a bad array fails the call below, not the build)
             int bad = 0;
             stamp("copies queued");
-            BUILD_CUDA(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-            BUILD_CUDA(cudaStreamSynchronize(ctx->stream));
+            CUDA_TRY(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+            CUDA_TRY(cudaStreamSynchronize(ctx->stream));
             stamp("heavy rows have landed");
             if (!bad)
             {
                 g->pr_bins_tried = 1;
                 const int rcb = vglb_pr_bins_build_rows(ctx, g, heavy_rows);
-                if (rcb != VGLB_OK && rcb != VGLB_ENOMEM) BUILD_TRY(rcb); // (no memory for the binned copy: PageRank falls back to warp tasks)
+                if (rcb != VGLB_ENOMEM) VGLB_TRY(rcb); // (no memory for the binned copy: PageRank falls back to warp tasks)
                 stamp("column bins built");
             }
         }
     }
-    BUILD_CUDA(queue_others());
+    CUDA_TRY(queue_others());
     const unsigned vgrid = (unsigned)ceil_div64(V, 256);
     if (chunks > 1 && !vglb_pr_bins_wanted(g))
     {
         // the host is idle while the DMA runs: PageRank's warp-task table of the rows with >= 32 edges (pagerank.cu) is built
         // from the caller's row pointers now instead of costing 3-4 ms later
-        BUILD_TRY(vglb_pr_build_tasks_host(ctx, g, h_out_ptr, rows_with_degree_at_least(vglb_tier_degree(1)),
+        VGLB_TRY(vglb_pr_build_tasks_host(ctx, g, h_out_ptr, rows_with_degree_at_least(vglb_tier_degree(1)),
                                            rows_with_degree_at_least(vglb_tier_degree(0))));
     }
-    BUILD_CUDA(cudaEventRecord(ctx->ev_chunk[0], ctx->copy_stream));
-    BUILD_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_chunk[0], 0)); // every upload is ordered before later work on `stream`
+    CUDA_TRY(cudaEventRecord(ctx->ev_chunk[0], ctx->copy_stream));
+    CUDA_TRY(cudaStreamWaitEvent(ctx->stream, ctx->ev_chunk[0], 0)); // every upload is ordered before later work on `stream`
     if (!h_orig_to_sorted)
     {
         iota_kernel<<<vgrid, 256, 0, ctx->stream>>>(g->d_fwd, V);
-        BUILD_CUDA(cudaGetLastError());
+        CUDA_TRY(cudaGetLastError());
     }
-    BUILD_CUDA(cudaMemsetAsync(g->d_bwd, 0xFF, (size_t)V * 4, ctx->stream));
-    invert_perm_checked_kernel<<<vgrid, 256, 0, ctx->stream>>>(g->d_fwd, g->d_bwd, V, d_bad);
-    BUILD_CUDA(cudaGetLastError());
-    if (h_in_ptr)
-    {
-        csr_ptr_check_kernel<<<(unsigned)ceil_div64((int64_t)V + 1, 256), 256, 0, ctx->stream>>>(g->d_in_ptr, V, E, d_bad);
-        BUILD_CUDA(cudaGetLastError());
-        if (E)
-        {
-            range_check_kernel<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(g->d_in_adj, E, V, d_bad);
-            BUILD_CUDA(cudaGetLastError());
-        }
-    }
+    CUDA_TRY(cudaMemsetAsync(g->d_bwd, 0xFF, (size_t)V * 4, ctx->stream));
+    VGLB_TRY(vglb_invert_map_checked(ctx, g->d_fwd, V, V, g->d_bwd));
+    if (h_in_ptr) VGLB_TRY(vglb_csr_validate_device(ctx, g->d_in_ptr, V, E, g->d_in_adj, V));
     int bad = 0;
     stamp("checks queued");
-    BUILD_CUDA(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-    BUILD_CUDA(cudaStreamSynchronize(ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     stamp("uploads and checks done");
     if (bad)
     {
         vglb_set_error("vglb_graph_from_csr: not a CSR (row pointers must be non-decreasing from 0 to E, vertex ids in [0, V), "
                        "the ORIGINAL -> sorted map a permutation)");
-        cleanup();
         return VGLB_EINVAL;
     }
-    BUILD_TRY(vglb_graph_compute_tiers(ctx, g));
+    VGLB_TRY(vglb_graph_compute_tiers(ctx, g));
     stamp("tiers");
     vglb_graph_set_unpartitioned(g);
-    *out_graph = g;
+    *out_graph = owner.release();
     return VGLB_OK;
 }
 
@@ -748,43 +708,17 @@ extern "C" int vglb_graph_borrow_csr(vglb_ctx *ctx, int32_t V, int64_t E, const 
     VGLB_REQUIRE(ctx != NULL && out_graph != NULL && d_ptr != NULL, "vglb_graph_borrow_csr: NULL argument");
     VGLB_REQUIRE(V > 0 && E >= 0 && (E == 0 || d_adj != NULL), "vglb_graph_borrow_csr: bad sizes");
     CUDA_TRY(cudaSetDevice(ctx->device));
-    vglb_graph *g = (vglb_graph *)calloc(1, sizeof(vglb_graph));
-    if (!g) return VGLB_ENOMEM;
+    graph_ptr owner = vglb_graph_new();
+    if (!owner) return VGLB_ENOMEM;
+    vglb_graph *g = owner.get();
     g->V = V;
     g->E = E;
     g->borrowed_csr = 1;
     g->d_out_ptr = const_cast<int64_t *>(d_ptr);
     g->d_out_adj = const_cast<int32_t *>(d_adj);
-    int rc = vglb_graph_compute_tiers(ctx, g); // also rejects rows that are not degree-sorted (VGLB_EUNSORTED)
-    if (rc != VGLB_OK)
-    {
-        free(g);
-        return rc;
-    }
+    VGLB_TRY(vglb_graph_compute_tiers(ctx, g)); // also rejects rows that are not degree-sorted (VGLB_EUNSORTED)
     vglb_graph_set_unpartitioned(g);
-    *out_graph = g;
-    return VGLB_OK;
-}
-
-int vglb_csr_validate_device(vglb_ctx *ctx, const int64_t *d_ptr, int32_t rows, int64_t E, const int32_t *d_adj, int64_t id_limit)
-{
-    int *d_bad = (int *)(ctx->d_counters + CTR_BAD);
-    CUDA_TRY(cudaMemsetAsync(d_bad, 0, sizeof(int), ctx->stream));
-    csr_ptr_check_kernel<<<(unsigned)ceil_div64((int64_t)rows + 1, 256), 256, 0, ctx->stream>>>(d_ptr, rows, E, d_bad);
-    KERNEL_TRY();
-    if (E > 0)
-    {
-        range_check_kernel<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(d_adj, E, (int32_t)id_limit, d_bad);
-        KERNEL_TRY();
-    }
-    int bad = 0;
-    CUDA_TRY(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    if (bad)
-    {
-        vglb_set_error("not a CSR: row pointers must be non-decreasing from 0 to the edge count and ids in range");
-        return VGLB_EINVAL;
-    }
+    *out_graph = owner.release();
     return VGLB_OK;
 }
 
@@ -812,29 +746,29 @@ int vglb_graph_derive_incoming(vglb_ctx *ctx, vglb_graph *g)
     const int32_t V = g->V;
     const int64_t E = g->E;
     const size_t eb = (size_t)(E ? E : 1) * 4;
-    uint32_t *d_row_of_pos = NULL;
-    int64_t *d_deg = NULL;
-    void *tmp = NULL;
-    auto cleanup = [&]() { vglb_dev_free(d_row_of_pos); vglb_dev_free(d_deg); vglb_dev_free(tmp); };
-    BUILD_CUDA(vglb_dev_alloc(&d_deg, ((size_t)V + 2) * 8));
-    BUILD_CUDA(cudaMemsetAsync(d_deg, 0, ((size_t)V + 2) * 8, ctx->stream));
-    BUILD_CUDA(vglb_dev_alloc(&g->d_in_ptr, ((size_t)V + 2) * 8));
-    BUILD_CUDA(vglb_dev_alloc(&g->d_in_adj, eb + 16));
+    dev_ptr<int64_t> d_deg, in_ptr;
+    dev_ptr<int32_t> in_adj;
+    dev_ptr<uint32_t> d_row_of_pos;
+    dev_ptr<void> tmp;
+    CUDA_TRY(vglb_dev_alloc(d_deg, ((size_t)V + 2) * 8));
+    CUDA_TRY(cudaMemsetAsync(d_deg.get(), 0, ((size_t)V + 2) * 8, ctx->stream));
+    CUDA_TRY(vglb_dev_alloc(in_ptr, ((size_t)V + 2) * 8));
+    CUDA_TRY(vglb_dev_alloc(in_adj, eb + 16));
     if (E)
     {
-        BUILD_CUDA(vglb_dev_alloc(&d_row_of_pos, eb));
-        row_of_position_kernel<<<ctx->sm_count * 16, 256, 0, ctx->stream>>>(g->d_out_ptr, V, d_row_of_pos);
-        BUILD_CUDA(cudaGetLastError());
-        indegree_from_adj_kernel<<<ctx->sm_count * 16, 256, 0, ctx->stream>>>(g->d_out_adj, E, (unsigned long long *)d_deg);
-        BUILD_CUDA(cudaGetLastError());
+        CUDA_TRY(vglb_dev_alloc(d_row_of_pos, eb));
+        row_of_position_kernel<<<ctx->sm_count * 16, 256, 0, ctx->stream>>>(g->d_out_ptr, V, d_row_of_pos.get());
+        KERNEL_TRY();
+        indegree_from_adj_kernel<<<ctx->sm_count * 16, 256, 0, ctx->stream>>>(g->d_out_adj, E, (unsigned long long *)d_deg.get());
+        KERNEL_TRY();
     }
-    size_t tmp_bytes = 0;
-    BUILD_CUDA(cub::DeviceScan::ExclusiveSum(NULL, tmp_bytes, d_deg, g->d_in_ptr, V + 1, ctx->stream));
-    BUILD_CUDA(vglb_dev_alloc(&tmp, tmp_bytes ? tmp_bytes : 16));
-    BUILD_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, d_deg, g->d_in_ptr, V + 1, ctx->stream));
-    BUILD_CUDA(cudaStreamSynchronize(ctx->stream));
-    BUILD_TRY(build_incoming(ctx, V, E, g->d_out_adj, d_row_of_pos, g->d_in_adj));
-    cleanup();
+    CUDA_TRY(vglb_cub(tmp, [&](void *t, size_t &bytes) {
+        return cub::DeviceScan::ExclusiveSum(t, bytes, d_deg.get(), in_ptr.get(), V + 1, ctx->stream);
+    }));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    VGLB_TRY(build_incoming(ctx, V, E, g->d_out_adj, d_row_of_pos.get(), in_adj.get()));
+    g->d_in_ptr = in_ptr.release(); // (the graph gets its incoming CSR only when it is complete)
+    g->d_in_adj = in_adj.release();
     return VGLB_OK;
 }
 
@@ -927,20 +861,16 @@ extern "C" int vglb_varray_reorder_u32(vglb_ctx *ctx, vglb_graph *g, const uint3
             ctx->launches++;
             return VGLB_OK;
         }
-        uint32_t *full = NULL;
-        CUDA_TRY(vglb_dev_alloc(&full, (size_t)g->cols * 4));
-        CUDA_TRY(cudaMemsetAsync(full + g->col_of_row0, 0, (size_t)g->vp * 4, ctx->stream));
-        CUDA_TRY(cudaMemcpyAsync(full + g->col_of_row0, d_in, (size_t)g->V * 4, cudaMemcpyDeviceToDevice, ctx->stream));
-        int rc = vglb_comm_allgather_async(g->comm, full, (size_t)g->vp * 4);
-        if (rc == VGLB_OK)
-        {
-            reorder_gather_kernel<<<(unsigned)ceil_div64(g->V_orig, 256), 256, 0, ctx->stream>>>(full, d_out, g->d_fwd, g->V_orig);
-            if (cudaGetLastError() != cudaSuccess) rc = VGLB_ECUDA;
-        }
-        cudaStreamSynchronize(ctx->stream);
-        vglb_dev_free(full);
+        dev_ptr<uint32_t> full;
+        CUDA_TRY(vglb_dev_alloc(full, (size_t)g->cols * 4));
+        CUDA_TRY(cudaMemsetAsync(full.get() + g->col_of_row0, 0, (size_t)g->vp * 4, ctx->stream));
+        CUDA_TRY(cudaMemcpyAsync(full.get() + g->col_of_row0, d_in, (size_t)g->V * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+        VGLB_TRY(vglb_comm_allgather_async(g->comm, full.get(), (size_t)g->vp * 4));
+        reorder_gather_kernel<<<(unsigned)ceil_div64(g->V_orig, 256), 256, 0, ctx->stream>>>(full.get(), d_out, g->d_fwd, g->V_orig);
+        KERNEL_TRY();
+        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
         ctx->launches++;
-        return rc;
+        return VGLB_OK;
     }
     const int32_t *index = to_orig ? g->d_fwd : g->d_bwd; // out[orig] = in[fwd[orig]] / out[sorted] = in[bwd[sorted]]
     reorder_gather_kernel<<<(unsigned)ceil_div64(g->V, 256), 256, 0, ctx->stream>>>(d_in, d_out, index, g->V);

@@ -167,46 +167,30 @@ extern "C" int vglb_graph_save_vgl(vglb_ctx *ctx, const char *path, int32_t vert
     }
     // outgoing container
     vglb_graph *g_out = NULL;
-    int rc = vglb_graph_from_edges(ctx, vertices, edges, src, dst, src_on_device, VGLB_GRAPH_WITH_EDGE_ORDER, &g_out);
-    if (rc != VGLB_OK) return rc;
-    rc = save_container(ctx, F, g_out);
+    VGLB_TRY(vglb_graph_from_edges(ctx, vertices, edges, src, dst, src_on_device, VGLB_GRAPH_WITH_EDGE_ORDER, &g_out));
+    graph_ptr out_owner(g_out);
+    VGLB_TRY(save_container(ctx, F, g_out));
     // incoming container = import of the transposed edge list — in the order the OUTGOING import left the container in:
     // VectorCSRGraph::import sorts the EdgesContainer by the new source id and only renumbers the ids back afterwards
     // (vect_csr/import.hpp:299-326), so VGL_Graph::import (vgl_graph.hpp:57-68) hands the incoming import the edges in
     // outgoing-CSR order, and its edges_reorder_indexes refer to that order.
-    int32_t *d_s = NULL, *d_d = NULL;
-    if (rc == VGLB_OK && edges > 0)
+    dev_ptr<int32_t> d_s, d_d;
+    if (edges > 0)
     {
-        if (vglb_dev_alloc(&d_s, (size_t)edges * 4) != cudaSuccess || vglb_dev_alloc(&d_d, (size_t)edges * 4) != cudaSuccess)
-        {
-            cudaGetLastError();
-            vglb_set_error("vglb_graph_save_vgl: out of device memory");
-            rc = VGLB_ENOMEM;
-        }
-        else
-        {
-            csr_order_edges_kernel<<<ctx->sm_count * 16, 256, 0, ctx->stream>>>(g_out->d_out_ptr, g_out->d_out_adj, g_out->d_bwd, vertices, d_s, d_d);
-            if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(ctx->stream) != cudaSuccess)
-            {
-                vglb_set_error("vglb_graph_save_vgl: kernel failure");
-                rc = VGLB_ECUDA;
-            }
-        }
+        CUDA_TRY(vglb_dev_alloc(d_s, (size_t)edges * 4));
+        CUDA_TRY(vglb_dev_alloc(d_d, (size_t)edges * 4));
+        csr_order_edges_kernel<<<ctx->sm_count * 16, 256, 0, ctx->stream>>>(g_out->d_out_ptr, g_out->d_out_adj, g_out->d_bwd, vertices,
+                                                                            d_s.get(), d_d.get());
+        KERNEL_TRY();
     }
-    vglb_graph_free(ctx, g_out);
-    if (rc == VGLB_OK)
-    {
-        vglb_graph *g_in = NULL;
-        rc = vglb_graph_from_edges(ctx, vertices, edges, d_d, d_s, 1, VGLB_GRAPH_WITH_EDGE_ORDER, &g_in); // transposed
-        if (rc == VGLB_OK)
-        {
-            rc = save_container(ctx, F, g_in);
-            vglb_graph_free(ctx, g_in);
-        }
-    }
-    vglb_dev_free(d_s);
-    vglb_dev_free(d_d);
-    return rc;
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    out_owner.reset();
+    vglb_graph *g_in = NULL;
+    VGLB_TRY(vglb_graph_from_edges(ctx, vertices, edges, d_d.get(), d_s.get(), 1, VGLB_GRAPH_WITH_EDGE_ORDER, &g_in)); // transposed
+    graph_ptr in_owner(g_in);
+    VGLB_TRY(save_container(ctx, F, g_in));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    return VGLB_OK;
 }
 
 // VGL_Graph::load_from_binary_file + move_to_device (vgl_graph.hpp:133-161, vect_csr_graph.hpp:158-196)

@@ -671,20 +671,19 @@ static int pr_build_tail_copy(vglb_ctx *ctx, vglb_graph *g)
     const int32_t segments = (int32_t)ceil_div64(zero_first - tail_first, 32);
     g->pr_ve_segments = segments;
     CUDA_TRY(vglb_dev_alloc(&g->d_pr_ve_ptr, ((size_t)segments + 2) * 8));
-    int64_t *d_len = NULL;
-    CUDA_TRY(vglb_dev_alloc(&d_len, ((size_t)segments + 2) * 8));
-    pr_ve_seglen_kernel<<<(unsigned)ceil_div64(segments + 1, 256), 256, 0, ctx->stream>>>(g->d_out_ptr, tail_first, segments, d_len);
+    dev_ptr<int64_t> d_len;
+    dev_ptr<void> tmp;
+    CUDA_TRY(vglb_dev_alloc(d_len, ((size_t)segments + 2) * 8));
+    pr_ve_seglen_kernel<<<(unsigned)ceil_div64(segments + 1, 256), 256, 0, ctx->stream>>>(g->d_out_ptr, tail_first, segments, d_len.get());
     KERNEL_TRY();
-    size_t tmp_bytes = 0;
-    void *tmp = NULL;
-    CUDA_TRY(cub::DeviceScan::ExclusiveSum(NULL, tmp_bytes, d_len, g->d_pr_ve_ptr, segments + 1, ctx->stream));
-    CUDA_TRY(vglb_dev_alloc(&tmp, tmp_bytes ? tmp_bytes : 16));
-    CUDA_TRY(cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, d_len, g->d_pr_ve_ptr, segments + 1, ctx->stream));
+    CUDA_TRY(vglb_cub(tmp, [&](void *t, size_t &bytes) {
+        return cub::DeviceScan::ExclusiveSum(t, bytes, d_len.get(), g->d_pr_ve_ptr, segments + 1, ctx->stream);
+    }));
     int64_t total = 0;
     CUDA_TRY(cudaMemcpyAsync(&total, g->d_pr_ve_ptr + segments, 8, cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    vglb_dev_free(tmp);
-    vglb_dev_free(d_len);
+    tmp.reset();
+    d_len.reset();
     CUDA_TRY(vglb_dev_alloc(&g->d_pr_ve_adj, (size_t)(total > 0 ? total : 1) * 4));
     if (segments > 0)
     {
@@ -736,55 +735,49 @@ int vglb_pr_prepare(vglb_ctx *ctx, vglb_graph *g, int iters)
     lap("contribution vectors");
     if (!g->d_pr_inv && g->comm) // part uploaded by vglb_graph_from_csr_partitioned: count columns locally, allreduce(sum)
     {
-        int32_t *d_indeg = NULL;
-        CUDA_TRY(vglb_dev_alloc(&d_indeg, (size_t)g->cols * 4));
-        CUDA_TRY(cudaMemsetAsync(d_indeg, 0, (size_t)g->cols * 4, ctx->stream));
-        pr_part_indegree_kernel<<<ctx->sm_count * 16, 256, 0, ctx->stream>>>(g->d_out_ptr, g->d_out_adj, g->V, g->col_of_row0, d_indeg);
+        dev_ptr<int32_t> d_indeg;
+        CUDA_TRY(vglb_dev_alloc(d_indeg, (size_t)g->cols * 4));
+        CUDA_TRY(cudaMemsetAsync(d_indeg.get(), 0, (size_t)g->cols * 4, ctx->stream));
+        pr_part_indegree_kernel<<<ctx->sm_count * 16, 256, 0, ctx->stream>>>(g->d_out_ptr, g->d_out_adj, g->V, g->col_of_row0, d_indeg.get());
         KERNEL_TRY();
-        int rc = vglb_comm_allreduce_async(g->comm, d_indeg, (size_t)g->cols, VGLB_DT_I32, VGLB_OP_SUM);
-        if (rc != VGLB_OK) { vglb_dev_free(d_indeg); return rc; }
+        VGLB_TRY(vglb_comm_allreduce_async(g->comm, d_indeg.get(), (size_t)g->cols, VGLB_DT_I32, VGLB_OP_SUM));
         CUDA_TRY(vglb_dev_alloc(&g->d_pr_inv, (size_t)g->vp * 4));
         CUDA_TRY(cudaMemsetAsync(g->d_pr_inv, 0, (size_t)g->vp * 4, ctx->stream));
         if (g->V > 0)
         {
-            pr_inverse_degree_kernel<<<(unsigned)ceil_div64(g->V, 256), 256, 0, ctx->stream>>>(d_indeg + g->col_of_row0, g->V, g->d_pr_inv);
+            pr_inverse_degree_kernel<<<(unsigned)ceil_div64(g->V, 256), 256, 0, ctx->stream>>>(d_indeg.get() + g->col_of_row0, g->V, g->d_pr_inv);
             KERNEL_TRY();
         }
         ctx->launches += 2;
         CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-        vglb_dev_free(d_indeg);
     }
     if (!g->d_pr_inv) // (the partitioned build fills it from its degree pass)
     {
-        int32_t *d_indeg = NULL;
-        CUDA_TRY(vglb_dev_alloc(&d_indeg, (size_t)g->V * 4));
-        int rc = vglb_graph_indegree_noloops(ctx, g, d_indeg);
-        if (rc != VGLB_OK) { vglb_dev_free(d_indeg); return rc; }
+        dev_ptr<int32_t> d_indeg;
+        CUDA_TRY(vglb_dev_alloc(d_indeg, (size_t)g->V * 4));
+        VGLB_TRY(vglb_graph_indegree_noloops(ctx, g, d_indeg.get()));
         CUDA_TRY(vglb_dev_alloc(&g->d_pr_inv, (size_t)g->V * 4));
-        pr_inverse_degree_kernel<<<(unsigned)ceil_div64(g->V, 256), 256, 0, ctx->stream>>>(d_indeg, g->V, g->d_pr_inv);
+        pr_inverse_degree_kernel<<<(unsigned)ceil_div64(g->V, 256), 256, 0, ctx->stream>>>(d_indeg.get(), g->V, g->d_pr_inv);
         KERNEL_TRY();
         ctx->launches++;
         CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-        vglb_dev_free(d_indeg);
     }
     lap("inverse in-degrees");
     if (vglb_pr_bins_wanted(g) && !g->pr_bins_tried)
     {
         g->pr_bins_tried = 1;
-        int rc = vglb_pr_bins_build(ctx, g);
-        if (rc != VGLB_OK && rc != VGLB_ENOMEM) return rc; // (out of memory for the binned copy, +0.9 GB at scale 24: warp tasks instead)
+        const int rc = vglb_pr_bins_build(ctx, g);
+        if (rc != VGLB_ENOMEM) VGLB_TRY(rc); // (out of memory for the binned copy, +0.9 GB at scale 24: warp tasks instead)
         lap("column bins of the heavy rows");
     }
     if (!g->d_pr_piece_count && !g->pr_bins)
     {
-        int rc = pr_build_tasks(ctx, g);
-        if (rc != VGLB_OK) return rc;
+        VGLB_TRY(pr_build_tasks(ctx, g));
         lap("warp tasks of the heavy rows");
     }
     if (!g->d_pr_ve_ptr)
     {
-        int rc = pr_build_tail_copy(ctx, g);
-        if (rc != VGLB_OK) return rc;
+        VGLB_TRY(pr_build_tail_copy(ctx, g));
         lap("padded copy of the tail rows");
     }
     if (!g->comm)
@@ -797,19 +790,20 @@ int vglb_pr_prepare(vglb_ctx *ctx, vglb_graph *g, int iters)
             g->V, zero_first + ceil_div64(std::max<int64_t>(0, smem_cols - zero_first), PR_ZERO_ROWS_PER_CTA) * PR_ZERO_ROWS_PER_CTA);
         if (!g->pr_zero_ready || g->pr_zero_kept != kept)
         {
-            unsigned long long *d_n = NULL, n = 0;
-            CUDA_TRY(vglb_dev_alloc(&d_n, sizeof(*d_n)));
-            CUDA_TRY(cudaMemsetAsync(d_n, 0, sizeof(*d_n), ctx->stream));
+            dev_ptr<unsigned long long> d_n;
+            unsigned long long n = 0;
+            CUDA_TRY(vglb_dev_alloc(d_n, sizeof(n)));
+            CUDA_TRY(cudaMemsetAsync(d_n.get(), 0, sizeof(n), ctx->stream));
             if (kept < g->V)
             {
                 pr_count_no_inv_kernel<<<(unsigned)std::min<int64_t>(ctx->sm_count * 8, ceil_div64(g->V - kept, 256)), 256, 0, ctx->stream>>>(
-                    g->d_pr_inv, kept, g->V, d_n);
+                    g->d_pr_inv, kept, g->V, d_n.get());
                 KERNEL_TRY();
                 ctx->launches++;
             }
-            CUDA_TRY(cudaMemcpyAsync(&n, d_n, sizeof(n), cudaMemcpyDeviceToHost, ctx->stream));
+            CUDA_TRY(cudaMemcpyAsync(&n, d_n.get(), sizeof(n), cudaMemcpyDeviceToHost, ctx->stream));
             CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-            vglb_dev_free(d_n);
+            d_n.reset();
             g->pr_zero_kept = kept;
             g->pr_zero_dangling = (int32_t)n;
             g->pr_zero_ready = 1;
@@ -926,8 +920,7 @@ extern "C" int vglb_pagerank_ex(vglb_ctx *ctx, vglb_graph *g, int iters, float d
     VGLB_REQUIRE(!ref_order || !g->comm, "vglb_pagerank_ex: the reference-order dangling sum needs the whole sorted id range (one GPU)");
     CUDA_TRY(cudaSetDevice(ctx->device));
     const int64_t launches0 = ctx->launches;
-    int rc = vglb_pr_prepare(ctx, g, iters);
-    if (rc != VGLB_OK) return rc;
+    VGLB_TRY(vglb_pr_prepare(ctx, g, iters));
 
     // On a partitioned graph (g->comm): V = this rank's rows, the vector is indexed by column id, and after every sweep
     // the owned slices are allgathered (exchange_vertices_array, mpi_exchange.hpp:155-271) and the dangling mass
@@ -974,27 +967,25 @@ extern "C" int vglb_pagerank_ex(vglb_ctx *ctx, vglb_graph *g, int iters, float d
         if (!comm) return VGLB_OK;
         if (!stored_by_peers)
         {
-            int rc = vglb_comm_allgather_async(comm, vec, (size_t)g->vp * 4);
-            if (rc != VGLB_OK) return rc;
+            VGLB_TRY(vglb_comm_allgather_async(comm, vec, (size_t)g->vp * 4));
         }
         return vglb_comm_allreduce_async(comm, dangling, 1, VGLB_DT_F64, VGLB_OP_SUM);
     };
 
-    float *d_ref_partial = NULL;
-    if (ref_order) CUDA_TRY(vglb_dev_alloc(&d_ref_partial, (size_t)ref_threads * sizeof(float)));
+    dev_ptr<float> d_ref_partial;
+    if (ref_order) CUDA_TRY(vglb_dev_alloc(d_ref_partial, (size_t)ref_threads * sizeof(float)));
     // dangling mass of the rank vector in d_ranks, summed in the reference's order, into dangling slot `slot`
     auto reference_dangling = [&](int slot) -> int {
         pr_dangling_reference_chunks_kernel<<<(unsigned)ceil_div64((int64_t)ref_threads * 32, 256), 256, 0, ctx->stream>>>(
-            d_ranks, g->d_pr_inv, V, P.v_as_float, ref_threads, d_ref_partial);
+            d_ranks, g->d_pr_inv, V, P.v_as_float, ref_threads, d_ref_partial.get());
         KERNEL_TRY();
-        pr_dangling_reference_combine_kernel<<<1, 1, 0, ctx->stream>>>(d_ref_partial, ref_threads, g->d_pr_dangling + slot);
+        pr_dangling_reference_combine_kernel<<<1, 1, 0, ctx->stream>>>(d_ref_partial.get(), ref_threads, g->d_pr_dangling + slot);
         KERNEL_TRY();
         ctx->launches += 2;
         return VGLB_OK;
     };
 
-    rc = pr_set_carveouts(ctx);
-    if (rc != VGLB_OK) return rc;
+    VGLB_TRY(pr_set_carveouts(ctx));
     CUDA_TRY(cudaEventRecord(ctx->ev_start, ctx->stream));
     CUDA_TRY(cudaMemsetAsync(g->d_pr_dangling, 0, (size_t)(iters + 1) * sizeof(double), ctx->stream));
     const float r0 = (float)(1.0 / (double)g->V_orig); // pr.hpp:42
@@ -1014,15 +1005,13 @@ extern "C" int vglb_pagerank_ex(vglb_ctx *ctx, vglb_graph *g, int iters, float d
                                                                         g->d_pr_contrib[0] + col0, g->d_pr_dangling);
         KERNEL_TRY();
         ctx->launches++;
-        rc = exchange(g->d_pr_contrib[0], g->d_pr_dangling, false);
-        if (rc != VGLB_OK) return rc;
+        VGLB_TRY(exchange(g->d_pr_contrib[0], g->d_pr_dangling, false));
         if (ref_order && V > 0)
         {
             pr_fill_kernel<<<(unsigned)ceil_div64(V, 256), 256, 0, ctx->stream>>>(d_ranks, V, r0);
             KERNEL_TRY();
             ctx->launches++;
-            rc = reference_dangling(0); // replaces the fp64 sum pr_init_kernel left in slot 0
-            if (rc != VGLB_OK) return rc;
+            VGLB_TRY(reference_dangling(0)); // replaces the fp64 sum pr_init_kernel left in slot 0
         }
     }
     for (int it = 0; it < iters; it++)
@@ -1039,8 +1028,7 @@ extern "C" int vglb_pagerank_ex(vglb_ctx *ctx, vglb_graph *g, int iters, float d
                 if (p != g->part_rank) P.peer_out[P.npeers++] = g->d_pr_peer[(it + 1) & 1][p] + col0;
         if (g->pr_bins)
         {
-            rc = vglb_pr_bins_launch(ctx, g, P.contrib_in); // partial sums of the heavy rows: the shared-memory bins
-            if (rc != VGLB_OK) return rc;
+            VGLB_TRY(vglb_pr_bins_launch(ctx, g, P.contrib_in)); // partial sums of the heavy rows: the shared-memory bins
             P.bins.contrib_in = P.contrib_in;
         }
         if (g->pr_bins && P.bin_cold_blocks > 0)
@@ -1050,24 +1038,20 @@ extern "C" int vglb_pagerank_ex(vglb_ctx *ctx, vglb_graph *g, int iters, float d
             ctx->launches++;
         }
         // the heavy rows' sums (all rows without the bins), the rows with < 32 edges and the rows without out-edges
-        rc = vglb_pr_launch_sweep(ctx, P, P.rank_out ? nblocks : nblocks_lean);
-        if (rc != VGLB_OK) return rc;
+        VGLB_TRY(vglb_pr_launch_sweep(ctx, P, P.rank_out ? nblocks : nblocks_lean));
         if (ref_order && it < iters - 1)
         {
-            rc = reference_dangling(it + 1); // replaces the fp64 sum the sweep's epilogue accumulated
-            if (rc != VGLB_OK) return rc;
+            VGLB_TRY(reference_dangling(it + 1)); // replaces the fp64 sum the sweep's epilogue accumulated
         }
         if (it < iters - 1 || p2p)
         {
             // (with peer stores the last sweep still ends in the allreduce: no rank may start its NEXT run — which
             // rewrites buffer 0 everywhere — before every peer has finished reading)
-            rc = exchange(g->d_pr_contrib[(it + 1) & 1], g->d_pr_dangling + it + 1, p2p);
-            if (rc != VGLB_OK) return rc;
+            VGLB_TRY(exchange(g->d_pr_contrib[(it + 1) & 1], g->d_pr_dangling + it + 1, p2p));
         }
     }
-    rc = vglb_finish_run(ctx, launches0, stats);
-    if (rc != VGLB_OK) return rc;
-    vglb_dev_free(d_ref_partial);
+    VGLB_TRY(vglb_finish_run(ctx, launches0, stats));
+    d_ref_partial.reset();
     if (!stats) return VGLB_OK;
     stats->iterations = iters;
     stats->edges_inspected = (int64_t)iters * g->E;

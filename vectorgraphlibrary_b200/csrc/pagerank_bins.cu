@@ -281,61 +281,29 @@ __global__ void prb_fill_u16_kernel(uint16_t *a, int64_t n, uint16_t val)
     }
 }
 
+// frees a PrBins and its arrays (the owner of one that is still being built, and vglb_pr_bins_free)
+struct prb_deleter
+{
+    void operator()(PrBins *B) const
+    {
+        vglb_dev_free(B->d_wcol);
+        vglb_dev_free(B->d_cold);
+        vglb_dev_free(B->d_meta);
+        vglb_dev_free(B->d_step_run0);
+        vglb_dev_free(B->d_run_slot);
+        vglb_dev_free(B->d_bin_chunk0);
+        vglb_dev_free(B->d_cta_chunk0);
+        vglb_dev_free(B->d_slot);
+        vglb_dev_free(B->d_rc_ptr);
+        free(B);
+    }
+};
+
 void vglb_pr_bins_free(vglb_graph *g)
 {
-    PrBins *B = (PrBins *)g->pr_bins;
-    if (!B) return;
-    vglb_dev_free(B->d_wcol);
-    vglb_dev_free(B->d_cold);
-    vglb_dev_free(B->d_meta);
-    vglb_dev_free(B->d_step_run0);
-    vglb_dev_free(B->d_run_slot);
-    vglb_dev_free(B->d_bin_chunk0);
-    vglb_dev_free(B->d_cta_chunk0);
-    vglb_dev_free(B->d_slot);
-    vglb_dev_free(B->d_rc_ptr);
-    free(B);
+    if (g->pr_bins) prb_deleter()((PrBins *)g->pr_bins);
     g->pr_bins = NULL;
 }
-
-template <class T>
-static int prb_exclusive_sum(vglb_ctx *ctx, const T *in, T *out, int64_t n, bool inclusive = false)
-{
-    size_t bytes = 0;
-    void *tmp = NULL;
-    if (inclusive) CUDA_TRY(cub::DeviceScan::InclusiveSum(NULL, bytes, in, out, n, ctx->stream));
-    else CUDA_TRY(cub::DeviceScan::ExclusiveSum(NULL, bytes, in, out, n, ctx->stream));
-    CUDA_TRY(vglb_dev_alloc(&tmp, bytes ? bytes : 16));
-    cudaError_t e = inclusive ? cub::DeviceScan::InclusiveSum(tmp, bytes, in, out, n, ctx->stream)
-                              : cub::DeviceScan::ExclusiveSum(tmp, bytes, in, out, n, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream); // (tmp goes back to the cache only after the scan ran)
-    vglb_dev_free(tmp);
-    CUDA_TRY(e);
-    return VGLB_OK;
-}
-
-#define PRB_TRY(call)            \
-    do                           \
-    {                            \
-        int rc_ = (call);        \
-        if (rc_ != VGLB_OK)      \
-        {                        \
-            cleanup();           \
-            return rc_;          \
-        }                        \
-    } while (0)
-#define PRB_CUDA(call)                                                                                        \
-    do                                                                                                        \
-    {                                                                                                         \
-        cudaError_t e_ = (call);                                                                              \
-        if (e_ != cudaSuccess)                                                                                \
-        {                                                                                                     \
-            cudaGetLastError();                                                                               \
-            vglb_set_error("%s failed at %s:%d: %s", #call, __FILE__, __LINE__, cudaGetErrorString(e_));      \
-            cleanup();                                                                                        \
-            return e_ == cudaErrorMemoryAllocation ? VGLB_ENOMEM : VGLB_ECUDA;                                \
-        }                                                                                                     \
-    } while (0)
 
 // Builds the binned copy of the heavy rows (degree >= 32) of a one-GPU graph. Leaves g->pr_bins NULL when there is nothing to
 // bin (no heavy rows).
@@ -349,65 +317,62 @@ int vglb_pr_bins_build_rows(vglb_ctx *ctx, vglb_graph *g, int32_t rows)
     const int64_t ncols = g->comm ? g->cols : (int64_t)g->V;
     cudaStream_t st = ctx->stream;
     int32_t long_rows = 0;
-    int rc = vglb_graph_threshold_vertex(ctx, g, PRB_RC + 1, &long_rows); // rows with more than one chunk
-    if (rc != VGLB_OK) return rc;
+    VGLB_TRY(vglb_graph_threshold_vertex(ctx, g, PRB_RC + 1, &long_rows)); // rows with more than one chunk
     // 32 bins = the hottest 9.4 % of the columns of the BASELINE graph = 91 % of the gathers of its heavy rows. Every further bin
     // costs the finish pass one more partial sum per heavy row: 64 bins are no faster there, and on 4 GPUs (scale 26: 32 bins hold
     // 74 % of the gathers) 32 / 64 / 128 bins gave 1034 / 1075 / 939 GTEPS against 1108 with the warp tasks.
     const int nb = (int)std::min<int64_t>(PRB_BINS, ceil_div64(ncols, PRB_H));
     const int nc = nb + 1;
 
-    PrBins *B = (PrBins *)calloc(1, sizeof(PrBins));
-    VGLB_REQUIRE(B != NULL, "vglb_pr_bins_build: out of host memory");
-    int32_t *d_nchunks = NULL, *d_rc_full = NULL, *d_cnt = NULL, *d_pflag = NULL, *d_flag_scan = NULL, *d_step_total = NULL;
-    int64_t *d_plen = NULL, *d_pos_scan = NULL, *d_bin_start = NULL, *d_out = NULL, *d_run_pos = NULL, *d_cost = NULL;
-    auto free_scratch = [&]() {
-        vglb_dev_free(d_nchunks); vglb_dev_free(d_rc_full); vglb_dev_free(d_cnt); vglb_dev_free(d_pflag); vglb_dev_free(d_flag_scan);
-        vglb_dev_free(d_step_total); vglb_dev_free(d_plen); vglb_dev_free(d_pos_scan); vglb_dev_free(d_bin_start); vglb_dev_free(d_out);
-        vglb_dev_free(d_run_pos); vglb_dev_free(d_cost);
-    };
-    auto cleanup = [&]() { // error path
-        free_scratch();
-        g->pr_bins = B;
-        vglb_pr_bins_free(g);
-    };
+    std::unique_ptr<PrBins, prb_deleter> owner((PrBins *)calloc(1, sizeof(PrBins)));
+    VGLB_REQUIRE(owner != NULL, "vglb_pr_bins_build: out of host memory");
+    PrBins *B = owner.get();
+    dev_ptr<int32_t> d_nchunks, d_rc_full, d_cnt, d_pflag, d_flag_scan, d_step_total;
+    dev_ptr<int64_t> d_plen, d_pos_scan, d_bin_start, d_out, d_run_pos, d_cost;
+    dev_ptr<void> tmp; // CUB temporaries, each freed where its scan has finished
     // row chunks
-    PRB_CUDA(vglb_dev_alloc(&d_nchunks, ((size_t)rows + 1) * 4));
-    PRB_CUDA(vglb_dev_alloc(&d_rc_full, ((size_t)rows + 1) * 4));
-    prb_row_chunks_kernel<<<(unsigned)ceil_div64(rows + 1, 256), 256, 0, st>>>(g->d_out_ptr, rows, d_nchunks);
-    PRB_CUDA(cudaGetLastError());
-    PRB_TRY(prb_exclusive_sum(ctx, d_nchunks, d_rc_full, (int64_t)rows + 1));
+    CUDA_TRY(vglb_dev_alloc(d_nchunks, ((size_t)rows + 1) * 4));
+    CUDA_TRY(vglb_dev_alloc(d_rc_full, ((size_t)rows + 1) * 4));
+    prb_row_chunks_kernel<<<(unsigned)ceil_div64(rows + 1, 256), 256, 0, st>>>(g->d_out_ptr, rows, d_nchunks.get());
+    KERNEL_TRY();
+    CUDA_TRY(vglb_cub(tmp, [&](void *t, size_t &bytes) { return cub::DeviceScan::ExclusiveSum(t, bytes, (const int32_t *)d_nchunks.get(), d_rc_full.get(), (int64_t)rows + 1, st); }));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    tmp.reset();
     int32_t nch = 0;
-    PRB_CUDA(cudaMemcpyAsync(&nch, d_rc_full + rows, 4, cudaMemcpyDeviceToHost, st));
-    PRB_CUDA(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaMemcpyAsync(&nch, d_rc_full.get() + rows, 4, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
     const int32_t xc = nch - rows; // chunks beyond one per row; all of them belong to the first long_rows rows
-    PRB_CUDA(vglb_dev_alloc(&B->d_rc_ptr, ((size_t)long_rows + 1) * 4));
-    PRB_CUDA(cudaMemcpyAsync(B->d_rc_ptr, d_rc_full, ((size_t)long_rows + 1) * 4, cudaMemcpyDeviceToDevice, st));
+    CUDA_TRY(vglb_dev_alloc(&B->d_rc_ptr, ((size_t)long_rows + 1) * 4));
+    CUDA_TRY(cudaMemcpyAsync(B->d_rc_ptr, d_rc_full.get(), ((size_t)long_rows + 1) * 4, cudaMemcpyDeviceToDevice, st));
     const int64_t n = (int64_t)nc * nch;
-    if (n >= 0x7fffffffLL) { cleanup(); vglb_set_error("vglb_pr_bins_build: too many runs"); return VGLB_EINVAL; }
+    if (n >= 0x7fffffffLL) { vglb_set_error("vglb_pr_bins_build: too many runs"); return VGLB_EINVAL; }
     // counts per (class, row chunk), scans, layout
-    PRB_CUDA(vglb_dev_alloc(&d_cnt, (size_t)n * 4));
+    CUDA_TRY(vglb_dev_alloc(d_cnt, (size_t)n * 4));
     prb_scatter_kernel<false><<<(unsigned)ceil_div64(nch, 8), 256, 0, st>>>(g->d_out_ptr, g->d_out_adj, B->d_rc_ptr, long_rows, xc, nch, nb,
-                                                                           g->col_of_row0, world, (uint32_t)g->vp, d_cnt, NULL, 0, NULL, NULL);
-    PRB_CUDA(cudaGetLastError());
-    PRB_CUDA(vglb_dev_alloc(&d_plen, ((size_t)n + 1) * 8));
-    PRB_CUDA(vglb_dev_alloc(&d_pflag, ((size_t)n + 1) * 4));
-    PRB_CUDA(vglb_dev_alloc(&d_pos_scan, ((size_t)n + 1) * 8));
-    PRB_CUDA(vglb_dev_alloc(&d_flag_scan, ((size_t)n + 1) * 4));
-    prb_lengths_kernel<<<(unsigned)ceil_div64(n + 1, 256), 256, 0, st>>>(d_cnt, n, d_plen, d_pflag);
-    PRB_CUDA(cudaGetLastError());
-    PRB_TRY(prb_exclusive_sum(ctx, d_plen, d_pos_scan, n + 1));
-    PRB_TRY(prb_exclusive_sum(ctx, d_pflag, d_flag_scan, n + 1));
-    PRB_CUDA(vglb_dev_alloc(&d_bin_start, ((size_t)nc + 1) * 8));
-    PRB_CUDA(vglb_dev_alloc(&B->d_bin_chunk0, ((size_t)nc + 1) * 4));
-    PRB_CUDA(vglb_dev_alloc(&d_out, 3 * 8));
-    prb_bins_kernel<<<1, 1, 0, st>>>(d_pos_scan, d_flag_scan, nch, nc, d_bin_start, B->d_bin_chunk0, d_out);
-    PRB_CUDA(cudaGetLastError());
+                                                                           g->col_of_row0, world, (uint32_t)g->vp, d_cnt.get(), NULL, 0, NULL, NULL);
+    KERNEL_TRY();
+    CUDA_TRY(vglb_dev_alloc(d_plen, ((size_t)n + 1) * 8));
+    CUDA_TRY(vglb_dev_alloc(d_pflag, ((size_t)n + 1) * 4));
+    CUDA_TRY(vglb_dev_alloc(d_pos_scan, ((size_t)n + 1) * 8));
+    CUDA_TRY(vglb_dev_alloc(d_flag_scan, ((size_t)n + 1) * 4));
+    prb_lengths_kernel<<<(unsigned)ceil_div64(n + 1, 256), 256, 0, st>>>(d_cnt.get(), n, d_plen.get(), d_pflag.get());
+    KERNEL_TRY();
+    CUDA_TRY(vglb_cub(tmp, [&](void *t, size_t &bytes) { return cub::DeviceScan::ExclusiveSum(t, bytes, (const int64_t *)d_plen.get(), d_pos_scan.get(), n + 1, st); }));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    tmp.reset();
+    CUDA_TRY(vglb_cub(tmp, [&](void *t, size_t &bytes) { return cub::DeviceScan::ExclusiveSum(t, bytes, (const int32_t *)d_pflag.get(), d_flag_scan.get(), n + 1, st); }));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    tmp.reset();
+    CUDA_TRY(vglb_dev_alloc(d_bin_start, ((size_t)nc + 1) * 8));
+    CUDA_TRY(vglb_dev_alloc(&B->d_bin_chunk0, ((size_t)nc + 1) * 4));
+    CUDA_TRY(vglb_dev_alloc(d_out, 3 * 8));
+    prb_bins_kernel<<<1, 1, 0, st>>>(d_pos_scan.get(), d_flag_scan.get(), nch, nc, d_bin_start.get(), B->d_bin_chunk0, d_out.get());
+    KERNEL_TRY();
     int64_t h_out[3];
-    PRB_CUDA(cudaMemcpyAsync(h_out, d_out, sizeof(h_out), cudaMemcpyDeviceToHost, st));
-    PRB_CUDA(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaMemcpyAsync(h_out, d_out.get(), sizeof(h_out), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
     const int64_t W = h_out[0], w_smem = h_out[1], nruns = h_out[2], nsteps = W / PRB_STEP;
-    if (W / PRB_CHUNK >= 0x7fffffffLL || nruns >= 0x7fffffffLL) { cleanup(); vglb_set_error("vglb_pr_bins_build: graph too large for 32-bit chunk / run numbers"); return VGLB_EINVAL; }
+    if (W / PRB_CHUNK >= 0x7fffffffLL || nruns >= 0x7fffffffLL) { vglb_set_error("vglb_pr_bins_build: graph too large for 32-bit chunk / run numbers"); return VGLB_EINVAL; }
     B->nb = nb;
     B->rows = rows;
     B->long_rows = long_rows;
@@ -419,52 +384,55 @@ int vglb_pr_bins_build_rows(vglb_ctx *ctx, vglb_graph *g, int32_t rows)
     B->nruns = (int32_t)nruns;
     B->grid = ctx->sm_count;
     // the arrays the sweep reads
-    PRB_CUDA(vglb_dev_alloc(&B->d_wcol, (size_t)(w_smem > 0 ? w_smem : 8) * 2));
-    PRB_CUDA(vglb_dev_alloc(&B->d_cold, (size_t)(W - w_smem) * 4));
-    PRB_CUDA(vglb_dev_alloc(&B->d_meta, (size_t)nsteps * 32 * 4));
-    PRB_CUDA(vglb_dev_alloc(&B->d_step_run0, ((size_t)nsteps + 1) * 4));
-    PRB_CUDA(vglb_dev_alloc(&B->d_run_slot, (size_t)nruns * 4));
-    PRB_CUDA(vglb_dev_alloc(&B->d_slot, ((size_t)n + 1) * 4));
-    PRB_CUDA(vglb_dev_alloc(&B->d_cta_chunk0, ((size_t)B->grid + 1) * 4));
-    PRB_CUDA(cudaMemsetAsync(B->d_slot, 0, ((size_t)n + 1) * 4, st));
-    PRB_CUDA(cudaMemsetAsync(B->d_meta, 0, (size_t)nsteps * 32 * 4, st));
-    PRB_CUDA(cudaMemsetAsync(B->d_cold, 0xFF, (size_t)(W - w_smem) * 4, st));
+    CUDA_TRY(vglb_dev_alloc(&B->d_wcol, (size_t)(w_smem > 0 ? w_smem : 8) * 2));
+    CUDA_TRY(vglb_dev_alloc(&B->d_cold, (size_t)(W - w_smem) * 4));
+    CUDA_TRY(vglb_dev_alloc(&B->d_meta, (size_t)nsteps * 32 * 4));
+    CUDA_TRY(vglb_dev_alloc(&B->d_step_run0, ((size_t)nsteps + 1) * 4));
+    CUDA_TRY(vglb_dev_alloc(&B->d_run_slot, (size_t)nruns * 4));
+    CUDA_TRY(vglb_dev_alloc(&B->d_slot, ((size_t)n + 1) * 4));
+    CUDA_TRY(vglb_dev_alloc(&B->d_cta_chunk0, ((size_t)B->grid + 1) * 4));
+    CUDA_TRY(cudaMemsetAsync(B->d_slot, 0, ((size_t)n + 1) * 4, st));
+    CUDA_TRY(cudaMemsetAsync(B->d_meta, 0, (size_t)nsteps * 32 * 4, st));
+    CUDA_TRY(cudaMemsetAsync(B->d_cold, 0xFF, (size_t)(W - w_smem) * 4, st));
     if (w_smem > 0)
     {
         prb_fill_u16_kernel<<<(unsigned)ceil_div64(w_smem / 8, 256), 256, 0, st>>>(B->d_wcol, w_smem, (uint16_t)PRB_H);
-        PRB_CUDA(cudaGetLastError());
+        KERNEL_TRY();
     }
     // edges to their slots
-    PRB_CUDA(vglb_dev_alloc(&d_run_pos, (size_t)n * 8));
-    prb_run_pos_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, st>>>(d_pos_scan, d_bin_start, nch, nc, d_run_pos);
-    PRB_CUDA(cudaGetLastError());
+    CUDA_TRY(vglb_dev_alloc(d_run_pos, (size_t)n * 8));
+    prb_run_pos_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, st>>>(d_pos_scan.get(), d_bin_start.get(), nch, nc, d_run_pos.get());
+    KERNEL_TRY();
     prb_scatter_kernel<true><<<(unsigned)ceil_div64(nch, 8), 256, 0, st>>>(g->d_out_ptr, g->d_out_adj, B->d_rc_ptr, long_rows, xc, nch, nb,
-                                                                          g->col_of_row0, world, (uint32_t)g->vp, NULL, d_run_pos, w_smem, B->d_wcol,
+                                                                          g->col_of_row0, world, (uint32_t)g->vp, NULL, d_run_pos.get(), w_smem, B->d_wcol,
                                                                           B->d_cold);
-    PRB_CUDA(cudaGetLastError());
+    KERNEL_TRY();
     // run starts, slots, per-lane metadata, run numbers of the steps
-    prb_runs_kernel<<<(unsigned)ceil_div64(n + nc, 256), 256, 0, st>>>(d_cnt, d_run_pos, d_pos_scan, d_flag_scan, d_bin_start, nch, nc,
+    prb_runs_kernel<<<(unsigned)ceil_div64(n + nc, 256), 256, 0, st>>>(d_cnt.get(), d_run_pos.get(), d_pos_scan.get(), d_flag_scan.get(), d_bin_start.get(), nch, nc,
                                                                       B->d_meta, B->d_run_slot);
-    PRB_CUDA(cudaGetLastError());
-    PRB_CUDA(vglb_dev_alloc(&d_step_total, ((size_t)nsteps + 1) * 4));
-    prb_meta_kernel<<<(unsigned)ceil_div64(nsteps * 32, 256), 256, 0, st>>>(B->d_meta, nsteps, d_step_total);
-    PRB_CUDA(cudaGetLastError());
-    PRB_TRY(prb_exclusive_sum(ctx, d_step_total, B->d_step_run0, nsteps + 1));
+    KERNEL_TRY();
+    CUDA_TRY(vglb_dev_alloc(d_step_total, ((size_t)nsteps + 1) * 4));
+    prb_meta_kernel<<<(unsigned)ceil_div64(nsteps * 32, 256), 256, 0, st>>>(B->d_meta, nsteps, d_step_total.get());
+    KERNEL_TRY();
+    CUDA_TRY(vglb_cub(tmp, [&](void *t, size_t &bytes) { return cub::DeviceScan::ExclusiveSum(t, bytes, (const int32_t *)d_step_total.get(), B->d_step_run0, nsteps + 1, st); }));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    tmp.reset();
     // cost-balanced chunk ranges of the persistent CTAs
     // (the cold bin's chunks are blocks of pr_sweep_kernel)
     if (B->cold_chunk0 > 0)
     {
-        PRB_CUDA(vglb_dev_alloc(&d_cost, (size_t)B->cold_chunk0 * 8));
-        prb_cost_kernel<<<(unsigned)ceil_div64(B->cold_chunk0, 256), 256, 0, st>>>(B->d_step_run0, B->cold_chunk0, d_cost);
-        PRB_CUDA(cudaGetLastError());
-        PRB_TRY(prb_exclusive_sum(ctx, d_cost, d_cost, B->cold_chunk0, true));
+        CUDA_TRY(vglb_dev_alloc(d_cost, (size_t)B->cold_chunk0 * 8));
+        prb_cost_kernel<<<(unsigned)ceil_div64(B->cold_chunk0, 256), 256, 0, st>>>(B->d_step_run0, B->cold_chunk0, d_cost.get());
+        KERNEL_TRY();
+        CUDA_TRY(vglb_cub(tmp, [&](void *t, size_t &bytes) { return cub::DeviceScan::InclusiveSum(t, bytes, (const int64_t *)d_cost.get(), d_cost.get(), (int64_t)B->cold_chunk0, st); }));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        tmp.reset();
     }
-    prb_cta_ranges_kernel<<<(unsigned)ceil_div64(B->grid + 1, 256), 256, 0, st>>>(d_cost, B->cold_chunk0, B->grid, B->d_cta_chunk0);
-    PRB_CUDA(cudaGetLastError());
-    PRB_CUDA(cudaStreamSynchronize(st));
+    prb_cta_ranges_kernel<<<(unsigned)ceil_div64(B->grid + 1, 256), 256, 0, st>>>(d_cost.get(), B->cold_chunk0, B->grid, B->d_cta_chunk0);
+    KERNEL_TRY();
+    CUDA_TRY(cudaStreamSynchronize(st));
     ctx->launches += 12;
-    free_scratch();
-    g->pr_bins = B;
+    g->pr_bins = owner.release();
     return VGLB_OK;
 }
 

@@ -409,17 +409,6 @@ __global__ void part_degree_kernel(const int32_t *__restrict__ src, const int32_
     }
 }
 
-__global__ void part_sort_keys_kernel(const int32_t *__restrict__ deg, int32_t V, uint32_t *__restrict__ keys,
-                                      uint32_t *__restrict__ ids)
-{
-    int32_t v = blockIdx.x * blockDim.x + threadIdx.x;
-    if (v < V)
-    {
-        keys[v] = ~(uint32_t)deg[v]; // stable ascending ~deg == the reference's stable descending-degree order
-        ids[v] = (uint32_t)v;
-    }
-}
-
 // sorted id s -> column (s mod P) * vp + s div P; also this rank's edge totals for both directions
 __global__ void part_numbering_kernel(const uint32_t *__restrict__ sorted_ids, int32_t V, int32_t P, int32_t vp, int32_t rank,
                                       const int32_t *__restrict__ deg_out, const int32_t *__restrict__ deg_in,
@@ -510,28 +499,7 @@ __global__ void part_pr_inverse_kernel(const int32_t *__restrict__ deg_in_noloop
     }
 }
 
-int bits_for64(int64_t n)
-{
-    int b = 1;
-    while (b < 32 && ((int64_t)1 << b) < n) b++;
-    return b;
-}
-
 } // namespace
-
-#define PBUILD_CUDA(call)                                                                                  \
-    do                                                                                                     \
-    {                                                                                                      \
-        cudaError_t err__ = (call);                                                                        \
-        if (err__ != cudaSuccess)                                                                          \
-        {                                                                                                  \
-            vglb_set_error("CUDA error %s at %s:%d (%s)", cudaGetErrorString(err__), __FILE__, __LINE__,   \
-                           #call);                                                                         \
-            cudaGetLastError();                                                                            \
-            cleanup();                                                                                     \
-            return err__ == cudaErrorMemoryAllocation ? VGLB_ENOMEM : VGLB_ECUDA;                          \
-        }                                                                                                  \
-    } while (0)
 
 static const int64_t kChunkEdges = (int64_t)1 << 26;
 
@@ -579,83 +547,63 @@ static int build_partitioned(vglb_ctx *ctx, vglb_comm *comm, int32_t V, const Ed
     const int32_t rows = V > rank ? (V - rank + P - 1) / P : 0; // sorted ids rank, rank + P, ...
     const int halves = symmetrize ? 2 : 1;
 
-    vglb_graph *g = (vglb_graph *)calloc(1, sizeof(vglb_graph));
-    if (!g) return VGLB_ENOMEM;
-    int32_t *buf_a = NULL, *buf_b = NULL, *d_deg_out = NULL, *d_deg_in = NULL, *d_deg_nl = NULL;
-    uint32_t *k0 = NULL, *k1 = NULL, *v0 = NULL, *v1 = NULL;
-    uint64_t *keys0 = NULL, *keys1 = NULL;
-    unsigned long long *d_rowcnt = NULL, *d_misc = NULL;
-    void *tmp = NULL;
-    int *d_bad = NULL;
-    auto cleanup = [&]() {
-        vglb_dev_free(buf_a); vglb_dev_free(buf_b); vglb_dev_free(d_deg_out); vglb_dev_free(d_deg_in); vglb_dev_free(d_deg_nl); vglb_dev_free(k0);
-        vglb_dev_free(k1); vglb_dev_free(v0); vglb_dev_free(v1); vglb_dev_free(keys0); vglb_dev_free(keys1); vglb_dev_free(d_rowcnt); vglb_dev_free(d_misc);
-        vglb_dev_free(tmp); vglb_dev_free(d_bad);
-        if (g) { vglb_graph_free_fields(g); free(g); }
-    };
+    graph_ptr owner = vglb_graph_new();
+    if (!owner) return VGLB_ENOMEM;
+    vglb_graph *g = owner.get();
+    dev_ptr<int32_t> buf_a, buf_b, d_deg_out, d_deg_in, d_deg_nl;
+    dev_ptr<unsigned long long> d_rowcnt, d_misc;
+    dev_ptr<int> d_bad;
     const int grid = ctx->sm_count * 16;
     cudaStream_t st = ctx->stream;
     const int64_t chunk = S.edges < kChunkEdges ? (S.edges > 0 ? S.edges : 1) : kChunkEdges;
     if (S.mode != 1)
     {
-        PBUILD_CUDA(vglb_dev_alloc(&buf_a, (size_t)chunk * 4));
-        PBUILD_CUDA(vglb_dev_alloc(&buf_b, (size_t)chunk * 4));
+        CUDA_TRY(vglb_dev_alloc(buf_a, (size_t)chunk * 4));
+        CUDA_TRY(vglb_dev_alloc(buf_b, (size_t)chunk * 4));
     }
     // pass 1: degrees of every vertex (identical on every rank)
-    PBUILD_CUDA(vglb_dev_alloc(&d_deg_out, (size_t)V * 4));
-    PBUILD_CUDA(vglb_dev_alloc(&d_deg_in, (size_t)V * 4));
-    PBUILD_CUDA(vglb_dev_alloc(&d_deg_nl, (size_t)V * 4));
-    PBUILD_CUDA(vglb_dev_alloc(&d_bad, 4));
-    PBUILD_CUDA(vglb_dev_alloc(&d_misc, 8 * 8));
-    PBUILD_CUDA(cudaMemsetAsync(d_deg_out, 0, (size_t)V * 4, st));
-    PBUILD_CUDA(cudaMemsetAsync(d_deg_in, 0, (size_t)V * 4, st));
-    PBUILD_CUDA(cudaMemsetAsync(d_deg_nl, 0, (size_t)V * 4, st));
-    PBUILD_CUDA(cudaMemsetAsync(d_bad, 0, 4, st));
-    PBUILD_CUDA(cudaMemsetAsync(d_misc, 0, 8 * 8, st));
+    CUDA_TRY(vglb_dev_alloc(d_deg_out, (size_t)V * 4));
+    CUDA_TRY(vglb_dev_alloc(d_deg_in, (size_t)V * 4));
+    CUDA_TRY(vglb_dev_alloc(d_deg_nl, (size_t)V * 4));
+    CUDA_TRY(vglb_dev_alloc(d_bad, 4));
+    CUDA_TRY(vglb_dev_alloc(d_misc, 8 * 8));
+    CUDA_TRY(cudaMemsetAsync(d_deg_out.get(), 0, (size_t)V * 4, st));
+    CUDA_TRY(cudaMemsetAsync(d_deg_in.get(), 0, (size_t)V * 4, st));
+    CUDA_TRY(cudaMemsetAsync(d_deg_nl.get(), 0, (size_t)V * 4, st));
+    CUDA_TRY(cudaMemsetAsync(d_bad.get(), 0, 4, st));
+    CUDA_TRY(cudaMemsetAsync(d_misc.get(), 0, 8 * 8, st));
     for (int half = 0; half < halves; half++)
         for (int64_t first = 0; first < S.edges; first += chunk)
         {
             const int64_t n = S.edges - first < chunk ? S.edges - first : chunk;
             const int32_t *ps, *pd;
-            int rc = provide_chunk(ctx, S, half, first, n, buf_a, buf_b, &ps, &pd);
-            if (rc != VGLB_OK) { cleanup(); return rc; }
-            part_degree_kernel<<<grid, 256, 0, st>>>(ps, pd, n, V, d_deg_out, d_deg_in, d_deg_nl, d_bad);
-            PBUILD_CUDA(cudaGetLastError());
-            PBUILD_CUDA(cudaStreamSynchronize(st)); // the chunk buffers are reused
+            VGLB_TRY(provide_chunk(ctx, S, half, first, n, buf_a.get(), buf_b.get(), &ps, &pd));
+            part_degree_kernel<<<grid, 256, 0, st>>>(ps, pd, n, V, d_deg_out.get(), d_deg_in.get(), d_deg_nl.get(), d_bad.get());
+            KERNEL_TRY();
+            CUDA_TRY(cudaStreamSynchronize(st)); // the chunk buffers are reused
         }
     int bad = 0;
-    PBUILD_CUDA(cudaMemcpy(&bad, d_bad, 4, cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(&bad, d_bad.get(), 4, cudaMemcpyDeviceToHost));
     if (bad)
     {
         vglb_set_error("partitioned build: vertex id out of range [0, V)");
-        cleanup();
         return VGLB_EINVAL;
     }
     // the reference's numbering: stable sort by out-degree descending, then the round-robin deal
-    PBUILD_CUDA(vglb_dev_alloc(&k0, (size_t)V * 4)); PBUILD_CUDA(vglb_dev_alloc(&k1, (size_t)V * 4));
-    PBUILD_CUDA(vglb_dev_alloc(&v0, (size_t)V * 4)); PBUILD_CUDA(vglb_dev_alloc(&v1, (size_t)V * 4));
-    part_sort_keys_kernel<<<(unsigned)ceil_div64(V, 256), 256, 0, st>>>(d_deg_out, V, k0, v0);
-    PBUILD_CUDA(cudaGetLastError());
     const int64_t cols = (int64_t)vp * P;
     {
-        cub::DoubleBuffer<uint32_t> keys(k0, k1), vals(v0, v1);
-        size_t tmp_bytes = 0;
-        PBUILD_CUDA(cub::DeviceRadixSort::SortPairs(NULL, tmp_bytes, keys, vals, V, 0, 32, st));
-        PBUILD_CUDA(vglb_dev_alloc(&tmp, tmp_bytes ? tmp_bytes : 16));
-        PBUILD_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, keys, vals, V, 0, 32, st));
-        PBUILD_CUDA(vglb_dev_alloc(&g->d_fwd, (size_t)V * 4));
-        PBUILD_CUDA(vglb_dev_alloc(&g->d_bwd, (size_t)cols * 4));
-        PBUILD_CUDA(cudaMemsetAsync(g->d_bwd, 0xFF, (size_t)cols * 4, st));
-        part_numbering_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(vals.Current(), V, P, vp, rank, d_deg_out, d_deg_in, g->d_fwd,
-                                                                g->d_bwd, d_misc);
-        PBUILD_CUDA(cudaGetLastError());
-        PBUILD_CUDA(cudaStreamSynchronize(st));
-        vglb_dev_free(tmp); tmp = NULL;
+        DegreeOrder order;
+        VGLB_TRY(vglb_degree_order(ctx, d_deg_out.get(), V, order));
+        CUDA_TRY(vglb_dev_alloc(&g->d_fwd, (size_t)V * 4));
+        CUDA_TRY(vglb_dev_alloc(&g->d_bwd, (size_t)cols * 4));
+        CUDA_TRY(cudaMemsetAsync(g->d_bwd, 0xFF, (size_t)cols * 4, st));
+        part_numbering_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(order.sorted, V, P, vp, rank, d_deg_out.get(), d_deg_in.get(), g->d_fwd,
+                                                                g->d_bwd, d_misc.get());
+        KERNEL_TRY();
+        CUDA_TRY(cudaStreamSynchronize(st));
     }
-    vglb_dev_free(k0); vglb_dev_free(k1); vglb_dev_free(v0); vglb_dev_free(v1);
-    k0 = k1 = v0 = v1 = NULL;
     unsigned long long totals[2] = {0, 0};
-    PBUILD_CUDA(cudaMemcpy(totals, d_misc, 16, cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(totals, d_misc.get(), 16, cudaMemcpyDeviceToHost));
     g->V = rows;
     g->vp = vp;
     g->cols = cols;
@@ -667,84 +615,75 @@ static int build_partitioned(vglb_ctx *ctx, vglb_comm *comm, int32_t V, const Ed
     g->comm = comm;
 
     // PageRank's inverse in-degrees of the owned rows come from pass 1 (the single-GPU path counts them from the CSR)
-    PBUILD_CUDA(vglb_dev_alloc(&g->d_pr_inv, (size_t)(vp > 0 ? vp : 1) * 4));
-    PBUILD_CUDA(cudaMemsetAsync(g->d_pr_inv, 0, (size_t)vp * 4, st));
+    CUDA_TRY(vglb_dev_alloc(&g->d_pr_inv, (size_t)(vp > 0 ? vp : 1) * 4));
+    CUDA_TRY(cudaMemsetAsync(g->d_pr_inv, 0, (size_t)vp * 4, st));
     if (rows > 0)
     {
-        part_pr_inverse_kernel<<<(unsigned)ceil_div64(rows, 256), 256, 0, st>>>(d_deg_nl, g->d_bwd, g->col_of_row0, rows, g->d_pr_inv);
-        PBUILD_CUDA(cudaGetLastError());
+        part_pr_inverse_kernel<<<(unsigned)ceil_div64(rows, 256), 256, 0, st>>>(d_deg_nl.get(), g->d_bwd, g->col_of_row0, rows, g->d_pr_inv);
+        KERNEL_TRY();
     }
 
     // pass 2, once per direction
-    PBUILD_CUDA(vglb_dev_alloc(&d_rowcnt, ((size_t)vp + 2) * 8));
+    CUDA_TRY(vglb_dev_alloc(d_rowcnt, ((size_t)vp + 2) * 8));
     for (int dir = 0; dir < ((flags & VGLB_GRAPH_WITH_INCOMING) ? 2 : 1); dir++)
     {
         const int64_t e_local = (int64_t)totals[dir];
         if (e_local >= 0xFFFFFFFFLL)
         {
             vglb_set_error("partitioned build: more than 2^32-1 edges on one rank");
-            cleanup();
             return VGLB_EINVAL;
         }
         const size_t kb = (size_t)(e_local > 0 ? e_local : 1) * 8;
-        PBUILD_CUDA(vglb_dev_alloc(&keys0, kb));
-        PBUILD_CUDA(vglb_dev_alloc(&keys1, kb));
-        PBUILD_CUDA(cudaMemsetAsync(d_rowcnt, 0, ((size_t)vp + 2) * 8, st));
-        PBUILD_CUDA(cudaMemsetAsync(d_misc + 2, 0, 8, st));
+        dev_ptr<uint64_t> keys0, keys1;
+        CUDA_TRY(vglb_dev_alloc(keys0, kb));
+        CUDA_TRY(vglb_dev_alloc(keys1, kb));
+        CUDA_TRY(cudaMemsetAsync(d_rowcnt.get(), 0, ((size_t)vp + 2) * 8, st));
+        CUDA_TRY(cudaMemsetAsync(d_misc.get() + 2, 0, 8, st));
         for (int half = 0; half < halves; half++)
             for (int64_t first = 0; first < S.edges; first += chunk)
             {
                 const int64_t n = S.edges - first < chunk ? S.edges - first : chunk;
                 const int32_t *ps, *pd;
-                int rc = provide_chunk(ctx, S, half, first, n, buf_a, buf_b, &ps, &pd);
-                if (rc != VGLB_OK) { cleanup(); return rc; }
-                part_collect_kernel<<<grid, 256, 0, st>>>(ps, pd, n, g->d_fwd, P, vp, rank, dir, keys0, d_misc + 2, d_rowcnt);
-                PBUILD_CUDA(cudaGetLastError());
-                PBUILD_CUDA(cudaStreamSynchronize(st));
+                VGLB_TRY(provide_chunk(ctx, S, half, first, n, buf_a.get(), buf_b.get(), &ps, &pd));
+                part_collect_kernel<<<grid, 256, 0, st>>>(ps, pd, n, g->d_fwd, P, vp, rank, dir, keys0.get(), d_misc.get() + 2,
+                                                          d_rowcnt.get());
+                KERNEL_TRY();
+                CUDA_TRY(cudaStreamSynchronize(st));
             }
         unsigned long long kept = 0;
-        PBUILD_CUDA(cudaMemcpy(&kept, d_misc + 2, 8, cudaMemcpyDeviceToHost));
+        CUDA_TRY(cudaMemcpy(&kept, d_misc.get() + 2, 8, cudaMemcpyDeviceToHost));
         if ((int64_t)kept != e_local)
         {
             vglb_set_error("partitioned build: kept %lld edges, expected %lld", (long long)kept, (long long)e_local);
-            cleanup();
             return VGLB_ECUDA;
         }
         int64_t **ptr_field = dir == 0 ? &g->d_out_ptr : &g->d_in_ptr;
         int32_t **adj_field = dir == 0 ? &g->d_out_adj : &g->d_in_adj;
-        PBUILD_CUDA(vglb_dev_alloc(ptr_field, ((size_t)vp + 2) * 8));
-        PBUILD_CUDA(vglb_dev_alloc(adj_field, (size_t)(e_local > 0 ? e_local : 1) * 4 + 16));
+        CUDA_TRY(vglb_dev_alloc(ptr_field, ((size_t)vp + 2) * 8));
+        CUDA_TRY(vglb_dev_alloc(adj_field, (size_t)(e_local > 0 ? e_local : 1) * 4 + 16));
         {
-            size_t tmp_bytes = 0;
-            PBUILD_CUDA(cub::DeviceScan::ExclusiveSum(NULL, tmp_bytes, (const int64_t *)d_rowcnt, *ptr_field, vp + 1, st));
-            PBUILD_CUDA(vglb_dev_alloc(&tmp, tmp_bytes ? tmp_bytes : 16));
-            PBUILD_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, (const int64_t *)d_rowcnt, *ptr_field, vp + 1, st));
-            PBUILD_CUDA(cudaStreamSynchronize(st));
-            vglb_dev_free(tmp); tmp = NULL;
+            dev_ptr<void> tmp;
+            CUDA_TRY(vglb_cub(tmp, [&](void *t, size_t &bytes) {
+                return cub::DeviceScan::ExclusiveSum(t, bytes, (const int64_t *)d_rowcnt.get(), *ptr_field, vp + 1, st);
+            }));
+            CUDA_TRY(cudaStreamSynchronize(st));
         }
         if (e_local > 0)
         {
-            cub::DoubleBuffer<uint64_t> keys(keys0, keys1);
-            size_t tmp_bytes = 0;
-            const int end_bit = 32 + bits_for64(vp);
-            PBUILD_CUDA(cub::DeviceRadixSort::SortKeys(NULL, tmp_bytes, keys, e_local, 0, end_bit, st));
-            PBUILD_CUDA(vglb_dev_alloc(&tmp, tmp_bytes ? tmp_bytes : 16));
-            PBUILD_CUDA(cub::DeviceRadixSort::SortKeys(tmp, tmp_bytes, keys, e_local, 0, end_bit, st));
+            cub::DoubleBuffer<uint64_t> keys(keys0.get(), keys1.get());
+            const int end_bit = 32 + vglb_key_bits(vp);
+            dev_ptr<void> tmp;
+            CUDA_TRY(vglb_cub(tmp, [&](void *t, size_t &bytes) {
+                return cub::DeviceRadixSort::SortKeys(t, bytes, keys, e_local, 0, end_bit, st);
+            }));
             part_adjacency_kernel<<<grid, 256, 0, st>>>(keys.Current(), e_local, P, vp, *adj_field);
-            PBUILD_CUDA(cudaGetLastError());
-            PBUILD_CUDA(cudaStreamSynchronize(st));
-            vglb_dev_free(tmp); tmp = NULL;
+            KERNEL_TRY();
+            CUDA_TRY(cudaStreamSynchronize(st));
         }
-        vglb_dev_free(keys0); vglb_dev_free(keys1);
-        keys0 = keys1 = NULL;
         if (dir == 0) g->E = e_local;
     }
-    int rc = vglb_graph_compute_tiers(ctx, g);
-    if (rc != VGLB_OK) { cleanup(); return rc; }
-    vglb_graph *result = g;
-    g = NULL; // keep the graph
-    cleanup();
-    *out_graph = result;
+    VGLB_TRY(vglb_graph_compute_tiers(ctx, g));
+    *out_graph = owner.release();
     return VGLB_OK;
 }
 
@@ -785,32 +724,6 @@ extern "C" int vglb_graph_from_generator_partitioned(vglb_ctx *ctx, vglb_comm *c
 // ---- VGL_Graph::move_to_device for one rank's part (vect_csr_graph.hpp:185-196): host arrays of an already-built part
 //      (this rank's row pointers and adjacency in column ids, the ORIGINAL -> column map) copied to HBM ----------------
 
-// bwd was filled with -1; a caller-supplied map must send every vertex to a distinct column in [0, cols)
-__global__ void part_invert_map_kernel(const int32_t *__restrict__ fwd, int32_t V, int64_t cols, int32_t *__restrict__ bwd,
-                                       int *__restrict__ bad)
-{
-    int32_t v = blockIdx.x * blockDim.x + threadIdx.x;
-    if (v >= V) return;
-    const int32_t c = fwd[v];
-    if (c < 0 || c >= cols) { *bad = 1; return; }
-    if (atomicExch(&bwd[c], v) != -1) *bad = 1;
-}
-
-__global__ void part_ptr_check_kernel(const int64_t *__restrict__ ptr, int32_t rows, int64_t E, int *__restrict__ bad)
-{
-    const int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (v == 0 && (ptr[0] != 0 || ptr[rows] != E)) *bad = 1;
-    if (v < rows && ptr[v] > ptr[v + 1]) *bad = 1;
-}
-
-__global__ void part_id_check_kernel(const int32_t *__restrict__ ids, int64_t n, int64_t limit, int *__restrict__ bad)
-{
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (; i < n; i += stride)
-        if (ids[i] < 0 || ids[i] >= limit) *bad = 1;
-}
-
 extern "C" int vglb_graph_from_csr_partitioned(vglb_ctx *ctx, vglb_comm *comm, int32_t vertices_global, int32_t rows,
                                                const int64_t *h_out_ptr, const int32_t *h_out_adj,
                                                const int32_t *h_orig_to_col, const int64_t *h_in_ptr,
@@ -825,9 +738,9 @@ extern "C" int vglb_graph_from_csr_partitioned(vglb_ctx *ctx, vglb_comm *comm, i
     const int32_t vp = (int32_t)(((ceil_div64(V, P) + 31) / 32) * 32);
     const int64_t E = h_out_ptr[rows], E_in = h_in_ptr ? h_in_ptr[rows] : 0;
     VGLB_REQUIRE(E >= 0 && E_in >= 0 && (E == 0 || h_out_adj != NULL), "vglb_graph_from_csr_partitioned: bad sizes");
-    vglb_graph *g = (vglb_graph *)calloc(1, sizeof(vglb_graph));
-    if (!g) return VGLB_ENOMEM;
-    auto cleanup = [&]() { vglb_graph_free_fields(g); free(g); };
+    graph_ptr owner = vglb_graph_new();
+    if (!owner) return VGLB_ENOMEM;
+    vglb_graph *g = owner.get();
     cudaStream_t st = ctx->stream;
     g->V = rows;
     g->E = E;
@@ -838,48 +751,39 @@ extern "C" int vglb_graph_from_csr_partitioned(vglb_ctx *ctx, vglb_comm *comm, i
     g->part_world = P;
     g->col_of_row0 = rank * vp;
     g->comm = comm;
-    PBUILD_CUDA(vglb_dev_alloc(&g->d_out_ptr, ((size_t)vp + 2) * 8));
-    PBUILD_CUDA(vglb_dev_alloc(&g->d_out_adj, (size_t)(E > 0 ? E : 1) * 4 + 16));
-    PBUILD_CUDA(cudaMemcpyAsync(g->d_out_ptr, h_out_ptr, ((size_t)rows + 1) * 8, cudaMemcpyHostToDevice, st));
-    PBUILD_CUDA(cudaMemcpyAsync(g->d_out_adj, h_out_adj, (size_t)E * 4, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(vglb_dev_alloc(&g->d_out_ptr, ((size_t)vp + 2) * 8));
+    CUDA_TRY(vglb_dev_alloc(&g->d_out_adj, (size_t)(E > 0 ? E : 1) * 4 + 16));
+    CUDA_TRY(cudaMemcpyAsync(g->d_out_ptr, h_out_ptr, ((size_t)rows + 1) * 8, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(g->d_out_adj, h_out_adj, (size_t)E * 4, cudaMemcpyHostToDevice, st));
     if (h_in_ptr)
     {
-        PBUILD_CUDA(vglb_dev_alloc(&g->d_in_ptr, ((size_t)vp + 2) * 8));
-        PBUILD_CUDA(vglb_dev_alloc(&g->d_in_adj, (size_t)(E_in > 0 ? E_in : 1) * 4 + 16));
-        PBUILD_CUDA(cudaMemcpyAsync(g->d_in_ptr, h_in_ptr, ((size_t)rows + 1) * 8, cudaMemcpyHostToDevice, st));
-        PBUILD_CUDA(cudaMemcpyAsync(g->d_in_adj, h_in_adj, (size_t)E_in * 4, cudaMemcpyHostToDevice, st));
+        CUDA_TRY(vglb_dev_alloc(&g->d_in_ptr, ((size_t)vp + 2) * 8));
+        CUDA_TRY(vglb_dev_alloc(&g->d_in_adj, (size_t)(E_in > 0 ? E_in : 1) * 4 + 16));
+        CUDA_TRY(cudaMemcpyAsync(g->d_in_ptr, h_in_ptr, ((size_t)rows + 1) * 8, cudaMemcpyHostToDevice, st));
+        CUDA_TRY(cudaMemcpyAsync(g->d_in_adj, h_in_adj, (size_t)E_in * 4, cudaMemcpyHostToDevice, st));
     }
-    PBUILD_CUDA(vglb_dev_alloc(&g->d_fwd, (size_t)V * 4));
-    PBUILD_CUDA(vglb_dev_alloc(&g->d_bwd, (size_t)g->cols * 4));
-    PBUILD_CUDA(cudaMemcpyAsync(g->d_fwd, h_orig_to_col, (size_t)V * 4, cudaMemcpyHostToDevice, st));
-    PBUILD_CUDA(cudaMemsetAsync(g->d_bwd, 0xFF, (size_t)g->cols * 4, st));
+    CUDA_TRY(vglb_dev_alloc(&g->d_fwd, (size_t)V * 4));
+    CUDA_TRY(vglb_dev_alloc(&g->d_bwd, (size_t)g->cols * 4));
+    CUDA_TRY(cudaMemcpyAsync(g->d_fwd, h_orig_to_col, (size_t)V * 4, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemsetAsync(g->d_bwd, 0xFF, (size_t)g->cols * 4, st));
     // caller-supplied arrays are checked on the device before anything indexes with them (row pointers non-decreasing
     // from 0 to E, column ids in [0, cols), the map injective); the verdict travels with the edge count so that a
     // rank with a bad part takes every rank out of the call together instead of leaving the others in a collective
     int *d_bad = (int *)(ctx->d_counters + CTR_BAD);
-    PBUILD_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int), st));
-    part_invert_map_kernel<<<(unsigned)ceil_div64(V, 256), 256, 0, st>>>(g->d_fwd, V, g->cols, g->d_bwd, d_bad);
-    PBUILD_CUDA(cudaGetLastError());
-    part_ptr_check_kernel<<<(unsigned)ceil_div64((int64_t)rows + 1, 256), 256, 0, st>>>(g->d_out_ptr, rows, E, d_bad);
-    PBUILD_CUDA(cudaGetLastError());
-    if (E > 0) part_id_check_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(g->d_out_adj, E, g->cols, d_bad);
-    if (h_in_ptr)
-    {
-        part_ptr_check_kernel<<<(unsigned)ceil_div64((int64_t)rows + 1, 256), 256, 0, st>>>(g->d_in_ptr, rows, E_in, d_bad);
-        if (E_in > 0) part_id_check_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(g->d_in_adj, E_in, g->cols, d_bad);
-    }
-    PBUILD_CUDA(cudaGetLastError());
+    CUDA_TRY(cudaMemsetAsync(d_bad, 0, sizeof(int), st));
+    VGLB_TRY(vglb_invert_map_checked(ctx, g->d_fwd, V, g->cols, g->d_bwd));
+    VGLB_TRY(vglb_csr_validate_device(ctx, g->d_out_ptr, rows, E, g->d_out_adj, g->cols));
+    if (h_in_ptr) VGLB_TRY(vglb_csr_validate_device(ctx, g->d_in_ptr, rows, E_in, g->d_in_adj, g->cols));
     int bad = 0;
-    PBUILD_CUDA(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, st));
-    PBUILD_CUDA(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
     // whole-graph edge count and the number of ranks with a bad part (a collective when the communicator is live)
     g->E_global = E;
     int64_t bad_ranks = bad ? 1 : 0;
     if (comm->nccl && P > 1)
     {
         int64_t r2[2] = {E, bad_ranks};
-        int rc = vglb_comm_allreduce_host(comm, r2, 2, VGLB_DT_I64, VGLB_OP_SUM);
-        if (rc != VGLB_OK) { cleanup(); return rc; }
+        VGLB_TRY(vglb_comm_allreduce_host(comm, r2, 2, VGLB_DT_I64, VGLB_OP_SUM));
         g->E_global = r2[0];
         bad_ranks = r2[1];
     }
@@ -887,11 +791,9 @@ extern "C" int vglb_graph_from_csr_partitioned(vglb_ctx *ctx, vglb_comm *comm, i
     {
         vglb_set_error("vglb_graph_from_csr_partitioned: %s part is not a CSR (row pointers non-decreasing from 0 to E, column "
                        "ids in [0, columns), ORIGINAL -> column map injective)", bad ? "this rank's" : "another rank's");
-        cleanup();
         return VGLB_EINVAL;
     }
-    int rc = vglb_graph_compute_tiers(ctx, g);
-    if (rc != VGLB_OK) { cleanup(); return rc; }
-    *out_graph = g;
+    VGLB_TRY(vglb_graph_compute_tiers(ctx, g));
+    *out_graph = owner.release();
     return VGLB_OK;
 }

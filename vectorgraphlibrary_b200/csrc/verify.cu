@@ -164,37 +164,33 @@ extern "C" int vglb_verify_ranking_f32(vglb_ctx *ctx, const float *d_a, const fl
 extern "C" int vglb_verify_components_i32(vglb_ctx *ctx, const int32_t *d_a, const int32_t *d_b, int32_t n, int64_t *error_count)
 {
     VGLB_REQUIRE(ctx != NULL && d_a != NULL && d_b != NULL && error_count != NULL && n >= 0, "vglb_verify_components_i32: bad argument");
-    int32_t *last = NULL;
-    CUDA_TRY(vglb_dev_alloc(&last, 2 * ((size_t)n + 2) * 4));
-    int32_t *last_a = last, *last_b = last + n + 2;
+    dev_ptr<int32_t> last;
+    CUDA_TRY(vglb_dev_alloc(last, 2 * ((size_t)n + 2) * 4));
+    int32_t *last_a = last.get(), *last_b = last.get() + n + 2;
     unsigned long long *d_out = (unsigned long long *)(ctx->d_counters + CTR_VERIFY_COUNT);
     int *d_bad = (int *)(ctx->d_counters + CTR_BAD);
-    CUDA_TRY(cudaMemsetAsync(last, 0xFF, 2 * ((size_t)n + 2) * 4, ctx->stream));
+    CUDA_TRY(cudaMemsetAsync(last.get(), 0xFF, 2 * ((size_t)n + 2) * 4, ctx->stream));
     CUDA_TRY(cudaMemsetAsync(d_out, 0, 8, ctx->stream));
     CUDA_TRY(cudaMemsetAsync(d_bad, 0, 4, ctx->stream));
-    int rc = VGLB_OK;
     if (n > 0)
     {
         components_last_index_kernel<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(d_a, d_b, n, last_a, last_b, d_bad);
+        KERNEL_TRY();
         int bad = 0;
-        if (cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, ctx->stream) != cudaSuccess || cudaStreamSynchronize(ctx->stream) != cudaSuccess)
-            rc = VGLB_ECUDA;
-        else if (bad)
+        CUDA_TRY(cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, ctx->stream));
+        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+        if (bad)
         {
             vglb_set_error("vglb_verify_components_i32: labels must lie in [0, n + 1]");
-            rc = VGLB_EINVAL;
+            return VGLB_EINVAL;
         }
-        if (rc == VGLB_OK)
-        {
-            components_compare_kernel<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(d_a, d_b, n, last_a, last_b, d_out);
-            if (cudaGetLastError() != cudaSuccess) rc = VGLB_ECUDA;
-            ctx->launches += 2;
-        }
+        components_compare_kernel<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(d_a, d_b, n, last_a, last_b, d_out);
+        KERNEL_TRY();
+        ctx->launches += 2;
     }
-    if (rc == VGLB_OK) rc = fetch_count(ctx, d_out, error_count);
-    cudaStreamSynchronize(ctx->stream);
-    vglb_dev_free(last);
-    return rc;
+    VGLB_TRY(fetch_count(ctx, d_out, error_count));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    return VGLB_OK;
 }
 
 // ---- EdgesArray: outgoing -> incoming mirror ---------------------------------------------------------------------------
@@ -204,52 +200,29 @@ static int edge_mirror_prepare(vglb_ctx *ctx, vglb_graph *g)
     if (g->d_in_to_out_pos) return VGLB_OK;
     VGLB_REQUIRE(g->comm == NULL, "vglb_earray_mirror_out_to_in: not available on a partitioned graph");
     VGLB_REQUIRE(g->E < 0xFFFFFFFFLL, "vglb_earray_mirror_out_to_in: more than 2^32 - 1 edges");
-    int rc = vglb_graph_derive_incoming(ctx, g); // no-op when the incoming CSR exists
-    if (rc != VGLB_OK) return rc;
+    VGLB_TRY(vglb_graph_derive_incoming(ctx, g)); // no-op when the incoming CSR exists
     const int64_t E = g->E;
     const size_t eb = (size_t)(E ? E : 1) * 4;
-    uint32_t *k0 = NULL, *k1 = NULL, *v0 = NULL, *v1 = NULL;
-    void *tmp = NULL;
-    auto cleanup = [&]() { vglb_dev_free(k0); vglb_dev_free(k1); vglb_dev_free(v0); vglb_dev_free(v1); vglb_dev_free(tmp); };
-#define MIRROR_CUDA(call)                                                                                   \
-    do                                                                                                      \
-    {                                                                                                       \
-        cudaError_t e__ = (call);                                                                           \
-        if (e__ != cudaSuccess)                                                                             \
-        {                                                                                                   \
-            vglb_set_error("CUDA error %s at %s:%d (%s)", cudaGetErrorString(e__), __FILE__, __LINE__, #call); \
-            cudaGetLastError();                                                                             \
-            cleanup();                                                                                      \
-            return e__ == cudaErrorMemoryAllocation ? VGLB_ENOMEM : VGLB_ECUDA;                             \
-        }                                                                                                   \
-    } while (0)
-    MIRROR_CUDA(vglb_dev_alloc(&k0, eb)); MIRROR_CUDA(vglb_dev_alloc(&k1, eb));
-    MIRROR_CUDA(vglb_dev_alloc(&v0, eb)); MIRROR_CUDA(vglb_dev_alloc(&v1, eb));
+    dev_ptr<uint32_t> k0, k1, v0, v1;
+    dev_ptr<void> tmp;
+    CUDA_TRY(vglb_dev_alloc(k0, eb)); CUDA_TRY(vglb_dev_alloc(k1, eb));
+    CUDA_TRY(vglb_dev_alloc(v0, eb)); CUDA_TRY(vglb_dev_alloc(v1, eb));
     if (E > 0)
     {
         // the sort that built the incoming CSR (stable, by destination, over the out positions), with the position as payload
-        MIRROR_CUDA(cudaMemcpyAsync(k0, g->d_out_adj, eb, cudaMemcpyDeviceToDevice, ctx->stream));
-        iota_u32_kernel<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(v0, E);
-        MIRROR_CUDA(cudaGetLastError());
-        int bits = 1;
-        while (bits < 32 && ((int64_t)1 << bits) < (int64_t)g->V) bits++;
-        cub::DoubleBuffer<uint32_t> keys(k0, k1), vals(v0, v1);
-        size_t tmp_bytes = 0;
-        MIRROR_CUDA(cub::DeviceRadixSort::SortPairs(NULL, tmp_bytes, keys, vals, E, 0, bits, ctx->stream));
-        MIRROR_CUDA(vglb_dev_alloc(&tmp, tmp_bytes ? tmp_bytes : 16));
-        MIRROR_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, keys, vals, E, 0, bits, ctx->stream));
-        MIRROR_CUDA(cudaStreamSynchronize(ctx->stream));
-        g->d_in_to_out_pos = vals.Current();
-        if (vals.Current() == v0) v0 = NULL;
-        else v1 = NULL;
+        CUDA_TRY(cudaMemcpyAsync(k0.get(), g->d_out_adj, eb, cudaMemcpyDeviceToDevice, ctx->stream));
+        iota_u32_kernel<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(v0.get(), E);
+        KERNEL_TRY();
+        const int bits = vglb_key_bits(g->V);
+        cub::DoubleBuffer<uint32_t> keys(k0.get(), k1.get()), vals(v0.get(), v1.get());
+        CUDA_TRY(vglb_cub(tmp, [&](void *t, size_t &bytes) {
+            return cub::DeviceRadixSort::SortPairs(t, bytes, keys, vals, E, 0, bits, ctx->stream);
+        }));
+        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+        g->d_in_to_out_pos = (vals.Current() == v0.get() ? v0 : v1).release();
     }
     else
-    {
-        g->d_in_to_out_pos = v0;
-        v0 = NULL;
-    }
-    cleanup();
-#undef MIRROR_CUDA
+        g->d_in_to_out_pos = v0.release();
     return VGLB_OK;
 }
 
@@ -258,8 +231,7 @@ extern "C" int vglb_earray_mirror_out_to_in_u32(vglb_ctx *ctx, vglb_graph *g, co
     VGLB_REQUIRE(ctx != NULL && g != NULL && d_out_values != NULL && d_in_values != NULL, "vglb_earray_mirror_out_to_in_u32: NULL argument");
     VGLB_REQUIRE(d_out_values != (const uint32_t *)d_in_values, "vglb_earray_mirror_out_to_in_u32: the mirror is out-of-place");
     CUDA_TRY(cudaSetDevice(ctx->device));
-    int rc = edge_mirror_prepare(ctx, g);
-    if (rc != VGLB_OK) return rc;
+    VGLB_TRY(edge_mirror_prepare(ctx, g));
     if (g->E > 0)
     {
         gather_u32_kernel<<<ctx->sm_count * 16, 256, 0, ctx->stream>>>(d_out_values, g->d_in_to_out_pos, g->E, d_in_values);
