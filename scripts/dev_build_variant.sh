@@ -6,7 +6,7 @@ cd "$(dirname "$0")/.."
 mkdir -p dev/obj_$name
 for f in vectorgraphlibrary_b200/csrc/*.cu; do
   o=dev/obj_$name/$(basename ${f%.cu}).o
-  if [ "$(basename $f)" = "pagerank.cu" ] || [ "$(basename $f)" = "sssp.cu" ] || [ ! -f $o ]; then
+  if [ "$(basename $f)" = "pagerank.cu" ] || [ "$(basename $f)" = "pagerank_bins.cu" ] || [ "$(basename $f)" = "sssp.cu" ] || [ ! -f $o ]; then
     nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -lineinfo --expt-relaxed-constexpr --extended-lambda -Xcompiler -fPIC,-O2,-fopenmp -I include -I vectorgraphlibrary_b200/csrc "$@" -c $f -o $o &
   fi
 done

@@ -76,6 +76,7 @@ struct PrBins
     int32_t *d_step_run0;
     int32_t *d_run_slot;
     int32_t *d_bin_chunk0, *d_cta_chunk0;
+    int32_t *d_warp_step0; // first step of every warp's piece of every (CTA, bin) (prb_warp_ranges_kernel)
     float *d_slot;       // [class][row chunk] partial sums, + 1 dummy
     int32_t *d_rc_ptr;   // first chunk of rows 0..long_rows
 };
@@ -85,7 +86,7 @@ struct PrbBinParams
     const uint16_t *wcol;
     const int32_t *cold;
     const uint32_t *meta;
-    const int32_t *step_run0, *run_slot, *bin_chunk0, *cta_chunk0;
+    const int32_t *step_run0, *run_slot, *bin_chunk0, *cta_chunk0, *warp_step0;
     const float *contrib_in;
     const float *inv;
     float *slot;

@@ -13,9 +13,9 @@
 // The run structure is static, so everything the segmented sum needs is precomputed per lane and warp step (`meta`), runs start
 // at multiples of 4 slots (padding gathers a zero) and a row's edges are cut into chunks of PRB_RC edges first, so no run is
 // longer than that (the longest rows of a power-law graph would otherwise serialise one warp).
-// Persistent kernel: one CTA of 32 warps per SM walks a contiguous, cost-balanced range of 4096-slot chunks; the warp that owns
-// a chunk emits the runs that START in it (it runs on past the end of the chunk until the next start). No atomics, fixed
-// summation order.
+// Persistent kernel: one CTA of 32 warps per SM walks a contiguous, cost-balanced range of 4096-slot chunks, and its warps take
+// cost-balanced pieces of its steps of each bin; the warp that owns a piece emits the runs that START in it (it runs on past the
+// end of the piece until the next start). No atomics, fixed summation order, whatever the cuts.
 #include <stdlib.h>
 
 #include <cub/device/device_scan.cuh>
@@ -27,6 +27,16 @@
 #define PRB_WARPS (PRB_THREADS / 32)
 #define PRB_DROP 0xff                   // class of a self loop: not part of the sum (pr.hpp:112)
 #define PRB_SMEM_BYTES ((PRB_H + 4) * 4 + PRB_WARPS * 2 * PRB_STAGE * 4)
+// estimated cost of a piece of a shared-memory bin = PRB_COST_STEP per step + PRB_COST_RUN per run that starts in it; it cuts
+// the bins' chunks into the persistent CTAs' ranges and a CTA's steps of a bin into its warps' pieces (-D: developer A/B builds;
+// pr_bin_kernel at RMAT-24 with 32 / 64 / 128 / 256 / 384 / 512 / 768 / 1024 per step: 378 / 292 / 246 / 225 / 226 / 235 / 240 /
+// 242 us, profiles/r6_pr_bin_cta_trace.txt)
+#ifndef PRB_COST_STEP
+#define PRB_COST_STEP 256
+#endif
+#ifndef PRB_COST_RUN
+#define PRB_COST_RUN 1
+#endif
 
 // meta word of one lane and step:
 //   bits 0..3   a run starts at slot 4 g of the lane         bits 4..11  run starts in the lanes before (this step)
@@ -241,13 +251,17 @@ __global__ void prb_meta_kernel(uint32_t *__restrict__ meta, int64_t nsteps, int
     if (s == nsteps - 1 && lane == 0) step_total[nsteps] = 0;
 }
 
-// estimated cost of a chunk of a shared-memory bin: its 8 steps + the runs it closes
+// estimated cost of the steps [s0, s1) of a shared-memory bin: its steps + the runs they close
+__device__ __forceinline__ int64_t prb_cost(const int32_t *__restrict__ step_run0, int64_t s0, int64_t s1)
+{
+    return (int64_t)PRB_COST_STEP * (s1 - s0) + (int64_t)PRB_COST_RUN * (step_run0[s1] - step_run0[s0]);
+}
+
 __global__ void prb_cost_kernel(const int32_t *__restrict__ step_run0, int32_t nkchunks, int64_t *__restrict__ cost)
 {
     const int32_t k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= nkchunks) return;
-    const int32_t closes = step_run0[(int64_t)(k + 1) * PRB_SPC] - step_run0[(int64_t)k * PRB_SPC];
-    cost[k] = 2048 + closes;
+    cost[k] = prb_cost(step_run0, (int64_t)k * PRB_SPC, (int64_t)(k + 1) * PRB_SPC);
 }
 
 __global__ void prb_cta_ranges_kernel(const int64_t *__restrict__ cum, int32_t nkchunks, int grid, int32_t *__restrict__ cta_chunk0)
@@ -268,6 +282,35 @@ __global__ void prb_cta_ranges_kernel(const int64_t *__restrict__ cum, int32_t n
         else lo = mid + 1;
     }
     cta_chunk0[b] = b == 0 ? 0 : lo;
+}
+
+// The steps of CTA b in bin c are cut into one piece per warp of equal estimated cost, with the estimate that cuts the CTA ranges
+// (equal steps per warp: 239 instead of 225 us at RMAT-24, profiles/r6_pr_bin_cta_trace.txt). Piece index b + c is unique: a
+// later CTA never starts in an earlier bin. warp_step0[(b + c) * (PRB_WARPS + 1) + w] = first step of warp w.
+__global__ void prb_warp_ranges_kernel(const int32_t *__restrict__ step_run0, const int32_t *__restrict__ bin_chunk0,
+                                       const int32_t *__restrict__ cta_chunk0, int grid, int nb, int32_t *__restrict__ warp_step0)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= grid * nb) return;
+    const int b = i / nb, c = i % nb;
+    const int b_lo = max(cta_chunk0[b], bin_chunk0[c]), b_hi = min(cta_chunk0[b + 1], bin_chunk0[c + 1]);
+    if (b_lo >= b_hi) return;
+    const int64_t S0 = (int64_t)b_lo * PRB_SPC, S1 = (int64_t)b_hi * PRB_SPC, total = prb_cost(step_run0, S0, S1);
+    int32_t *out = warp_step0 + (int64_t)(b + c) * (PRB_WARPS + 1);
+    out[0] = (int32_t)S0;
+    out[PRB_WARPS] = (int32_t)S1;
+    for (int w = 1; w < PRB_WARPS; w++)
+    {
+        const int64_t want = total * w / PRB_WARPS;
+        int64_t lo = S0, hi = S1; // first step s with cost(S0, s) >= want
+        while (lo < hi)
+        {
+            const int64_t mid = (lo + hi) >> 1;
+            if (prb_cost(step_run0, S0, mid) >= want) hi = mid;
+            else lo = mid + 1;
+        }
+        out[w] = (int32_t)lo;
+    }
 }
 
 __global__ void prb_fill_u16_kernel(uint16_t *a, int64_t n, uint16_t val)
@@ -293,6 +336,7 @@ struct prb_deleter
         vglb_dev_free(B->d_run_slot);
         vglb_dev_free(B->d_bin_chunk0);
         vglb_dev_free(B->d_cta_chunk0);
+        vglb_dev_free(B->d_warp_step0);
         vglb_dev_free(B->d_slot);
         vglb_dev_free(B->d_rc_ptr);
         free(B);
@@ -391,6 +435,8 @@ int vglb_pr_bins_build_rows(vglb_ctx *ctx, vglb_graph *g, int32_t rows)
     CUDA_TRY(vglb_dev_alloc(&B->d_run_slot, (size_t)nruns * 4));
     CUDA_TRY(vglb_dev_alloc(&B->d_slot, ((size_t)n + 1) * 4));
     CUDA_TRY(vglb_dev_alloc(&B->d_cta_chunk0, ((size_t)B->grid + 1) * 4));
+    CUDA_TRY(vglb_dev_alloc(&B->d_warp_step0, ((size_t)B->grid + nb) * (PRB_WARPS + 1) * 4));
+    CUDA_TRY(cudaMemsetAsync(B->d_warp_step0, 0, ((size_t)B->grid + nb) * (PRB_WARPS + 1) * 4, st)); // (a CTA without chunks: empty pieces)
     CUDA_TRY(cudaMemsetAsync(B->d_slot, 0, ((size_t)n + 1) * 4, st));
     CUDA_TRY(cudaMemsetAsync(B->d_meta, 0, (size_t)nsteps * 32 * 4, st));
     CUDA_TRY(cudaMemsetAsync(B->d_cold, 0xFF, (size_t)(W - w_smem) * 4, st));
@@ -430,8 +476,11 @@ int vglb_pr_bins_build_rows(vglb_ctx *ctx, vglb_graph *g, int32_t rows)
     }
     prb_cta_ranges_kernel<<<(unsigned)ceil_div64(B->grid + 1, 256), 256, 0, st>>>(d_cost.get(), B->cold_chunk0, B->grid, B->d_cta_chunk0);
     KERNEL_TRY();
+    prb_warp_ranges_kernel<<<(unsigned)ceil_div64((int64_t)B->grid * nb, 256), 256, 0, st>>>(B->d_step_run0, B->d_bin_chunk0, B->d_cta_chunk0,
+                                                                                              B->grid, nb, B->d_warp_step0);
+    KERNEL_TRY();
     CUDA_TRY(cudaStreamSynchronize(st));
-    ctx->launches += 12;
+    ctx->launches += 13;
     g->pr_bins = owner.release();
     return VGLB_OK;
 }
@@ -440,6 +489,28 @@ int vglb_pr_bins_build_rows(vglb_ctx *ctx, vglb_graph *g, int32_t rows)
 
 extern __shared__ __align__(16) float prb_smem[];
 
+#ifdef PRB_CTA_TRACE
+// developer build (scripts/dev_pr_bin_cta_trace.py): the last launch of pr_bin_kernel records, per CTA, %globaltimer at its start
+// and end, its chunks, runs and bins and the time between the two barriers of its slice loads; per warp, the time in its units,
+// their steps and runs and %globaltimer at its end
+#define PRB_TRACE_CTAS 1024
+__device__ unsigned long long prb_trace_cta[PRB_TRACE_CTAS][8];
+__device__ unsigned long long prb_trace_warp[PRB_TRACE_CTAS][PRB_WARPS][4];
+__device__ __forceinline__ unsigned long long prb_now()
+{
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+extern "C" int vglb_dev_prb_cta_trace(unsigned long long *cta, unsigned long long *warp, int ctas)
+{
+    if (ctas > PRB_TRACE_CTAS) return VGLB_EINVAL;
+    CUDA_TRY(cudaMemcpyFromSymbol(cta, prb_trace_cta, (size_t)ctas * 8 * 8));
+    CUDA_TRY(cudaMemcpyFromSymbol(warp, prb_trace_warp, (size_t)ctas * PRB_WARPS * 4 * 8));
+    return VGLB_OK;
+}
+#endif
+
 __global__ void __launch_bounds__(PRB_THREADS, 1) pr_bin_kernel(const __grid_constant__ PrbBinParams P)
 {
     L2Pol pol;
@@ -447,16 +518,22 @@ __global__ void __launch_bounds__(PRB_THREADS, 1) pr_bin_kernel(const __grid_con
     pol.keep = l2_policy_evict_last();
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int k_lo = P.cta_chunk0[blockIdx.x], k_hi = P.cta_chunk0[blockIdx.x + 1];
+#ifdef PRB_CTA_TRACE
+    if (threadIdx.x == 0 && blockIdx.x < PRB_TRACE_CTAS) prb_trace_cta[blockIdx.x][0] = prb_now();
+    unsigned t_load = 0, w_busy = 0, w_steps = 0, w_runs = 0, nbins = 0; // (32 bits: the trace must not cost the kernel registers)
+#endif
     float *stage = prb_smem + PRB_H + 4 + warp * 2 * PRB_STAGE;
     const int nc = P.nb; // (the cold bin's chunks are blocks of pr_sweep_kernel: they need the L1 this kernel gives to shared memory)
     int bin = 0;
     while (bin < nc && P.bin_chunk0[bin + 1] <= k_lo) bin++;
     for (; bin < nc && P.bin_chunk0[bin] < k_hi; bin++)
     {
-        const int b_lo = max(k_lo, P.bin_chunk0[bin]), b_hi = min(k_hi, P.bin_chunk0[bin + 1]);
         const int bin_end_step = P.bin_chunk0[bin + 1] * PRB_SPC;
         {
             __syncthreads();
+#ifdef PRB_CTA_TRACE
+            const unsigned t_l0 = (unsigned)prb_now();
+#endif
             // this bin's slice of the contribution vector (the last bin of a small graph is shorter)
             const int64_t c0 = (int64_t)bin * PRB_H;
             const int n = (int)min((int64_t)PRB_H, P.cols - c0);
@@ -479,12 +556,47 @@ __global__ void __launch_bounds__(PRB_THREADS, 1) pr_bin_kernel(const __grid_con
             }
             if (threadIdx.x < 4) prb_smem[PRB_H + threadIdx.x] = 0.f; // what a padding slot gathers
             __syncthreads();
-            // every warp streams one contiguous piece of this CTA's steps of the bin
-            const int64_t nst = (int64_t)(b_hi - b_lo) * PRB_SPC;
-            const int s0 = b_lo * PRB_SPC + (int)(nst * warp / PRB_WARPS), s1 = b_lo * PRB_SPC + (int)(nst * (warp + 1) / PRB_WARPS);
+#ifdef PRB_CTA_TRACE
+            t_load += (unsigned)prb_now() - t_l0;
+            nbins++;
+#endif
+            // every warp streams one contiguous piece of this CTA's steps of the bin, cut by estimated cost
+            const int32_t *ws = P.warp_step0 + (int64_t)(blockIdx.x + bin) * (PRB_WARPS + 1) + warp;
+            const int s0 = ws[0], s1 = ws[1];
+#ifdef PRB_CTA_TRACE
+            const unsigned t_u0 = (unsigned)prb_now();
+#endif
             if (s0 < s1) prb_unit<false>(P, pol, prb_smem, s0, s1, bin_end_step, lane, stage, 0.f);
+#ifdef PRB_CTA_TRACE
+            w_busy += (unsigned)prb_now() - t_u0;
+            w_steps += s1 - s0;
+            w_runs += P.step_run0[s1] - P.step_run0[s0];
+#endif
         }
     }
+#ifdef PRB_CTA_TRACE
+    if (blockIdx.x < PRB_TRACE_CTAS)
+    {
+        if (lane == 0)
+        {
+            unsigned long long *w = prb_trace_warp[blockIdx.x][warp];
+            w[0] = w_busy;
+            w[1] = w_steps;
+            w[2] = w_runs;
+            w[3] = prb_now();
+        }
+        __syncthreads();
+        if (threadIdx.x == 0)
+        {
+            unsigned long long *c = prb_trace_cta[blockIdx.x];
+            c[1] = prb_now();
+            c[2] = (unsigned long long)(k_hi - k_lo);
+            c[3] = (unsigned long long)(P.step_run0[k_hi * PRB_SPC] - P.step_run0[k_lo * PRB_SPC]);
+            c[4] = nbins;
+            c[5] = t_load;
+        }
+    }
+#endif
 }
 
 void vglb_pr_bins_params(const vglb_graph *g, const float *contrib_in, PrbBinParams *P)
@@ -497,6 +609,7 @@ void vglb_pr_bins_params(const vglb_graph *g, const float *contrib_in, PrbBinPar
     P->run_slot = B->d_run_slot;
     P->bin_chunk0 = B->d_bin_chunk0;
     P->cta_chunk0 = B->d_cta_chunk0;
+    P->warp_step0 = B->d_warp_step0;
     P->contrib_in = contrib_in;
     P->inv = g->d_pr_inv;
     P->slot = B->d_slot;
