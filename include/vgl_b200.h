@@ -254,6 +254,22 @@ int vglb_sssp(vglb_ctx *ctx, vglb_graph *g, const float *d_weights, int32_t sour
  * {v} U ancestors(v) (= component minimum on symmetric graphs). */
 int vglb_cc(vglb_ctx *ctx, vglb_graph *g, int32_t *d_labels, vglb_stats *stats);
 
+/* HITS hub and authority scores (algorithms/hits/hits.hpp:5-100): `steps` (1 <= steps < 2^20) steps of
+ *   a_raw[v] = sum_{u->v} h_{t-1}[u],  a_t = a_raw / ||a_raw||_2;   then  h_raw[u] = sum_{u->v} a_t[v],  h_t = h_raw / ||h_raw||_2
+ * (Kleinberg's sequential form: the hub update uses the new authorities). Every CSR edge counts: duplicate edges with their
+ * multiplicity, self loops included (unlike PageRank's v != u). After the first normalisation the start vector does not matter
+ * (h_0 = 1). A vector whose sum of squares is 0 (only when the graph has no edges) stays all zero, with no NaN. d_auth and d_hub
+ * are fp32[V] in SCATTER numbering, owned by the caller; between passes they hold the raw sums. The authority pass pulls over the
+ * incoming CSR, the hub pass over the outgoing one, each in one kernel whose load balance does not depend on row order (the
+ * incoming rows are not degree-sorted). Row sums are fp32 in a fixed order, squared norms are summed in fp64 in a fixed order
+ * and there are no float atomics on the vectors: two calls give the same bits. A one-GPU graph without the incoming CSR gets it
+ * derived by the first call (as vglb_bfs); partitioned graphs return VGLB_EINVAL. The only host synchronisation is the end of
+ * the run. stats: iterations = steps, edges_inspected = 2 E steps, vertices_processed = 2 V steps, and
+ *   algorithmic_bytes = 2 steps (8 E + 12 V) + 16 V
+ * (per pass: an edge reads its 4-byte index and one gathered fp32, a row its 8-byte row pointer and writes its 4-byte result;
+ * the final normalisation reads and writes both vectors). */
+int vglb_hits(vglb_ctx *ctx, vglb_graph *g, int steps, float *d_auth, float *d_hub, vglb_stats *stats);
+
 /* ---- operators with fixed predicates (generate_new_frontier / reduce / compute without lambdas) ----
  * FrontierVectorCSR (frontier_vect_csr.h:5-53): sparse id queue + dense bitmap, chosen by density. */
 typedef struct vglb_frontier vglb_frontier;

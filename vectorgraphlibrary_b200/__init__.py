@@ -10,6 +10,7 @@ and benchmarks and mirrors the reference's object model for the hot path:
     PageRank::vgl_page_rank        -> Graph.pagerank                (algorithms/pr/pr.hpp:7-148)
     ShortestPaths::vgl_dijkstra    -> Graph.sssp                    (algorithms/sssp/shortest_paths.hpp:298-317)
     ConnectedComponents::vgl_shiloach_vishkin -> Graph.cc           (algorithms/cc/shiloach_vishkin.hpp:7-88)
+    HITS::vgl_hits                 -> Graph.hits                    (algorithms/hits/hits.hpp:5-100)
 
 There is no CPU fallback: importing works anywhere (so the symbol table can be checked on a CPU box), but creating a
 Context raises VglbError when no CUDA device is usable, and a missing shared object raises at import of `lib()`.
@@ -114,6 +115,7 @@ _SIGNATURES = {
     "vglb_bfs_multi": (C.c_int, [_P, _P, C.c_int32, _P, _P, C.POINTER(BfsOpts), C.POINTER(Stats)]),
     "vglb_sssp": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.POINTER(Stats)]),
     "vglb_cc": (C.c_int, [_P, _P, _P, C.POINTER(Stats)]),
+    "vglb_hits": (C.c_int, [_P, _P, C.c_int, _P, _P, C.POINTER(Stats)]),
     "vglb_frontier_create": (C.c_int, [_P, _P, C.POINTER(_P)]),
     "vglb_frontier_create_borrowed": (C.c_int, [_P, _P, _P, C.POINTER(_P)]),
     "vglb_frontier_set_ids": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int]),
@@ -559,6 +561,14 @@ class Graph:
         st = Stats()
         _check(lib().vglb_cc(self.ctx.h, self.h, labels.ptr, C.byref(st)))
         return labels, st
+
+    def hits(self, steps: int = 20, auth: DeviceArray | None = None, hub: DeviceArray | None = None):
+        """vglb_hits: `steps` HITS steps. Returns (authority scores, hub scores, Stats), fp32 in SCATTER numbering."""
+        auth = auth or self.ctx.empty(self.V, np.float32)
+        hub = hub or self.ctx.empty(self.V, np.float32)
+        st = Stats()
+        _check(lib().vglb_hits(self.ctx.h, self.h, int(steps), auth.ptr, hub.ptr, C.byref(st)))
+        return auth, hub, st
 
 
 def verify_results(ctx: "Context", a: DeviceArray, b: DeviceArray) -> int:
