@@ -270,6 +270,25 @@ int vglb_cc(vglb_ctx *ctx, vglb_graph *g, int32_t *d_labels, vglb_stats *stats);
  * the final normalisation reads and writes both vectors). */
 int vglb_hits(vglb_ctx *ctx, vglb_graph *g, int steps, float *d_auth, float *d_hub, vglb_stats *stats);
 
+/* Triangle counting (algorithms/tc). Counts the triangles of the undirected simple graph under the OUTGOING CSR: {u, v} is an
+ * edge when u != v and u->v or v->u is in the CSR. Duplicate edges count once, self loops are ignored and the direction of an
+ * edge does not matter, so a symmetrised input gives the same result. Only the outgoing CSR is read: graphs without the
+ * incoming CSR, from vglb_graph_from_csr and from vglb_graph_borrow_csr all work.
+ * d_counts is an int64[V] array owned by the caller, in SCATTER numbering: d_counts[v] = triangles that contain v. *h_total =
+ * the number of triangles (3 * total == sum of d_counts). Both must be non-NULL. All arithmetic is integer: two calls return
+ * identical arrays. A graph without edges gives zero counts and a total of 0; partitioned graphs return VGLB_EINVAL.
+ * Every call builds a degree-oriented CSR on the device (row u holds its undirected neighbours with a smaller SCATTER id,
+ * ascending) and nothing is kept with the graph; stats->seconds covers the build. The only host synchronisation is the end
+ * of the call. For each oriented edge (u, v) at position j of row u, the kernel intersects the row's first j entries with
+ * row v: when 2 j < |row v| the j entries are read and each is looked up in row v by binary search, otherwise row v is read
+ * and each entry is looked up in the first j.
+ * stats: iterations = 1, edges_inspected = the list elements the intersections read (sum over oriented edges of
+ * j if 2 j < |row v|, else |row v|), vertices_processed = the rows of the oriented CSR with at least one entry, and
+ *   algorithmic_bytes = 8 E + 12 E+ + 4 edges_inspected + 16 V
+ * (E+ = edges of the oriented CSR; the build reads 8 bytes per CSR edge, an oriented edge its 4-byte id and the 8-byte row
+ * pointer of its target, a list element 4 bytes, a vertex its 8-byte row pointer and its 8-byte count store). */
+int vglb_tc(vglb_ctx *ctx, vglb_graph *g, int64_t *d_counts, int64_t *h_total, vglb_stats *stats);
+
 /* ---- operators with fixed predicates (generate_new_frontier / reduce / compute without lambdas) ----
  * FrontierVectorCSR (frontier_vect_csr.h:5-53): sparse id queue + dense bitmap, chosen by density. */
 typedef struct vglb_frontier vglb_frontier;

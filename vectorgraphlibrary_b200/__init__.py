@@ -11,6 +11,7 @@ and benchmarks and mirrors the reference's object model for the hot path:
     ShortestPaths::vgl_dijkstra    -> Graph.sssp                    (algorithms/sssp/shortest_paths.hpp:298-317)
     ConnectedComponents::vgl_shiloach_vishkin -> Graph.cc           (algorithms/cc/shiloach_vishkin.hpp:7-88)
     HITS::vgl_hits                 -> Graph.hits                    (algorithms/hits/hits.hpp:5-100)
+    triangle counting              -> Graph.tc                      (algorithms/tc)
 
 There is no CPU fallback: importing works anywhere (so the symbol table can be checked on a CPU box), but creating a
 Context raises VglbError when no CUDA device is usable, and a missing shared object raises at import of `lib()`.
@@ -116,6 +117,7 @@ _SIGNATURES = {
     "vglb_sssp": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.POINTER(Stats)]),
     "vglb_cc": (C.c_int, [_P, _P, _P, C.POINTER(Stats)]),
     "vglb_hits": (C.c_int, [_P, _P, C.c_int, _P, _P, C.POINTER(Stats)]),
+    "vglb_tc": (C.c_int, [_P, _P, _P, C.POINTER(C.c_int64), C.POINTER(Stats)]),
     "vglb_frontier_create": (C.c_int, [_P, _P, C.POINTER(_P)]),
     "vglb_frontier_create_borrowed": (C.c_int, [_P, _P, _P, C.POINTER(_P)]),
     "vglb_frontier_set_ids": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int]),
@@ -569,6 +571,15 @@ class Graph:
         st = Stats()
         _check(lib().vglb_hits(self.ctx.h, self.h, int(steps), auth.ptr, hub.ptr, C.byref(st)))
         return auth, hub, st
+
+    def tc(self, counts: DeviceArray | None = None):
+        """vglb_tc: triangles of the undirected simple graph under the outgoing CSR. Returns (int64 triangles per vertex in
+        SCATTER numbering, total, Stats)."""
+        counts = counts or self.ctx.empty(self.V, np.int64)
+        total = C.c_int64()
+        st = Stats()
+        _check(lib().vglb_tc(self.ctx.h, self.h, counts.ptr, C.byref(total), C.byref(st)))
+        return counts, total.value, st
 
 
 def verify_results(ctx: "Context", a: DeviceArray, b: DeviceArray) -> int:

@@ -165,6 +165,13 @@ enum
     CTR_PEER_TABLE = 24,
     CTR_REDUCE = 32,         // vglb_reduce_*: the frontier reduce result (i64 or f64)
     CTR_CC_CHANGED = 40,     // CC: a hook changed a label this round (int32, device and host)
+    // triangle counting (u64, tc.cu): cleared at the start of vglb_tc, read back once at its end
+    CTR_TC_TOTAL = 41,       // triangles (row sums of tc_count_kernel)
+    CTR_TC_UNIQUE = 42,      // distinct keys of the oriented-CSR build (the self-loop key included)
+    CTR_TC_EDGES = 43,       // E+: edges of the oriented CSR
+    CTR_TC_ROWS = 44,        // rows of the oriented CSR with at least one entry
+    CTR_TC_ELEMENTS = 45,    // list elements the intersections read
+    CTR_TC_END = 46,
     CTR_HOST_ALLREDUCE = 52, // vglb_comm_allreduce_host: up to two 8-byte host values on their way through the allreduce
     CTR_BAD = 56,            // CSR / label validation: a check failed (int32)
     CTR_VERIFY_COUNT = 57,   // vglb_verify_*: mismatches (u64)
@@ -174,11 +181,13 @@ enum
     MAILBOX_WORDS = 56,      // vglb_counters_fetch copies at most this many words
     MAILBOX_SEQ = 63         // mailbox word that carries the sequence number
 };
-static_assert(DR_END <= CTR_PEER_TABLE && CTR_REDUCE < CTR_CC_CHANGED && CTR_CC_CHANGED < CTR_HOST_ALLREDUCE &&
+static_assert(DR_END <= CTR_PEER_TABLE && CTR_REDUCE < CTR_CC_CHANGED && CTR_CC_CHANGED < CTR_TC_TOTAL &&
+                  CTR_TC_END <= CTR_HOST_ALLREDUCE &&
                   CTR_HOST_ALLREDUCE + 2 <= CTR_BAD && CTR_VERIFY_SUMS + 2 <= CTR_SSSP_WMAX && CTR_SSSP_WMAX < CTR_WORDS &&
                   MAILBOX_WORDS < MAILBOX_SEQ && MAILBOX_SEQ < CTR_WORDS,
               "counter slots in order, each inside the block");
-static_assert(C_COUNT <= MAILBOX_WORDS && CTR_SSSP_ROUND <= MAILBOX_WORDS && DR_END <= MAILBOX_WORDS && M_COUNT <= MAILBOX_WORDS,
+static_assert(C_COUNT <= MAILBOX_WORDS && CTR_SSSP_ROUND <= MAILBOX_WORDS && DR_END <= MAILBOX_WORDS && M_COUNT <= MAILBOX_WORDS &&
+                  CTR_TC_END <= MAILBOX_WORDS,
               "every run read through the mailbox fits it");
 
 struct vglb_graph
